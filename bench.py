@@ -100,7 +100,15 @@ def parse_args():
     ap.add_argument("--no-precheck", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned to DIR/<name>.npy (float64): "
+                         "counts (satisfied blocks per pair), product_blocks (a fixed, seeded sample of block indices of "
+                         "the products, pair-major) and product_words (those blocks' words, [..., 0] = high and [..., 1] = "
+                         "low 32 bits); one file set per rank, suffixed _rank<r>, when N > 1")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path (--impl ours)")
+    return args
 
 
 def words_per_block(N):
@@ -362,6 +370,29 @@ def event_time_us(torch, fn, n_items, reps=3, rounds=3):
         torch.cuda.synchronize()
         res.append(e0.elapsed_time(e1) * 1e3 / (reps * n_items))
     return float(np.median(res))
+
+
+DUMP_BYTES = 48 << 20      # product words of a whole dump (all ranks), as float64 halves: 16 bytes per word
+
+
+def sample_outputs(torch, products, L, counts, world):
+    """What --dump-outputs writes: the counts and a fixed sample of product blocks.  `products` is a device tensor of
+    int64 words holding whole blocks, pair-major.  The sample depends only on the number of blocks and ranks, so two
+    runs with the same arguments sample the same blocks; every rank takes 1/world of the budget."""
+    total = products.numel() // L
+    rng = np.random.default_rng(20240613)
+    idx = np.unique(rng.integers(0, total, size=min(total, DUMP_BYTES // (16 * L * world))))
+    rows = products.reshape(total, L)[torch.from_numpy(idx).to(products.device)]
+    words = rows.cpu().numpy().view(np.uint64)
+    return {"counts": counts.cpu().numpy().astype(np.float64),
+            "product_blocks": idx.astype(np.float64),
+            "product_words": np.stack([words >> np.uint64(32), words & np.uint64(0xFFFFFFFF)], axis=-1).astype(np.float64)}
+
+
+def write_outputs(path, arrays, rank, world):
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ("_rank%d" % rank if world > 1 else "") + ".npy"), a)
 
 
 def precheck(eng, torch, dev, rank, world, comm):
@@ -842,6 +873,7 @@ def run_ours(args):
 
     K = args.steps
     main = timed_run(K, fused)
+    dump = sample_outputs(torch, out, L, counts2[(K - 1) & 1], world) if args.dump_outputs else None   # the last step's slot
     blocks_per_step = P * T1 * T2 * world            # whole job (T1 = per-rank share)
     value = blocks_per_step * K / (main["total_ms"] * 1e-3)
     bytes_per_block = 8 * L
@@ -1055,12 +1087,14 @@ def run_ours(args):
     if rank == 0:
         if world == 1 and extras and args.workload == "cfg2" and not (args.t1 or args.t2):
             torch.cuda.synchronize()
-            line["e2e_cpp"] = cpp_e2e(P, 50)
+            line["e2e_cpp"] = cpp_e2e(P, K)
         if world == 1 and not args.no_cpu_baseline:
             # the reference overflows its int counters above 131,080 blocks at N=16383 (SURVEY hazard 4): the CPU
             # sample always uses the workload's own sizes, whatever --t1/--t2 say
             line["cpu_baseline"] = cpu_baseline(N, D, *WORKLOADS[args.workload][2:4])
         print(json.dumps(line), flush=True)
+    if dump:
+        write_outputs(args.dump_outputs, dump, rank, world)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
@@ -1171,6 +1205,7 @@ def run_chain(args):
     launches = eng.launch_count() - launches0
     if not torch.equal(want, counts):
         raise SystemExit("cfg4 check failed after the timed region: %s != %s" % (counts, want))
+    dump = sample_outputs(torch, y, L, counts, world) if args.dump_outputs else None
     phases = [sum(e[i].elapsed_time(e[i + 1]) for e in evs) for i in range(4)]
     t = torch.tensor([evs[0][0].elapsed_time(evs[K - 1][4])] + phases, dtype=torch.float64, device=dev)
     if world > 1:
@@ -1250,6 +1285,8 @@ def run_chain(args):
             cb["sample"] += "; per-block cost of the chain is the same multiply+decrypt work"
             line["cpu_baseline"] = cb
         print(json.dumps(line), flush=True)
+    if dump:
+        write_outputs(args.dump_outputs, dump, rank, world)
     if world > 1:
         dist.destroy_process_group()
     return 0

@@ -7,11 +7,36 @@
 // identities on random circuits.  Exit status 0 = all good.
 #include "certFHE.h"
 
+#include <cstdio>
+#include <cstdlib>
 #include <sstream>
+#include <string>
+#include <vector>
+
+#include <unistd.h>
 
 using namespace certFHE;
 
 static int failures = 0;
+
+// the files this program writes go to a fresh directory under $TMPDIR (default /tmp), so that runs by several users or
+// at the same time never meet each other's files
+static std::string scratch;
+static std::string scratch_file(const char *name) {
+    if (scratch.empty()) {
+        const char *base = getenv("TMPDIR");
+        std::string tmpl = std::string(base && *base ? base : "/tmp") + "/csgn_accept_XXXXXX";
+        std::vector<char> buf(tmpl.begin(), tmpl.end());
+        buf.push_back('\0');
+        if (!mkdtemp(buf.data())) {
+            perror("mkdtemp");
+            exit(2);
+        }
+        scratch = buf.data();
+    }
+    return scratch + "/" + name;
+}
+
 #define EXPECT(cond)                                                            \
     do {                                                                        \
         if (!(cond)) {                                                          \
@@ -182,7 +207,7 @@ static void lazy_products() {
     EXPECT(seckey.decrypt(mixed).getValue() == ((pa & pb & pd) ^ (pa & pb)));
     Library::setLazyProducts(false);
     // save / load: the words, the context and the decrypted bit survive the file
-    const std::string path = "/tmp/csgn_accept_demo.ct";
+    const std::string path = scratch_file("demo.ct");
     eager.save(path);
     Ciphertext loaded = Ciphertext::load(path);
     EXPECT(loaded.getLen() == eager.getLen() && loaded.getContext().getN() == 1247 && loaded.getContext().getD() == 16);
@@ -338,28 +363,29 @@ static void files() {
     int parity = 0;
     for (size_t i = 0; i < bits.size(); ++i) { bits[i] = rand() & 1; parity ^= bits[i]; }
     Ciphertext c = seckey.encryptBatch(bits.data(), bits.size(), 9);
-    seckey.save("/tmp/csgn_accept.sk");
-    pi.save("/tmp/csgn_accept.pm");
+    const std::string sk = scratch_file("accept.sk"), pm = scratch_file("accept.pm"), ct = scratch_file("accept.ct");
+    seckey.save(sk);
+    pi.save(pm);
     srand(5);
     const int before = rand();
     srand(5);
-    SecretKey k2 = SecretKey::load("/tmp/csgn_accept.sk");
+    SecretKey k2 = SecretKey::load(sk);
     EXPECT(rand() == before);                                   // loading a key leaves the caller's rand() sequence alone
-    Permutation p2 = Permutation::load("/tmp/csgn_accept.pm");
+    Permutation p2 = Permutation::load(pm);
     EXPECT(k2.getLength() == seckey.getLength() && memcmp(k2.getKey(), seckey.getKey(), 16 * 8) == 0);
     EXPECT(p2.getLength() == 1247 && memcmp(p2.getPermutation(), pi.getPermutation(), 1247 * 8) == 0);
     EXPECT(k2.decrypt(c).getValue() == parity);
     EXPECT(k2.applyPermutation(p2).decrypt(*new Ciphertext(c.applyPermutation(p2))).getValue() == parity);
-    c.saveSharded("/tmp/csgn_accept.ct");
-    Ciphertext back = Ciphertext::loadSharded("/tmp/csgn_accept.ct");
+    c.saveSharded(ct);
+    Ciphertext back = Ciphertext::loadSharded(ct);
     EXPECT(back.isSharded() && back.getBlocks() == 5000);
     EXPECT(memcmp(back.getValues(), c.getValues(), c.getLen() * 8) == 0);
     bool threw = false;
-    try { Ciphertext::load("/tmp/csgn_accept.ct.shard0of1"); } catch (const Error &) { threw = true; }
+    try { Ciphertext::load(ct + ".shard0of1"); } catch (const Error &) { threw = true; }
     EXPECT(threw);
-    remove("/tmp/csgn_accept.sk");
-    remove("/tmp/csgn_accept.pm");
-    remove("/tmp/csgn_accept.ct.shard0of1");
+    remove(sk.c_str());
+    remove(pm.c_str());
+    remove((ct + ".shard0of1").c_str());
 }
 
 static void misuse_is_loud() {
@@ -408,6 +434,7 @@ int main() {
     Library::setFusedProducts(true);
     Library::setAutoLanes(true);
     misuse_is_loud();
+    if (!scratch.empty()) rmdir(scratch.c_str());
     if (failures) {
         std::cerr << failures << " expectation(s) failed" << endl;
         return 1;

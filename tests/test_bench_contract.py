@@ -34,15 +34,20 @@ def test_reference_arm_line():
     assert d["gpu_launches"] == 0 and d["config"]["workload"].startswith("cfg2")
 
 
-def test_bench_numpy_restatement_matches_the_oracle():
-    """bench.py checks the GPU with its OWN numpy restatement (precheck, host-known truth); that restatement is pinned
-    to the oracle here, on CPU, for three contexts incl. odd L."""
+def _bench_module():
     import importlib.util
-    import numpy as np
-    from oracle.pyoracle import Oracle, random_blocks, random_key
     spec = importlib.util.spec_from_file_location("bench_module", os.path.join(ROOT, "bench.py"))
     bench = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(bench)
+    return bench
+
+
+def test_bench_numpy_restatement_matches_the_oracle():
+    """bench.py checks the GPU with its OWN numpy restatement (precheck, host-known truth); that restatement is pinned
+    to the oracle here, on CPU, for three contexts incl. odd L."""
+    import numpy as np
+    from oracle.pyoracle import Oracle, random_blocks, random_key
+    bench = _bench_module()
     o = Oracle()
     rng = np.random.default_rng(31)
     for N, D in ((1247, 3), (191, 2), (16383, 4), (128, 2)):
@@ -94,3 +99,37 @@ def test_two_pass_mode_line():
     d = _run(["--steps", "3", "--warmup", "3", "--no-cpu-baseline", "--no-extras", "--mode", "two-pass"], 600)
     assert d["config"]["mode"].startswith("two-pass") and d["gpu_launches"] == 3 * 32
     assert set(d["kernels"]) >= {"multiply", "decrypt"} and d["value"] > 5e9
+
+
+@pytest.mark.gpu
+def test_dump_outputs(tmp_path):
+    """--dump-outputs: the counts of the last timed step and a seeded sample of its products, float64, within 64 MB,
+    equal to the numpy restatement on the bench's seeded inputs and identical from run to run.  One timed step: only
+    the first of the two count slots is written, so the dump must take the last step's slot."""
+    import numpy as np
+    P = 2
+    args = ["--steps", "1", "--warmup", "3", "--pairs", str(P), "--no-extras", "--no-cpu-baseline", "--no-e2e"]
+    runs = []
+    for i in range(2):
+        d = _run(args + ["--dump-outputs", str(tmp_path / str(i))], 600)
+        assert d["steps"] == 1 and d["gpu_launches"] == P
+        runs.append({p.name: np.load(p) for p in (tmp_path / str(i)).iterdir()})
+    out = runs[0]
+    assert set(out) == {"counts.npy", "product_blocks.npy", "product_words.npy"}
+    assert set(runs[1]) == set(out) and all(np.array_equal(out[k], runs[1][k]) for k in out)
+    assert all(a.dtype == np.float64 for a in out.values()) and sum(a.nbytes for a in out.values()) <= 64 << 20
+    bench = _bench_module()
+    N, D, T1, T2, _ = bench.WORKLOADS["cfg2"]
+    L = bench.words_per_block(N)
+    mask = bench.np_key_mask(N, np.random.default_rng(7).permutation(N)[:D])
+    halves = out["product_words.npy"].astype(np.uint64)
+    words = (halves[..., 0] << np.uint64(32)) | halves[..., 1]
+    blocks = out["product_blocks.npy"].astype(np.int64)
+    assert words.shape == (blocks.size, L) and blocks.size > 1000
+    for p in range(P):
+        a = bench.planted_blocks(np.random.default_rng([1000 + p, 0]), T1, N, mask).reshape(T1, L)
+        b = bench.planted_blocks(np.random.default_rng([2000 + p]), T2, N, mask).reshape(T2, L)
+        assert out["counts.npy"][p] == bench.np_count(a, L, mask) * bench.np_count(b, L, mask)
+        mine = blocks // (T1 * T2) == p
+        ij = blocks[mine] % (T1 * T2)
+        assert mine.any() and np.array_equal(words[mine], a[ij // T2] & b[ij % T2])

@@ -4,12 +4,15 @@ CPU: the library exists in-tree, exports the reference's public class API and re
 the C ABI it sits on.  GPU: the acceptance program, the one-process differential run
 against the unmodified reference, and the reference's own demo programs compiled
 UNMODIFIED against our headers all run on the B200."""
+import json
 import os
 import re
 import subprocess
 
+import numpy as np
 import pytest
 
+from conftest import sha, unhex
 from csgn_b200 import build
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -19,6 +22,65 @@ DEMOS = os.path.join(ROOT, "build", "dropin", "bin")
 
 def _run(path, timeout=600):
     return subprocess.run([path], stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=timeout)
+
+
+def _ref_built():
+    return os.path.exists(os.path.join(ROOT, "oracle", "_ref", "libcertfhe_ref.so"))
+
+
+def _stored_cases():
+    """The reference's outputs on the golden cases (tests/golden/make_golden.py)."""
+    with open(os.path.join(ROOT, "tests", "golden", "csgn_golden.json")) as f:
+        return json.load(f)["cases"]
+
+
+def _dropin_on_stored_inputs(exe, mode, cases, env=None):
+    """tests/cpp/dropin_golden.cpp on the stored cases' inputs: {observable: printed value} per case."""
+    lines = [str(len(cases))] + [" ".join(str(x) for x in [c["N"], c["D"], c["seed"], len(c["bits_a"]), len(c["bits_b"])]
+                                          + c["bits_a"] + c["bits_b"] + c["key"]) for c in cases]
+    r = subprocess.run([exe, mode], input="\n".join(lines) + "\n", stdout=subprocess.PIPE, stderr=subprocess.STDOUT,
+                       text=True, timeout=600, env=env)
+    assert r.returncode == 0, r.stdout[-3000:]
+    out = []
+    for line in r.stdout.splitlines():
+        name, _, rest = line.partition(" ")
+        if name == "case":
+            out.append({})
+        elif out:
+            out[-1][name] = rest
+    assert len(out) == len(cases), r.stdout[-3000:]
+    return out, r.stdout
+
+
+def _check_host_side(c, o):
+    nums = lambda s: np.array([int(x) for x in s.split()], dtype=np.uint64)
+    assert [int(x) for x in o["context"].split()] == c["context"] and int(o["sk_size"]) == c["sk_size"]
+    perm = nums(o["perm"])
+    assert sha(perm) == c["perm_sha256"] and [int(x) for x in perm[:16]] == c["perm_head"]
+    if "perm" in c:
+        assert [int(x) for x in perm] == c["perm"]
+    assert sha(nums(o["perm_inverse"])) == c["perm_inverse_sha256"]
+    assert np.array_equal(nums(o["perm_compose"]), np.arange(c["N"], dtype=np.uint64)) == c["perm_compose_is_identity"]
+    assert [int(x) for x in o["permuted_key"].split()] == c["permuted_key"]
+
+
+def _check_evaluation(c, o):
+    L = c["L"]
+    assert o["enc_a"] == c["enc_a"] and o["enc_b"] == c["enc_b"]        # encryption in the reference's rand() order
+    prod, summ = unhex(o["mul"]), unhex(o["add"])
+    assert prod.size == c["mul_len"] and sha(prod) == c["mul_sha256"] and sha(unhex(o["mul_bitlen"])) == c["mul_bitlen_sha256"]
+    assert np.array_equal(prod[:2 * L], unhex(c["mul_head"])) and np.array_equal(prod[-L:], unhex(c["mul_tail"]))
+    if "mul" in c:
+        assert o["mul"] == c["mul"]
+    assert summ.size == c["add_len"] and sha(summ) == c["add_sha256"] and sha(unhex(o["add_bitlen"])) == c["add_bitlen_sha256"]
+    assert [int(x) for x in o["dec"].split()] == [c["dec_a"], c["dec_b"], c["dec_mul"], c["dec_add"]]
+    strict_bl = [int(x) for x in o["permute_strict_bitlen"].split()]
+    assert len(strict_bl) == c["permute_strict_len"] and o["permute_strict"] == c["permute_strict"]
+    assert strict_bl == c["permute_strict_bitlen"] if L <= 32 else sha(np.array(strict_bl, dtype=np.uint64)) == c["permute_strict_bitlen"]
+    assert sha(unhex(o["permute_each_block"])) == c["permute_each_block_sha256"]
+    if "permute_each_block" in c:
+        assert o["permute_each_block"] == c["permute_each_block"]
+    assert int(o["dec_permuted"]) == c["dec_permuted"] and int(o["ct_size_one_block"]) == c["ct_size_one_block"]
 
 
 def test_libcertfhe_exports_the_reference_api():
@@ -69,10 +131,14 @@ def test_cpp_test_programs_are_built():
 
 
 def test_host_side_classes_match_the_reference_without_a_gpu():
-    """Context / Plaintext / Permutation / SecretKey host logic, one process with the unmodified reference."""
+    """Context / Plaintext / Permutation / SecretKey host logic, one process with the unmodified reference; where that
+    build is absent, the same classes on the stored reference cases against the reference's stored outputs."""
     exe = os.path.join(BIN, "host_vs_reference")
-    if not os.path.exists(exe) or not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "libcertfhe_ref.so")):
-        pytest.skip("host_vs_reference is built only where /root/reference was present")
+    if not os.path.exists(exe) or not _ref_built():
+        cases = _stored_cases()
+        for c, o in zip(cases, _dropin_on_stored_inputs(os.path.join(BIN, "dropin_golden"), "host", cases)[0]):
+            _check_host_side(c, o)
+        return
     r = _run(exe)
     assert r.returncode == 0, r.stdout[-4000:]
     assert "host-side classes identical to the reference" in r.stdout
@@ -92,9 +158,15 @@ def test_acceptance_program():
 
 @pytest.mark.gpu
 def test_differential_against_the_unmodified_reference():
+    """The drop-in and the unmodified reference in one process; where that build is absent, every observable of the
+    drop-in on the stored reference cases against the reference's stored outputs."""
     exe = os.path.join(BIN, "diff_vs_reference")
-    if not os.path.exists(exe) or not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "libcertfhe_ref.so")):
-        pytest.skip("diff_vs_reference is built only where /root/reference was present")
+    if not os.path.exists(exe) or not _ref_built():
+        cases = _stored_cases()
+        for c, o in zip(cases, _dropin_on_stored_inputs(os.path.join(BIN, "dropin_golden"), "all", cases)[0]):
+            _check_host_side(c, o)
+            _check_evaluation(c, o)
+        return
     r = _run(exe, timeout=1200)
     assert r.returncode == 0, r.stdout[-4000:]
     assert "identical to the reference on every observable" in r.stdout
@@ -150,12 +222,27 @@ def test_cpp_api_sharded_over_the_gpus_of_the_box(tmp_path):
 def test_host_classes_clean_under_sanitizers(tmp_path):
     """The host-side classes (Context, Plaintext, Permutation, SecretKey key handling, encrypt, Timer, Helper) built with
     -fsanitize=address,undefined and driven by the differential program: no report, same verdict (SURVEY.md 5: the
-    reference itself trips ASan/UBSan in several places -- App. B; this port must not).  CPU only; needs the reference's
-    headers to compile, so it runs where /root/reference is present."""
+    reference itself trips ASan/UBSan in several places -- App. B; this port must not).  CPU only.  Where the reference's
+    headers and build are absent, the driver of the stored reference cases (host mode) is built instead and its output
+    checked against the reference's stored outputs."""
     ref_hdr = os.path.join(build.REFERENCE, "src", "certFHE.h")
     ref_lib = os.path.join(ROOT, "oracle", "_ref", "libcertfhe_ref.so")
+    env = dict(os.environ, ASAN_OPTIONS="detect_leaks=0:protect_shadow_gap=0:halt_on_error=1",
+               UBSAN_OPTIONS="halt_on_error=1:print_stacktrace=1")
     if not (os.path.exists(ref_hdr) and os.path.exists(ref_lib)):
-        pytest.skip("needs /root/reference (headers) and oracle/_ref")
+        exe = str(tmp_path / "dropin_golden_asan")
+        cmd = ["g++", "-O1", "-g", "-std=c++11", "-fsanitize=address,undefined", "-fno-omit-frame-pointer", "-w",
+               "-I" + build.CERTFHE, "-I" + build.INCLUDE, "-o", exe, os.path.join(ROOT, "tests", "cpp", "dropin_golden.cpp"),
+               os.path.join(build.CERTFHE, "host_types.cpp"), os.path.join(build.CERTFHE, "device_types.cpp"),
+               "-L" + build.LIBDIR, "-lcsgn", "-Wl,-rpath," + build.LIBDIR]
+        c = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=600)
+        assert c.returncode == 0, c.stdout[-3000:]
+        cases = _stored_cases()
+        outs, text = _dropin_on_stored_inputs(exe, "host", cases, env=env)
+        assert "AddressSanitizer" not in text and "runtime error" not in text, text[-3000:]
+        for case, o in zip(cases, outs):
+            _check_host_side(case, o)
+        return
     exe = str(tmp_path / "host_vs_reference_asan")
     cmd = ["g++", "-O1", "-g", "-std=c++11", "-fsanitize=address,undefined", "-fno-omit-frame-pointer", "-w",
            "-I" + build.CERTFHE, "-I" + build.INCLUDE, '-DCSGN_REFERENCE_HEADER="%s"' % ref_hdr, "-o", exe,
@@ -165,8 +252,6 @@ def test_host_classes_clean_under_sanitizers(tmp_path):
            "-Wl,-rpath," + build.LIBDIR, "-Wl,-rpath," + os.path.dirname(ref_lib)]
     c = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=600)
     assert c.returncode == 0, c.stdout[-3000:]
-    env = dict(os.environ, ASAN_OPTIONS="detect_leaks=0:protect_shadow_gap=0:halt_on_error=1",
-               UBSAN_OPTIONS="halt_on_error=1:print_stacktrace=1")
     r = subprocess.run([exe], env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=600)
     assert r.returncode == 0, r.stdout[-3000:]
     assert "identical to the reference" in r.stdout

@@ -75,6 +75,12 @@ SIGNATURES = {
     "csgn_decrypt_sharded_batch_async": (ctypes.c_int, [ctypes.POINTER(_vp), ctypes.c_uint32, _vp, _vp, ctypes.c_uint32, _vp]),
     "csgn_decrypt_positions": (ctypes.c_int, [_vp, _u64, _vp, ctypes.c_uint32, ctypes.POINTER(ctypes.c_uint8)]),
     "csgn_encrypt_batch": (ctypes.c_int, [_vp, _vp, _u64, _u64, _u64, _vpp]),
+    "csgn_seg_mul": (ctypes.c_int, [_vp, _vp, _vp, _vp, _u64, _vp, _vpp]),
+    "csgn_seg_concat": (ctypes.c_int, [_vp, _vp, _vp, _vp, _u64, _vp, _vpp]),
+    "csgn_seg_gather": (ctypes.c_int, [_vp, _vp, _u64, _vp, _u64, _vp, _vpp]),
+    "csgn_concat_n": (ctypes.c_int, [ctypes.POINTER(_vp), _u64, _vpp]),
+    "csgn_seg_decrypt_count_async": (ctypes.c_int, [_vp, _vp, _u64, _vp, _vp]),
+    "csgn_seg_decrypt": (ctypes.c_int, [_vp, _vp, _u64, _vp, _vp, _vp]),
     "csgn_perm_create": (ctypes.c_int, [_u64, _vp, _vpp]),
     "csgn_perm_free": (ctypes.c_int, [_vp]),
     "csgn_permute": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vpp]),

@@ -1,0 +1,127 @@
+// array_types.cpp -- CiphertextArray and the array members of SecretKey over the C ABI's ciphertext arrays
+// (include/csgn.h): each operation is ONE call, which makes one kernel launch for all small elements.
+//   CiphertextArray(vector)   -> csgn_concat_n
+//   operator* / operator+     -> csgn_seg_mul / csgn_seg_concat
+//   gather                    -> csgn_seg_gather
+//   applyPermutation          -> csgn_permute on the storage (a permutation acts on every block by itself)
+//   encryptArray / decryptArray -> csgn_encrypt_batch / csgn_seg_decrypt
+#include "certFHE.h"
+#include "engine_glue.h"
+
+namespace certFHE {
+
+namespace {
+
+std::shared_ptr<csgn_buf> adopt(csgn_buf *b) {
+    return std::shared_ptr<csgn_buf>(b, [](csgn_buf *p) { csgn_buf_free(p); });
+}
+
+Context first_context(const std::vector<Ciphertext> &elements) {
+    if (elements.empty()) throw Error("CiphertextArray: no elements");
+    return elements[0].getContext();
+}
+
+}  // namespace
+
+CiphertextArray::CiphertextArray(csgn_buf *buf, const std::vector<uint64_t> &off, const Context &ctx)
+    : storage(adopt(buf)), offsets(off), context(ctx) {}
+
+CiphertextArray::CiphertextArray(const std::vector<Ciphertext> &elements) : context(first_context(elements)) {
+    std::vector<const csgn_buf *> parts;
+    offsets.assign(1, 0);
+    for (size_t i = 0; i < elements.size(); ++i) {
+        const Ciphertext &c = elements[i];
+        if (c.isSharded()) throw Error("CiphertextArray: element " + to_string(i) + " is sharded");
+        const csgn_buf *b = c.deviceBuffer();   // writes a pending product; csgn_concat_n makes a lazy sum dense
+        if (b) parts.push_back(b);
+        offsets.push_back(offsets.back() + (b ? csgn_buf_blocks(b) : 0));
+    }
+    if (parts.empty()) throw Error("CiphertextArray: every element is empty");
+    csgn_buf *out = nullptr;
+    glue::check(csgn_concat_n(parts.data(), parts.size(), &out), "csgn_concat_n");
+    storage = adopt(out);
+}
+
+uint64_t CiphertextArray::size() const { return offsets.size() - 1; }
+
+uint64_t CiphertextArray::getBlocks(uint64_t k) const {
+    if (k >= size()) throw Error("CiphertextArray::getBlocks: element " + to_string(k) + " of " + to_string(size()));
+    return offsets[k + 1] - offsets[k];
+}
+
+Ciphertext CiphertextArray::get(uint64_t k) const {
+    const uint64_t n = getBlocks(k);
+    csgn_buf *b = nullptr;
+    glue::check(csgn_buf_slice(storage.get(), offsets[k], n, &b), "csgn_buf_slice");
+    Ciphertext out;
+    out.certFHEcontext = new Context(context);
+    out.dev = adopt(b);
+    return out;
+}
+
+Context CiphertextArray::getContext() const { return context; }
+
+const std::vector<uint64_t> &CiphertextArray::getOffsets() const { return offsets; }
+
+const csgn_buf *CiphertextArray::deviceBuffer() const { return storage.get(); }
+
+CiphertextArray CiphertextArray::operator*(const CiphertextArray &c) const {
+    if (c.size() != size()) throw Error("CiphertextArray::operator*: arrays of " + to_string(size()) + " and " +
+                                        to_string(c.size()) + " elements");
+    std::vector<uint64_t> off(size() + 1);
+    csgn_buf *out = nullptr;
+    glue::check(csgn_seg_mul(storage.get(), offsets.data(), c.storage.get(), c.offsets.data(), size(), off.data(), &out),
+                "csgn_seg_mul");
+    return CiphertextArray(out, off, context);
+}
+
+CiphertextArray CiphertextArray::operator+(const CiphertextArray &c) const {
+    if (c.size() != size()) throw Error("CiphertextArray::operator+: arrays of " + to_string(size()) + " and " +
+                                        to_string(c.size()) + " elements");
+    std::vector<uint64_t> off(size() + 1);
+    csgn_buf *out = nullptr;
+    glue::check(csgn_seg_concat(storage.get(), offsets.data(), c.storage.get(), c.offsets.data(), size(), off.data(),
+                                &out),
+                "csgn_seg_concat");
+    return CiphertextArray(out, off, context);
+}
+
+CiphertextArray CiphertextArray::gather(const std::vector<uint64_t> &idx) const {
+    std::vector<uint64_t> off(idx.size() + 1);
+    csgn_buf *out = nullptr;
+    glue::check(csgn_seg_gather(storage.get(), offsets.data(), size(), idx.data(), idx.size(), off.data(), &out),
+                "csgn_seg_gather");
+    return CiphertextArray(out, off, context);
+}
+
+CiphertextArray CiphertextArray::applyPermutation(const Permutation &permutation) const {
+    csgn_buf *out = nullptr;
+    if (csgn_buf_blocks(storage.get()) == 0)
+        glue::check(csgn_buf_clone(storage.get(), &out), "csgn_buf_clone");
+    else
+        glue::check(csgn_permute(storage.get(), permutation.deviceMap(context.getN()), 0, &out), "csgn_permute");
+    return CiphertextArray(out, offsets, context);
+}
+
+CiphertextArray SecretKey::encryptArray(const unsigned char *bits, uint64_t n, uint64_t seed) {
+    if (!device_key) {
+        glue::ensure_engine();
+        glue::check(csgn_key_create(certFHEContext->getN(), s, (uint32_t)length, &device_key), "csgn_key_create");
+    }
+    csgn_buf *buf = nullptr;
+    glue::check(csgn_encrypt_batch(device_key, bits, n, 0, seed, &buf), "csgn_encrypt_batch");
+    std::vector<uint64_t> off(n + 1);
+    for (uint64_t k = 0; k <= n; ++k) off[k] = k;
+    return CiphertextArray(buf, off, *certFHEContext);
+}
+
+void SecretKey::decryptArray(const CiphertextArray &array, unsigned char *bits) {
+    if (!device_key) {
+        glue::ensure_engine();
+        glue::check(csgn_key_create(certFHEContext->getN(), s, (uint32_t)length, &device_key), "csgn_key_create");
+    }
+    glue::check(csgn_seg_decrypt(array.deviceBuffer(), array.getOffsets().data(), array.size(), device_key, bits, nullptr),
+                "csgn_seg_decrypt");
+}
+
+}  // namespace certFHE

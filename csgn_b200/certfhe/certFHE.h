@@ -33,6 +33,8 @@ struct csgn_result;
 
 namespace certFHE {
 
+class CiphertextArray;
+
 // Raised where the reference would run into undefined behaviour or where the GPU
 // engine reports a failure.  The reference has no error channel at all; an uncaught
 // Error terminates with its message, which is the loud failure we want.
@@ -212,6 +214,7 @@ class Ciphertext {
     void collect_factors(std::vector<std::shared_ptr<csgn_buf> > &into, bool flatten) const;
     bool adopt_written_product() const;  // a copy has already written the pending product: take it
     friend class SecretKey;
+    friend class CiphertextArray;
 
 public:
     Ciphertext();
@@ -284,6 +287,10 @@ public:
     // Extension: decrypt n ciphertexts with ONE synchronisation (csgn_decrypt_batch: the folds are spread over
     // the library's lanes and overlap); bits[i] = decrypt(ciphertexts[i]).getValue().
     void decryptBatch(Ciphertext *ciphertexts, uint64_t n, unsigned char *bits);
+    // Extension: n fresh one-block encryptions as a CiphertextArray of n elements (csgn_encrypt_batch), and the
+    // decryption of every element of an array with one launch and one synchronisation (csgn_seg_decrypt).
+    CiphertextArray encryptArray(const unsigned char *bits, uint64_t n, uint64_t seed);
+    void decryptArray(const CiphertextArray &array, unsigned char *bits);
     void applyPermutation_inplace(const Permutation &permutation);
     SecretKey applyPermutation(const Permutation &permutation);
 
@@ -299,6 +306,38 @@ public:
     // csgn_key_positions_save / _load).  The file holds the secret: protect it like the key.
     void save(const std::string &path) const;
     static SecretKey load(const std::string &path);
+};
+
+// ---- CiphertextArray (extension; include/csgn.h, "ciphertext arrays") ----------------------------------------------
+// n independent ciphertexts -- the encrypted bits of a circuit over encrypted integers, say -- held as ONE device buffer
+// plus block offsets: element k is blocks [offsets[k], offsets[k+1]).  operator*, operator+, gather and
+// applyPermutation act element by element with one kernel launch for all small elements, where a loop over
+// Ciphertext operators costs one launch and its host bookkeeping per element.  Arrays are always evaluated eagerly:
+// the fused, lazy and rope modes of Ciphertext do not apply to them.
+class CiphertextArray {
+    std::shared_ptr<csgn_buf> storage;
+    std::vector<uint64_t> offsets;   // n + 1 block offsets
+    Context context;
+    CiphertextArray(csgn_buf *storage, const std::vector<uint64_t> &offsets, const Context &context);
+    friend class SecretKey;
+
+public:
+    // Packs the ciphertexts into one array with one launch (csgn_concat_n); pending products and lazy sums are
+    // written first.  Sharded ciphertexts are refused.
+    explicit CiphertextArray(const std::vector<Ciphertext> &elements);
+
+    uint64_t size() const;                 // number of elements
+    uint64_t getBlocks(uint64_t k) const;  // blocks of element k
+    Ciphertext get(uint64_t k) const;      // element k as an ordinary Ciphertext (a device copy of its blocks)
+    Context getContext() const;
+
+    CiphertextArray operator*(const CiphertextArray &c) const;   // element k = this_k * c_k
+    CiphertextArray operator+(const CiphertextArray &c) const;   // element k = this_k + c_k
+    CiphertextArray gather(const std::vector<uint64_t> &idx) const;   // element j = this_{idx[j]}
+    CiphertextArray applyPermutation(const Permutation &permutation) const;   // every element permuted
+
+    const std::vector<uint64_t> &getOffsets() const;
+    const csgn_buf *deviceBuffer() const;
 };
 
 // ---- Timer (reference src/Timer.h:13-74) -------------------------------------------------

@@ -627,6 +627,44 @@ void copy_to_staging(void *dst, const void *src, size_t bytes) {
 }
 }  // namespace
 
+}  // extern "C"
+
+namespace csgn {
+namespace detail {
+
+// A small host table (work items, offsets) to fresh device memory on the current stream, through the pinned staging:
+// no host synchronisation, and the caller may reuse its array at once.  Tables beyond the staging limit are copied
+// straight from the caller's memory, and the call waits for that copy.
+int stage_to_device(const void *host, size_t bytes, void **out) {
+    *out = nullptr;
+    if (bytes == 0) return CSGN_OK;
+    uint64_t *d = nullptr;
+    int rc = dev_alloc((bytes + 7) / 8, &d);
+    if (rc != CSGN_OK) return rc;
+    StagingSlot *sl = bytes <= kStagingMaxOne ? take_staging(bytes) : nullptr;
+    cudaError_t e;
+    if (sl) {
+        copy_to_staging(sl->p, host, bytes);
+        e = cudaMemcpyAsync(d, sl->p, bytes, cudaMemcpyHostToDevice, g.stream);
+        cudaEventRecord(sl->done, g.stream);
+    } else {
+        e = cudaMemcpyAsync(d, host, bytes, cudaMemcpyHostToDevice, g.stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(g.stream);
+        if (e == cudaSuccess) note_synced(g.stream);
+    }
+    if (e != cudaSuccess) {
+        dev_free(d);
+        return cuda_fail(e, "table upload");
+    }
+    *out = d;
+    return CSGN_OK;
+}
+
+}  // namespace detail
+}  // namespace csgn
+
+extern "C" {
+
 int csgn_buf_upload_copy(const uint64_t *host_words, uint64_t n_blocks, uint32_t L, csgn_buf **out) {
     NEED_INIT();
     if (L == 0) return fail(CSGN_ERR_INVALID_ARGUMENT, "words per block must be > 0");

@@ -1,5 +1,5 @@
 // capi_internal.cuh -- shared by the translation units that implement include/csgn.h (capi.cu: library, buffers,
-// the hot path, batches; capi_comm.cu: the peer communicator; capi_io.cu: save / load): the handle types, the
+// the hot path, batches; capi_comm.cu: the peer communicator; capi_io.cu: save / load; capi_seg.cu: ciphertext arrays): the handle types, the
 // process-wide state and the small helpers every entry point uses.  Internal: not part of the C ABI.
 #pragma once
 
@@ -190,6 +190,10 @@ inline bool is_rope(const csgn_buf *b) { return b && !b->segs.empty(); }
 uint64_t *fold_scratch();
 // True inside a batch call or with automatic lanes: folds run next to other kernels (several shorter waves).
 bool folds_overlap();
+
+// Copy a host table of `bytes` bytes to fresh device memory (dev_alloc) on the current stream through the library's
+// pinned staging, without a host synchronisation; the caller frees it with dev_free after the launches that read it.
+int stage_to_device(const void *host, size_t bytes, void **out);
 
 // Scope of one batch call: item i runs with the work stream set to way i % n, where way 0 is the caller's own stream
 // and ways 1.. are the library's side lanes, forked from the caller's stream on construction; join() makes the

@@ -48,6 +48,31 @@ bool mul_fold_supported(uint32_t L);
 cudaError_t launch_concat(const uint64_t *a, uint64_t n_words_a, const uint64_t *b, uint64_t n_words_b,
                           uint64_t *out, cudaStream_t stream);
 
+// Piece-table copy (ciphertext arrays: element-wise concat, gather, pack): destination units [dst[p], dst[p+1]) come
+// from src[p], p < n_pieces; src and dst are device arrays, dst[n_pieces] == total_units.  Units of 16 bytes
+// (units16: every source, the destination and every piece 16-byte granular) or 8 bytes.  One launch.
+cudaError_t launch_piece_copy(const void *const *src, const uint64_t *dst, uint32_t n_pieces, uint64_t total_units,
+                              bool units16, void *out, cudaStream_t stream);
+
+// Ciphertext arrays (segments.cu).  Grouped multiply: work item k multiplies rows [a, a + rows) of its left operand
+// by the t2 blocks starting at block b of the right operand, into the rows*t2 blocks at block `out` of the output
+// (all in blocks of L words); a warp task is a run of consecutive items [task[t], task[t+1]).  One launch.
+struct SegMulItem {
+    uint64_t a, b, out;
+    uint32_t t2, rows;
+};
+cudaError_t launch_seg_mul(const uint64_t *a, const uint64_t *b, uint64_t *out, uint32_t L, const SegMulItem *items,
+                           const uint32_t *tasks, uint32_t n_tasks, cudaStream_t stream);
+// Segmented decrypt: a warp task walks blocks [first, end), which belong to elements [elem, elem_last] (element e =
+// blocks [off[e], off[e+1]), off on the device), and adds each element's satisfied-block count to counts[e] (zeroed
+// by the caller in stream order).  One launch.
+struct SegDecTask {
+    uint64_t first, end;
+    uint64_t elem, elem_last;
+};
+cudaError_t launch_seg_decrypt(const uint64_t *v, uint32_t L, const uint64_t *mask, const uint64_t *off,
+                               const SegDecTask *tasks, uint32_t n_tasks, uint64_t *counts, cudaStream_t stream);
+
 // out[0] = sum of in[0..n): the partial counts of a ciphertext held as several segments (a lazy sum)
 cudaError_t launch_sum_words(const uint64_t *in, uint32_t n, uint64_t *out, cudaStream_t stream);
 

@@ -1,0 +1,161 @@
+// segments.cu -- kernels of ciphertext arrays: many independent small ciphertexts held in ONE buffer, element k being
+// blocks [off[k], off[k+1]) (include/csgn.h, "ciphertext arrays").  Each kernel serves any number of elements in one
+// launch; the host (capi_seg.cu) builds the work tables from the offsets, so no kernel searches or divides per unit.
+//
+//   grouped multiply   element k = a_k * b_k, all-pairs AND, i-major      (reference src/Ciphertext.cpp:153-163)
+//   segmented decrypt  counts[k] = satisfied blocks of element k           (reference src/SecretKey.cpp:126-140)
+//
+// (the element-wise concat / gather / pack copy is misc.cu's streaming copy over a piece table.)
+//
+// Units are 16 bytes (uint4) when L is even and the storage is 16-byte aligned, 8 bytes otherwise.  A warp handles a
+// block of U units with min(U, 32) lanes: for U < 32 one warp step covers 32/U (multiply) or 32/G (decrypt, G the
+// power of two >= U) whole blocks, for U >= 32 the lanes walk the block in steps of 32 units.
+#include "kernels.cuh"
+#include "launch.cuh"
+#include "fold.cuh"
+
+#include <algorithm>
+
+namespace csgn {
+namespace {
+
+constexpr int kSegThreads = 256;
+constexpr int kSegCtasPerSm = 8;
+
+__device__ __forceinline__ uint4 vand(const uint4 x, const uint4 y) {
+    return make_uint4(x.x & y.x, x.y & y.y, x.z & y.z, x.w & y.w);
+}
+__device__ __forceinline__ uint2 vand(const uint2 x, const uint2 y) { return make_uint2(x.x & y.x, x.y & y.y); }
+
+// ---------------------------------------------------------------------------------------
+// grouped multiply: a warp task is a run of items; an item is rows [a, a+rows) of one element's left operand times
+// the t2 blocks of its right operand at b, written to block `out` on.  Lane l holds unit w = l % U of block
+// j = l / U of each warp step (U < 32), or units l, l+32, ... of one block (U >= 32).
+// ---------------------------------------------------------------------------------------
+template <typename VT>
+__global__ void __launch_bounds__(kSegThreads)
+seg_mul_kernel(const VT *__restrict__ a, const VT *__restrict__ b, VT *__restrict__ out, const uint32_t U,
+               const SegMulItem *__restrict__ items, const uint32_t *__restrict__ tasks, const uint32_t n_tasks) {
+    const uint32_t lane = threadIdx.x & 31u;
+    const uint32_t G = U >= 32u ? 1u : 32u / U;                // blocks per warp step
+    const uint32_t w0 = U >= 32u ? lane : lane % U;
+    const uint32_t j0 = U >= 32u ? 0u : lane / U;
+    const uint32_t warps = gridDim.x * (blockDim.x >> 5);
+    pdl_enter();
+    if (j0 >= G) return;                                       // lanes beyond the last whole block of a step
+    for (uint32_t t = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); t < n_tasks; t += warps) {
+        const uint32_t it_end = __ldg(tasks + t + 1);
+        for (uint32_t it = __ldg(tasks + t); it < it_end; ++it) {
+            const SegMulItem m = items[it];
+            for (uint32_t r = 0; r < m.rows; ++r) {
+                const VT *arow = a + (m.a + r) * U;
+                VT *orow = out + (m.out + (uint64_t)r * m.t2) * U;
+                if (U < 32u) {
+                    const VT x = __ldg(arow + w0);
+#pragma unroll 4
+                    for (uint32_t j = j0; j < m.t2; j += G)
+                        __stcs(orow + (uint64_t)j * U + w0, vand(x, __ldg(b + (m.b + j) * U + w0)));
+                } else {
+                    for (uint32_t j = 0; j < m.t2; ++j) {
+                        const VT *brow = b + (m.b + j) * U;
+                        VT *o = orow + (uint64_t)j * U;
+#pragma unroll 4
+                        for (uint32_t w = w0; w < U; w += 32u) __stcs(o + w, vand(__ldg(arow + w), __ldg(brow + w)));
+                    }
+                }
+            }
+        }
+    }
+}
+
+// ---------------------------------------------------------------------------------------
+// segmented decrypt: groups of G lanes (G a power of two, >= U up to 32) evaluate one block each per warp step; the
+// group's verdict is one ballot.  Group leaders that hold the same element find each other with match.any and add
+// their verdicts with one more ballot: one atomic per (warp step, element), not one per block.
+// ---------------------------------------------------------------------------------------
+template <typename VT>
+__global__ void __launch_bounds__(kSegThreads)
+seg_decrypt_kernel(const VT *__restrict__ v, const uint32_t U, const uint32_t log2g, const VT *__restrict__ mask,
+                   const uint64_t *__restrict__ off, const SegDecTask *__restrict__ tasks, const uint32_t n_tasks,
+                   uint64_t *counts) {
+    const uint32_t lane = threadIdx.x & 31u;
+    const uint32_t G = 1u << log2g, sub = lane & (G - 1u), grp = lane >> log2g, B = 32u >> log2g;
+    const uint32_t gmask = G == 32u ? 0xffffffffu : ((1u << G) - 1u) << (grp * G);
+    const uint32_t warps = gridDim.x * (blockDim.x >> 5);
+    pdl_enter();
+    for (uint32_t t = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); t < n_tasks; t += warps) {
+        const SegDecTask task = tasks[t];
+        uint64_t e = task.elem;                                // element of this lane's block: never decreases
+        for (uint64_t blk0 = task.first; blk0 < task.end; blk0 += B) {
+            const uint64_t blk = blk0 + grp;
+            const bool live = blk < task.end;
+            bool fails = false;
+            if (live) {
+                const VT *p = v + blk * U;
+                for (uint32_t w = sub; w < U; w += G) fails |= unit_fails(__ldcs(p + w), __ldg(mask + w));
+            }
+            // the vote is taken by every lane (a `live && ballot` would skip it on lanes past the task's end)
+            const uint32_t vote = __ballot_sync(0xffffffffu, fails);
+            const bool sat = live && (vote & gmask) == 0u;
+            const bool leader = live && sub == 0u;
+            if (leader) {                                      // last e in [e, elem_last] with off[e] <= blk
+                uint64_t lo = e, hi = task.elem_last;
+                while (lo < hi) {
+                    const uint64_t mid = lo + ((hi - lo + 1) >> 1);
+                    if (__ldg(off + mid) <= blk) lo = mid;
+                    else hi = mid - 1;
+                }
+                e = lo;
+            }
+            // Every lane executes both warp-wide votes with the full mask; a group's sum is the popcount of the
+            // satisfied leaders among its peers (verdicts are 0 / 1), so no reduction runs over a partial mask.
+            const uint64_t key = leader ? e : ~0ull;
+            const uint32_t peers = __match_any_sync(0xffffffffu, key);
+            const uint32_t sum = __popc(peers & __ballot_sync(0xffffffffu, leader && sat));
+            if (leader && sum && lane == (uint32_t)(__ffs(peers) - 1))
+                atomicAdd(reinterpret_cast<unsigned long long *>(counts + e), (unsigned long long)sum);
+        }
+    }
+}
+
+uint32_t seg_grid(uint32_t n_tasks) {
+    const uint32_t warps_per_cta = kSegThreads / 32;
+    const uint64_t want = ((uint64_t)n_tasks + warps_per_cta - 1) / warps_per_cta;
+    return (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(want, (uint64_t)device_props().sm_count * kSegCtasPerSm));
+}
+
+}  // namespace
+
+cudaError_t launch_seg_mul(const uint64_t *a, const uint64_t *b, uint64_t *out, uint32_t L, const SegMulItem *items,
+                           const uint32_t *tasks, uint32_t n_tasks, cudaStream_t stream) {
+    if (n_tasks == 0) return cudaSuccess;
+    const bool units16 = !(L & 1u) && ((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b) |
+                                        reinterpret_cast<uintptr_t>(out)) & 15u) == 0;
+    count_launch();
+    if (units16)
+        return launch_kernel(seg_mul_kernel<uint4>, seg_grid(n_tasks), kSegThreads, 0, stream,
+                             reinterpret_cast<const uint4 *>(a), reinterpret_cast<const uint4 *>(b),
+                             reinterpret_cast<uint4 *>(out), L / 2, items, tasks, n_tasks);
+    return launch_kernel(seg_mul_kernel<uint2>, seg_grid(n_tasks), kSegThreads, 0, stream,
+                         reinterpret_cast<const uint2 *>(a), reinterpret_cast<const uint2 *>(b),
+                         reinterpret_cast<uint2 *>(out), L, items, tasks, n_tasks);
+}
+
+cudaError_t launch_seg_decrypt(const uint64_t *v, uint32_t L, const uint64_t *mask, const uint64_t *off,
+                               const SegDecTask *tasks, uint32_t n_tasks, uint64_t *counts, cudaStream_t stream) {
+    if (n_tasks == 0) return cudaSuccess;
+    const bool units16 = !(L & 1u) && ((reinterpret_cast<uintptr_t>(v) | reinterpret_cast<uintptr_t>(mask)) & 15u) == 0;
+    const uint32_t U = units16 ? L / 2 : L;
+    uint32_t log2g = 0;
+    while (log2g < 5 && (1u << log2g) < U) ++log2g;
+    count_launch();
+    if (units16)
+        return launch_kernel(seg_decrypt_kernel<uint4>, seg_grid(n_tasks), kSegThreads, 0, stream,
+                             reinterpret_cast<const uint4 *>(v), U, log2g, reinterpret_cast<const uint4 *>(mask), off,
+                             tasks, n_tasks, counts);
+    return launch_kernel(seg_decrypt_kernel<uint2>, seg_grid(n_tasks), kSegThreads, 0, stream,
+                         reinterpret_cast<const uint2 *>(v), U, log2g, reinterpret_cast<const uint2 *>(mask), off, tasks,
+                         n_tasks, counts);
+}
+
+}  // namespace csgn

@@ -361,6 +361,101 @@ def mul_count_batch_async(key, a, b, device_counts_ptr, out=None, arrays=None):
     return None
 
 
+def _offsets(off):
+    o = np.ascontiguousarray(np.asarray(off, dtype=np.uint64).reshape(-1))
+    if o.size == 0:
+        raise ValueError("offsets need n + 1 entries")
+    return o
+
+
+class CiphertextArray:
+    """n independent ciphertexts as ONE device buffer (`storage`, a Ciphertext) plus numpy block offsets: element k is
+    blocks [offsets[k], offsets[k+1]) (include/csgn.h, "ciphertext arrays").  Element-wise *, + and gather are one
+    library call each, with one kernel launch for all small elements."""
+
+    def __init__(self, storage, offsets):
+        self.storage = storage
+        self.offsets = _offsets(offsets)
+        self.ctx = storage.ctx
+
+    # -- construction -----------------------------------------------------
+    @classmethod
+    def from_host(cls, elements, ctx):
+        """One upload of the host word arrays `elements` (each a multiple of ctx.L words)."""
+        words = [_host_words(e) for e in elements]
+        if any(w.size % ctx.L for w in words):
+            raise ValueError("every element needs a multiple of the %d words per block" % ctx.L)
+        off = np.zeros(len(words) + 1, dtype=np.uint64)
+        off[1:] = np.cumsum([w.size // ctx.L for w in words], dtype=np.uint64)
+        flat = np.concatenate(words) if words else np.empty(0, dtype=np.uint64)
+        return cls(Ciphertext.from_host(flat, ctx), off)
+
+    @classmethod
+    def pack(cls, cts):
+        """csgn_concat_n: the ciphertexts `cts` packed into one array in one launch."""
+        if not cts:
+            raise ValueError("pack needs at least one ciphertext")
+        h = _vp()
+        check(_lib().csgn_concat_n(handle_array(cts), len(cts), ctypes.byref(h)))
+        off = np.zeros(len(cts) + 1, dtype=np.uint64)
+        off[1:] = np.cumsum([c.n_blocks for c in cts], dtype=np.uint64)
+        return cls(Ciphertext(h, cts[0].ctx), off)
+
+    # -- access -------------------------------------------------------------
+    def __len__(self):
+        return self.offsets.size - 1
+
+    def blocks(self, k):
+        return int(self.offsets[k + 1] - self.offsets[k])
+
+    def element(self, k):
+        """Element k as an ordinary Ciphertext (a device copy of its blocks, csgn_buf_slice)."""
+        if not 0 <= k < len(self):
+            raise IndexError(k)
+        h = _vp()
+        check(_lib().csgn_buf_slice(self.storage._h, int(self.offsets[k]), self.blocks(k), ctypes.byref(h)))
+        return Ciphertext(h, self.ctx)
+
+    def to_host(self):
+        """The words of every element, as a list of numpy arrays."""
+        w = self.storage.getValues()
+        L = self.ctx.L
+        return [w[int(self.offsets[k]) * L:int(self.offsets[k + 1]) * L] for k in range(len(self))]
+
+    # -- element-wise operations --------------------------------------------
+    def _binary(self, fn, other):
+        if len(other) != len(self):
+            raise ValueError("arrays of %d and %d elements" % (len(self), len(other)))
+        out_off = np.empty(len(self) + 1, dtype=np.uint64)
+        h = _vp()
+        check(fn(self.storage._h, self.offsets.ctypes.data_as(_vp), other.storage._h, other.offsets.ctypes.data_as(_vp),
+                 len(self), out_off.ctypes.data_as(_vp), ctypes.byref(h)))
+        return CiphertextArray(Ciphertext(h, self.ctx), out_off)
+
+    def __mul__(self, other):
+        """csgn_seg_mul: element k = self_k * other_k."""
+        return self._binary(_lib().csgn_seg_mul, other)
+
+    def __add__(self, other):
+        """csgn_seg_concat: element k = self_k + other_k (block concatenation, the homomorphic XOR)."""
+        return self._binary(_lib().csgn_seg_concat, other)
+
+    def gather(self, idx):
+        """csgn_seg_gather: element j = self_{idx[j]} (any order, repeats allowed)."""
+        ix = np.ascontiguousarray(np.asarray(idx, dtype=np.uint64).reshape(-1))
+        out_off = np.empty(ix.size + 1, dtype=np.uint64)
+        h = _vp()
+        check(_lib().csgn_seg_gather(self.storage._h, self.offsets.ctypes.data_as(_vp), len(self), ix.ctypes.data_as(_vp),
+                                     ix.size, out_off.ctypes.data_as(_vp), ctypes.byref(h)))
+        return CiphertextArray(Ciphertext(h, self.ctx), out_off)
+
+    def applyPermutation(self, perm):
+        """Every element permuted (csgn_permute on the storage; the offsets do not change)."""
+        if self.storage.n_blocks == 0:
+            return CiphertextArray(self.storage.clone(), self.offsets.copy())
+        return CiphertextArray(self.storage.applyPermutation(perm), self.offsets.copy())
+
+
 class Result:
     """A decrypt whose count the host reads later (csgn_result)."""
 
@@ -459,6 +554,24 @@ class SecretKey:
         h = _vp()
         check(_lib().csgn_encrypt_batch(self._h, b.ctypes.data_as(_vp), b.size, int(first_block), int(seed), ctypes.byref(h)))
         return Ciphertext(h, self.ctx)
+
+    def encrypt_array(self, bits, seed, first_block=0):
+        """CiphertextArray of len(bits) one-block encryptions (csgn_encrypt_batch, offsets 0, 1, ..., n)."""
+        n = np.asarray(bits).size
+        return CiphertextArray(self.encrypt_batch(bits, seed, first_block), np.arange(n + 1, dtype=np.uint64))
+
+    def decrypt_array_count_async(self, arr, device_counts_ptr):
+        """csgn_seg_decrypt_count_async: device_counts[k] = satisfied blocks of element k, no synchronisation."""
+        check(_lib().csgn_seg_decrypt_count_async(arr.storage._h, arr.offsets.ctypes.data_as(_vp), len(arr), self._h,
+                                                  _vp(device_counts_ptr)))
+
+    def decrypt_array(self, arr):
+        """csgn_seg_decrypt: (bits, counts) of every element as numpy arrays, one synchronisation."""
+        n = len(arr)
+        bits, counts = np.zeros(n, dtype=np.uint8), np.zeros(n, dtype=np.uint64)
+        check(_lib().csgn_seg_decrypt(arr.storage._h, arr.offsets.ctypes.data_as(_vp), n, self._h,
+                                      bits.ctypes.data_as(_vp), counts.ctypes.data_as(_vp)))
+        return bits, counts
 
     def decrypt_product(self, factors):
         """Dec(f1*f2*...*fn) without materialising the product (csgn_decrypt_product).

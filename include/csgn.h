@@ -233,6 +233,39 @@ int csgn_decrypt_positions(const csgn_buf *c, uint64_t N, const uint64_t *positi
 int csgn_encrypt_batch(const csgn_key *key, const uint8_t *bits, uint64_t n, uint64_t first_block, uint64_t seed,
                        csgn_buf **out);
 
+/* ---- ciphertext arrays ---------------------------------------------------------------------------------------
+ * A plaintext is one bit, so a circuit over encrypted integers holds thousands of small, independent ciphertexts.  A
+ * ciphertext array of n elements is an ordinary dense csgn_buf (the elements' blocks one after another) plus a host
+ * array off[n+1] of uint64 BLOCK offsets: element k is blocks [off[k], off[k+1]) (empty elements allowed).  Every
+ * existing call works on the storage: csgn_permute permutes every element (offsets unchanged), csgn_buf_slice /
+ * csgn_buf_download_range read one element, and the n-block result of csgn_encrypt_batch is an array of n one-block
+ * encryptions with off = 0, 1, ..., n.
+ * Offsets are checked on the host on every call (off[0] == 0, non-decreasing, off[n] == csgn_buf_blocks(buf);
+ * CSGN_ERR_INVALID_ARGUMENT or CSGN_ERR_SHAPE_MISMATCH, nothing allocated) and copied to the device by the library
+ * through its pinned staging, without a host synchronisation: the caller may free its arrays when the call returns.
+ * Output arrays are allocated by the library; their offsets go to the caller's out_off[n+1] (m+1 for a gather).
+ * All small elements are served by ONE kernel launch per call; elements whose product (multiply) or whose blocks
+ * (decrypt) reach 8 MB run on the single-ciphertext kernels, one launch each, straight into the output.  Ordering,
+ * streams and automatic lanes are those of the single-ciphertext entry points. */
+/* element k = a_k * b_k (src/Ciphertext.cpp:153-163): T1_k*T2_k blocks, i-major; empty if either operand is empty. */
+int csgn_seg_mul(const csgn_buf *a, const uint64_t *a_off, const csgn_buf *b, const uint64_t *b_off, uint64_t n,
+                 uint64_t *out_off, csgn_buf **out);
+/* element k = a_k || b_k (src/Ciphertext.cpp:107-122): the element-wise homomorphic XOR. */
+int csgn_seg_concat(const csgn_buf *a, const uint64_t *a_off, const csgn_buf *b, const uint64_t *b_off, uint64_t n,
+                    uint64_t *out_off, csgn_buf **out);
+/* element j = src_{idx[j]}, j < m: any order, repeats allowed; idx[j] < n_src is checked. */
+int csgn_seg_gather(const csgn_buf *src, const uint64_t *src_off, uint64_t n_src, const uint64_t *idx, uint64_t m,
+                    uint64_t *out_off, csgn_buf **out);
+/* parts[0] || ... || parts[n-1] in one launch: n separate ciphertexts packed into an array (its offsets are the
+ * prefix sums of the parts' block counts). */
+int csgn_concat_n(const csgn_buf *const *parts, uint64_t n, csgn_buf **out);
+/* device_counts[k] = satisfied blocks of element k (0 for an empty one); no host synchronisation. */
+int csgn_seg_decrypt_count_async(const csgn_buf *c, const uint64_t *c_off, uint64_t n, const csgn_key *key,
+                                 uint64_t *device_counts);
+/* SecretKey::decrypt of every element with one synchronisation: bits[k] = count_k & 1 and/or counts[k]. */
+int csgn_seg_decrypt(const csgn_buf *c, const uint64_t *c_off, uint64_t n, const csgn_key *key, uint8_t *bits,
+                     uint64_t *counts);
+
 /* Permutation as a device source map: out_bit[i] = in_bit[perm[i]], i < N
  * (src/Ciphertext.cpp:33-34).  Fails unless perm is a bijection of [0,N). */
 int csgn_perm_create(uint64_t N, const uint64_t *perm, csgn_perm **out);

@@ -1,0 +1,282 @@
+"""Ciphertext arrays against per-ciphertext calls, on one GPU, in one run (include/csgn.h, "ciphertext arrays").
+
+  small   n one-block products and decrypts at Context(1247,16): csgn_seg_mul / csgn_seg_decrypt against
+          csgn_mul_batch / csgn_decrypt_batch on n handles -- time and kernel launches per call
+  mixed   operand elements of 1-64 blocks (log-uniform), >= 1 GB of product: write rate of csgn_seg_mul next to csgn_mul of
+          one product of the same size, read rate of csgn_seg_decrypt next to csgn_decrypt_count on the same storage,
+          both as a fraction of a device-to-device copy (torch) of the same bytes measured in the same run
+  adder   the 8-bit ripple-carry adder over 4096 lanes, end to end (encrypt, circuit, decrypt) on arrays and with
+          per-element Ciphertext calls (csgn_mul_batch for the products)
+  sweep   elements whose product is 64 KB .. 64 MB, ~1 GB per call: the grouped kernel against one launch_mul per
+          element (CSGN_SEG_LARGE_BYTES), which sets the large-element threshold of capi_seg.cu
+
+Timing: CUDA events around enough calls to fill >= 1 s after a warm-up call; inputs of the mixed and sweep runs are
+larger than the 126 MB L2.  Usage: python tools/seg_bench.py [--out FILE] [--quick]"""
+import argparse
+import ctypes
+import os
+import subprocess
+import sys
+import time
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+os.environ.setdefault("CSGN_TUNING", "1")      # CSGN_SEG_LARGE_BYTES is honoured only with it
+
+import torch  # noqa: E402
+
+from csgn_b200 import engine as eng  # noqa: E402
+
+LINES = []
+
+
+def log(s):
+    print(s, flush=True)
+    LINES.append(s)
+
+
+def timed(fn, min_s=1.0, min_reps=3):
+    """seconds per call: one warm-up call, then enough calls for >= min_s between two CUDA events"""
+    fn()
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    fn()
+    torch.cuda.synchronize()
+    one = max(time.perf_counter() - t0, 1e-6)
+    reps = max(min_reps, int(np.ceil(min_s / one)))
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    for _ in range(reps):
+        fn()
+    e1.record()
+    torch.cuda.synchronize()
+    return e0.elapsed_time(e1) / 1e3 / reps, reps
+
+
+def launches(fn):
+    c0 = eng.launch_count()
+    fn()
+    return eng.launch_count() - c0
+
+
+def gpu_header():
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.sm,clocks.max.sm", "--format=csv,noheader"],
+                       stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
+    log("gpu: %s" % q.stdout.strip().splitlines()[0] if q.returncode == 0 else "gpu: nvidia-smi unavailable")
+    log("torch %s, %s" % (torch.__version__, eng.version()))
+
+
+def one_block_operands(n, ctx, rng):
+    """n one-block csgn_bufs from one upload (csgn_buf_upload_batch), and the same words as one array"""
+    L = ctx.L
+    words = np.ascontiguousarray(rng.integers(0, 2**63, size=n * L, dtype=np.uint64))
+    ub = eng.UploadBatch([words.ctypes.data + 8 * L * k for k in range(n)], [1] * n, ctx)
+    handles = ub.upload()
+    eng.sync()
+    return words, handles
+
+
+def small(ctx, key, rng, sizes):
+    lib = eng._lib()
+    for n in sizes:
+        wa, ha = one_block_operands(n, ctx, rng)
+        wb, hb = one_block_operands(n, ctx, rng)
+        off = np.arange(n + 1, dtype=np.uint64)
+        A = eng.CiphertextArray(eng.Ciphertext.from_host(wa, ctx), off)
+        B = eng.CiphertextArray(eng.Ciphertext.from_host(wb, ctx), off)
+        res = {}
+        res["seg_mul"] = timed(lambda: A * B), launches(lambda: A * B)
+        res["seg_decrypt"] = timed(lambda: key.decrypt_array(A)), launches(lambda: key.decrypt_array(A))
+
+        out = (ctypes.c_void_p * n)()
+
+        def batch_mul():
+            eng.mul_batch_arrays(ha, hb, out)
+            eng.free_handles(out)
+        bits, counts = (ctypes.c_uint8 * n)(), (ctypes.c_uint64 * n)()
+
+        def batch_dec():
+            eng.check(lib.csgn_decrypt_batch(ha, n, key._h, bits, counts))
+        res["mul_batch"] = timed(batch_mul), launches(batch_mul)
+        res["decrypt_batch"] = timed(batch_dec), launches(batch_dec)
+        for k, ((t, reps), nl) in res.items():
+            log("small n=%-6d %-14s %10.1f us/call  %6d launches/call  (%d calls)" % (n, k, t * 1e6, nl, reps))
+        log("small n=%-6d speed-up: multiply %.1fx, decrypt %.1fx" % (
+            n, res["mul_batch"][0][0] / res["seg_mul"][0][0], res["decrypt_batch"][0][0] / res["seg_decrypt"][0][0]))
+        eng.free_handles(ha)
+        eng.free_handles(hb)
+
+
+def copy_rate(nbytes):
+    src = torch.empty(nbytes // 8, dtype=torch.int64, device="cuda")
+    dst = torch.empty_like(src)
+    t, _ = timed(lambda: dst.copy_(src))
+    del src, dst
+    torch.cuda.empty_cache()
+    return nbytes / t
+
+
+def log_uniform_sizes(rng, n, hi=64):
+    return np.minimum(hi, np.floor(np.exp(rng.uniform(0, np.log(hi + 1), n)))).astype(np.int64)
+
+
+def mixed(ctx, key, rng, target_bytes):
+    L = ctx.L
+    n = 1024
+    while True:
+        t1, t2 = log_uniform_sizes(rng, n), log_uniform_sizes(rng, n)
+        if int((t1 * t2).sum()) * L * 8 >= target_bytes:
+            break
+        n *= 2
+    prod_blocks = int((t1 * t2).sum())
+    pbytes = prod_blocks * L * 8
+    a = torch.randint(-2**62, 2**62, (int(t1.sum()) * L,), dtype=torch.int64, device="cuda")
+    b = torch.randint(-2**62, 2**62, (int(t2.sum()) * L,), dtype=torch.int64, device="cuda")
+    A = eng.CiphertextArray(eng.Ciphertext.from_tensor(a, ctx), np.concatenate([[0], np.cumsum(t1)]))
+    B = eng.CiphertextArray(eng.Ciphertext.from_tensor(b, ctx), np.concatenate([[0], np.cumsum(t2)]))
+    log("mixed: %d elements, operand blocks 1-64 log-uniform, product %d blocks = %.2f GB" % (n, prod_blocks, pbytes / 1e9))
+    cp = copy_rate(pbytes)
+    log("mixed: device-to-device copy of %.2f GB: %.0f GB/s (bytes copied per second)" % (pbytes / 1e9, cp / 1e9))
+    keep = []
+
+    def seg_mul():
+        keep[:] = [A * B]
+    t_seg, _ = timed(seg_mul)
+    keep.clear()
+    # one product of the same size
+    s1 = int(np.sqrt(prod_blocks))
+    s2 = (prod_blocks + s1 - 1) // s1
+    x = eng.Ciphertext.from_tensor(torch.randint(-2**62, 2**62, (s1 * L,), dtype=torch.int64, device="cuda"), ctx)
+    y = eng.Ciphertext.from_tensor(torch.randint(-2**62, 2**62, (s2 * L,), dtype=torch.int64, device="cuda"), ctx)
+    one = []
+
+    def one_mul():
+        one[:] = [x * y]
+    t_one, _ = timed(one_mul)
+    one_bytes = s1 * s2 * L * 8
+    r_seg, r_one = pbytes / t_seg, one_bytes / t_one
+    log("mixed: seg_mul  %8.2f ms  %6.0f GB/s written  %.2f of copy | csgn_mul %dx%d %8.2f ms  %6.0f GB/s  %.2f of copy"
+        " | seg / single %.2f" % (t_seg * 1e3, r_seg / 1e9, r_seg / cp, s1, s2, t_one * 1e3, r_one / 1e9, r_one / cp,
+                                  r_seg / r_one))
+    one.clear()
+    P = A * B
+    counts = torch.zeros(n, dtype=torch.int64, device="cuda")
+    t_sd, _ = timed(lambda: key.decrypt_array_count_async(P, counts.data_ptr()))
+    total = torch.zeros(1, dtype=torch.int64, device="cuda")
+    t_d, _ = timed(lambda: key.count_satisfied_async(P.storage, total.data_ptr()))
+    r_sd, r_d = pbytes / t_sd, pbytes / t_d
+    log("mixed: seg_decrypt %8.2f ms  %6.0f GB/s read  %.2f of copy | csgn_decrypt_count same storage %8.2f ms  %6.0f GB/s"
+        "  %.2f of copy | seg / single %.2f" % (t_sd * 1e3, r_sd / 1e9, r_sd / cp, t_d * 1e3, r_d / 1e9, r_d / cp,
+                                                 r_sd / r_d))
+    del P, A, B, a, b, x, y
+    torch.cuda.empty_cache()
+
+
+def adder(ctx, key, rng, lanes):
+    xb, yb = rng.integers(0, 256, lanes), rng.integers(0, 256, lanes)
+    bits = np.concatenate([np.concatenate([(xb >> i) & 1 for i in range(8)]),
+                           np.concatenate([(yb >> i) & 1 for i in range(8)])]).astype(np.uint8)
+
+    def on_arrays():
+        allb = key.encrypt_array(bits, seed=5)
+        row = lambda r: allb.gather(np.arange(r * lanes, (r + 1) * lanes))    # noqa: E731
+        X, Y = row(0), row(8)
+        S, C = [X + Y], X * Y
+        for i in range(1, 8):
+            X, Y = row(i), row(8 + i)
+            T = X + Y
+            S.append(T + C)
+            C = X * Y + T * C
+        out = [key.decrypt_array(s)[0] for s in S] + [key.decrypt_array(C)[0]]
+        return out
+
+    def per_element():
+        allb = key.encrypt_array(bits, seed=5)
+        el = [allb.element(k) for k in range(16 * lanes)]
+        x = [el[i * lanes:(i + 1) * lanes] for i in range(8)]
+        y = [el[(8 + i) * lanes:(9 + i) * lanes] for i in range(8)]
+        S = [[a + b for a, b in zip(x[0], y[0])]]
+        C = eng.mul_batch(x[0], y[0])
+        for i in range(1, 8):
+            T = [a + b for a, b in zip(x[i], y[i])]
+            S.append([t + c for t, c in zip(T, C)])
+            XY, TC = eng.mul_batch(x[i], y[i]), eng.mul_batch(T, C)
+            C = [p + q for p, q in zip(XY, TC)]
+        return [np.array(key.decrypt_batch(s)[0], dtype=np.uint8) for s in S] + [np.array(key.decrypt_batch(C)[0], np.uint8)]
+
+    got = on_arrays()
+    val = sum(got[i].astype(np.int64) << i for i in range(8))
+    assert np.array_equal(val, (xb + yb) % 256) and np.array_equal(got[8], (xb + yb) >> 8), "adder on arrays is wrong"
+    ref = per_element()
+    assert all(np.array_equal(p, q) for p, q in zip(got, ref)), "the two adders disagree"
+    t_arr, r1 = timed(on_arrays, min_s=2.0, min_reps=2)
+    l_arr = launches(on_arrays)
+    t_el, r2 = timed(per_element, min_s=2.0, min_reps=2)
+    l_el = launches(per_element)
+    log("adder: 8-bit, %d lanes, Context(%d,%d): arrays %8.2f ms (%d launches) | per-element calls %8.2f ms (%d launches)"
+        " | speed-up %.1fx" % (lanes, ctx.N, ctx.D, t_arr * 1e3, l_arr, t_el * 1e3, l_el, t_el / t_arr))
+
+
+def sweep(ctx, total_bytes, sizes_kb):
+    L = ctx.L
+    for kb in sizes_kb:
+        t = max(1, int(round(np.sqrt(kb * 1024 / (8 * L)))))
+        pbytes = t * t * L * 8
+        n = max(1, total_bytes // pbytes)
+        a = torch.randint(-2**62, 2**62, (n * t * L,), dtype=torch.int64, device="cuda")
+        off = np.arange(n + 1, dtype=np.uint64) * t
+        A = eng.CiphertextArray(eng.Ciphertext.from_tensor(a, ctx), off)
+        keep = []
+        res = {}
+        for mode, knob in (("grouped", str(1 << 50)), ("per-element", "0")):
+            os.environ["CSGN_SEG_LARGE_BYTES"] = knob
+
+            def run():
+                keep[:] = [A * A]
+            tt, _ = timed(run)
+            res[mode] = (tt, launches(run))
+            keep.clear()
+        os.environ.pop("CSGN_SEG_LARGE_BYTES", None)
+        g, p = res["grouped"], res["per-element"]
+        log("sweep: product %6.0f KB (%4dx%-4d blocks) x %5d elements = %.2f GB: grouped %7.0f GB/s (%d launches) | "
+            "per-element launch_mul %7.0f GB/s (%d launches) | grouped / per-element %.2f" % (
+                pbytes / 1024, t, t, n, n * pbytes / 1e9, n * pbytes / g[0] / 1e9, g[1], n * pbytes / p[0] / 1e9, p[1],
+                p[0] / g[0]))
+        del A, a
+        torch.cuda.empty_cache()
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--out", default="")
+    ap.add_argument("--quick", action="store_true", help="small sizes (a check of the script, not a measurement)")
+    ap.add_argument("--only", default="small,mixed,adder,sweep")
+    args = ap.parse_args()
+    torch.cuda.set_device(0)
+    eng.init(0)
+    st = torch.cuda.current_stream()
+    eng.set_stream(st.cuda_stream)
+    gpu_header()
+    rng = np.random.default_rng(1)
+    ctx = eng.Context(1247, 16)
+    key = eng.SecretKey(ctx, rng.permutation(1247)[:16].astype(np.uint64))
+    only = args.only.split(",")
+    if "small" in only:
+        small(ctx, key, rng, [100, 1000] if args.quick else [1000, 10000, 100000])
+    if "mixed" in only:
+        mixed(ctx, key, rng, (64 << 20) if args.quick else (1 << 30))
+    if "adder" in only:
+        adder(ctx, key, rng, 256 if args.quick else 4096)
+    if "sweep" in only:
+        sweep(ctx, (64 << 20) if args.quick else (1 << 30),
+              [64, 256] if args.quick else [64, 256, 1024, 4096, 16384, 65536])
+    eng.set_stream(0)
+    if args.out:
+        with open(args.out, "w") as f:
+            f.write("\n".join(LINES) + "\n")
+
+
+if __name__ == "__main__":
+    main()

@@ -3,6 +3,7 @@ library is missing or no B200 is visible -- there is no CPU fallback to fall to.
 import ctypes
 import os
 import re
+import warnings
 
 from . import build as _build
 
@@ -77,6 +78,9 @@ SIGNATURES = {
     "csgn_encrypt_batch": (ctypes.c_int, [_vp, _vp, _u64, _u64, _u64, _vpp]),
     "csgn_seg_mul": (ctypes.c_int, [_vp, _vp, _vp, _vp, _u64, _vp, _vpp]),
     "csgn_seg_concat": (ctypes.c_int, [_vp, _vp, _vp, _vp, _u64, _vp, _vpp]),
+    "csgn_seg_mul_sum": (ctypes.c_int, [ctypes.POINTER(_vp), ctypes.POINTER(_vp), ctypes.POINTER(_vp), ctypes.POINTER(_vp),
+                                        ctypes.c_uint32, ctypes.POINTER(_vp), ctypes.POINTER(_vp), ctypes.c_uint32, _u64,
+                                        _vp, _vpp]),
     "csgn_seg_gather": (ctypes.c_int, [_vp, _vp, _u64, _vp, _u64, _vp, _vpp]),
     "csgn_concat_n": (ctypes.c_int, [ctypes.POINTER(_vp), _u64, _vpp]),
     "csgn_seg_decrypt_count_async": (ctypes.c_int, [_vp, _vp, _u64, _vp, _vp]),
@@ -148,7 +152,13 @@ def load(build_if_missing=True):
         raise ImportError("CUDA extension %s is missing; build it with `python -m csgn_b200.build` "
                           "(no CPU fallback exists)" % path)
     lib = ctypes.CDLL(path)
+    unbound = [name for name in SIGNATURES if override and not hasattr(lib, name)]
+    if unbound:                  # an older build under A/B comparison: its newer entry points stay unbound
+        warnings.warn("CSGN_LIBRARY=%s lacks %d entry points of include/csgn.h, left unbound: %s"
+                      % (path, len(unbound), ", ".join(unbound)))
     for name, (res, args) in SIGNATURES.items():
+        if name in unbound:
+            continue
         fn = getattr(lib, name)  # AttributeError here = header and library disagree
         fn.restype = res
         fn.argtypes = args

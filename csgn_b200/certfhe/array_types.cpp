@@ -2,6 +2,7 @@
 // (include/csgn.h): each operation is ONE call, which makes one kernel launch for all small elements.
 //   CiphertextArray(vector)   -> csgn_concat_n
 //   operator* / operator+     -> csgn_seg_mul / csgn_seg_concat
+//   sumOfProducts             -> csgn_seg_mul_sum
 //   gather                    -> csgn_seg_gather
 //   applyPermutation          -> csgn_permute on the storage (a permutation acts on every block by itself)
 //   encryptArray / decryptArray -> csgn_encrypt_batch / csgn_seg_decrypt
@@ -84,6 +85,43 @@ CiphertextArray CiphertextArray::operator+(const CiphertextArray &c) const {
                                 &out),
                 "csgn_seg_concat");
     return CiphertextArray(out, off, context);
+}
+
+CiphertextArray CiphertextArray::sumOfProducts(const std::vector<std::pair<CiphertextArray, CiphertextArray>> &products,
+                                               const std::vector<CiphertextArray> &terms) {
+    std::vector<const CiphertextArray *> all;
+    for (size_t i = 0; i < products.size(); ++i) {
+        all.push_back(&products[i].first);
+        all.push_back(&products[i].second);
+    }
+    for (size_t i = 0; i < terms.size(); ++i) all.push_back(&terms[i]);
+    if (all.empty()) throw Error("CiphertextArray::sumOfProducts: no products and no terms");
+    const CiphertextArray &x0 = *all[0];
+    for (size_t i = 1; i < all.size(); ++i) {
+        if (all[i]->size() != x0.size())
+            throw Error("CiphertextArray::sumOfProducts: arrays of " + to_string(x0.size()) + " and " +
+                        to_string(all[i]->size()) + " elements");
+        if (all[i]->context.getN() != x0.context.getN() || all[i]->context.getD() != x0.context.getD())
+            throw Error("CiphertextArray::sumOfProducts: arrays of different contexts");
+    }
+    std::vector<const csgn_buf *> a, b, c;
+    std::vector<const uint64_t *> ao, bo, co;
+    for (size_t i = 0; i < products.size(); ++i) {
+        a.push_back(products[i].first.storage.get());
+        ao.push_back(products[i].first.offsets.data());
+        b.push_back(products[i].second.storage.get());
+        bo.push_back(products[i].second.offsets.data());
+    }
+    for (size_t i = 0; i < terms.size(); ++i) {
+        c.push_back(terms[i].storage.get());
+        co.push_back(terms[i].offsets.data());
+    }
+    std::vector<uint64_t> off(x0.size() + 1);
+    csgn_buf *out = nullptr;
+    glue::check(csgn_seg_mul_sum(a.data(), ao.data(), b.data(), bo.data(), (uint32_t)products.size(), c.data(), co.data(),
+                                 (uint32_t)terms.size(), x0.size(), off.data(), &out),
+                "csgn_seg_mul_sum");
+    return CiphertextArray(out, off, x0.context);
 }
 
 CiphertextArray CiphertextArray::gather(const std::vector<uint64_t> &idx) const {

@@ -25,6 +25,7 @@
 
 #include <memory>
 #include <stdexcept>
+#include <utility>
 
 struct csgn_buf;
 struct csgn_key;
@@ -335,6 +336,11 @@ public:
     CiphertextArray operator+(const CiphertextArray &c) const;   // element k = this_k + c_k
     CiphertextArray gather(const std::vector<uint64_t> &idx) const;   // element j = this_{idx[j]}
     CiphertextArray applyPermutation(const Permutation &permutation) const;   // every element permuted
+    // element k = A0_k*B0_k + A1_k*B1_k + ... + C0_k + ... (csgn_seg_mul_sum): one gate of a circuit -- carry,
+    // majority, multiplexer -- in one call, every output word written once.  Throws Error on arrays of different sizes
+    // or contexts, or when both lists are empty.
+    static CiphertextArray sumOfProducts(const std::vector<std::pair<CiphertextArray, CiphertextArray>> &products,
+                                         const std::vector<CiphertextArray> &terms = {});
 
     const std::vector<uint64_t> &getOffsets() const;
     const csgn_buf *deviceBuffer() const;

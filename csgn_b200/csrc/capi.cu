@@ -635,12 +635,8 @@ namespace detail {
 // A small host table (work items, offsets) to fresh device memory on the current stream, through the pinned staging:
 // no host synchronisation, and the caller may reuse its array at once.  Tables beyond the staging limit are copied
 // straight from the caller's memory, and the call waits for that copy.
-int stage_to_device(const void *host, size_t bytes, void **out) {
-    *out = nullptr;
+int stage_into(void *d, const void *host, size_t bytes) {
     if (bytes == 0) return CSGN_OK;
-    uint64_t *d = nullptr;
-    int rc = dev_alloc((bytes + 7) / 8, &d);
-    if (rc != CSGN_OK) return rc;
     StagingSlot *sl = bytes <= kStagingMaxOne ? take_staging(bytes) : nullptr;
     cudaError_t e;
     if (sl) {
@@ -652,9 +648,19 @@ int stage_to_device(const void *host, size_t bytes, void **out) {
         if (e == cudaSuccess) e = cudaStreamSynchronize(g.stream);
         if (e == cudaSuccess) note_synced(g.stream);
     }
-    if (e != cudaSuccess) {
+    return e == cudaSuccess ? CSGN_OK : cuda_fail(e, "table upload");
+}
+
+int stage_to_device(const void *host, size_t bytes, void **out) {
+    *out = nullptr;
+    if (bytes == 0) return CSGN_OK;
+    uint64_t *d = nullptr;
+    int rc = dev_alloc((bytes + 7) / 8, &d);
+    if (rc != CSGN_OK) return rc;
+    rc = stage_into(d, host, bytes);
+    if (rc != CSGN_OK) {
         dev_free(d);
-        return cuda_fail(e, "table upload");
+        return rc;
     }
     *out = d;
     return CSGN_OK;

@@ -19,6 +19,7 @@ constexpr long kSegLargeBytes = 8l << 20;
 constexpr uint64_t kSegTaskMinWords = 1024, kSegTaskMaxWords = 32768;
 
 uint64_t large_bytes() { return (uint64_t)std::max(0l, env_long("CSGN_SEG_LARGE_BYTES", kSegLargeBytes)); }
+uint64_t large_words() { return large_bytes() / 8; }
 
 uint64_t task_words(uint64_t total_words) {
     const uint64_t warps = (uint64_t)device_props().sm_count * 8 * 8;
@@ -48,6 +49,100 @@ int check_blocks(uint64_t total, uint32_t L) {
 struct DevTable {
     void *d = nullptr;
     ~DevTable() { dev_free(d); }
+};
+
+// The work of one grouped multiply (seg_mul_kernel), added piece by piece in output order: products, and plain terms
+// (items whose left operand is the all-ones block at the head of the staged table).  Small pieces become items packed
+// into tasks of about task_words(small_words) words; a long term is cut into items of about one task each.  A piece of
+// large_words() or more goes straight into its position: launch_mul for a product, a device-to-device copy for a term.
+class SegMulWork {
+public:
+    SegMulWork(uint32_t L, uint64_t small_words, csgn_buf *out)
+        : L_(L), large_(large_words()), target_(task_words(small_words)), out_(out) {}
+
+    void product(const uint64_t *a, uint64_t t1, const uint64_t *b, uint64_t t2) {
+        if (t1 && t2 && e_ == cudaSuccess) {
+            if (t1 * t2 * L_ >= large_) {
+                e_ = launch_mul(a, t1, b, t2, L_, out_->d + pos_ * L_, g.stream);
+            } else {
+                const uint64_t row = t2 * L_, step = std::max<uint64_t>(1, target_ / row);
+                for (uint64_t r = 0; r < t1; r += step) {
+                    const uint64_t rows = std::min(step, t1 - r);
+                    add({a + r * L_, b, pos_ + r * t2, (uint32_t)t2, (uint32_t)rows}, rows * row);
+                }
+            }
+        }
+        pos_ += t1 * t2;
+    }
+
+    void term(const uint64_t *c, uint64_t t) {
+        if (t && e_ == cudaSuccess) {
+            if (t * L_ >= large_) {
+                e_ = cudaMemcpyAsync(out_->d + pos_ * L_, c, t * L_ * sizeof(uint64_t), cudaMemcpyDeviceToDevice, g.stream);
+            } else {
+                const uint64_t step = std::max<uint64_t>(1, target_ / L_);
+                for (uint64_t r = 0; r < t; r += step) {
+                    const uint64_t blocks = std::min(step, t - r);
+                    add({nullptr, c + r * L_, pos_ + r, (uint32_t)blocks, 1}, blocks * L_);   // a: the ones block
+                }
+                terms_ = true;
+            }
+        }
+        pos_ += t;
+    }
+
+    // Stage the table and make the one grouped launch (none without small pieces).
+    int launch() {
+        if (e_ != cudaSuccess) return cuda_fail(e_, "grouped multiply kernel");
+        if (items_.empty()) return CSGN_OK;
+        if (tasks_.back() != items_.size()) tasks_.push_back((uint32_t)items_.size());
+        if (items_.size() >= UINT32_MAX) return fail(CSGN_ERR_INVALID_ARGUMENT, "too many work items");
+        // table: [the all-ones block, L words rounded up to 16 bytes, when there are terms] [items] [task bounds]
+        const size_t head = terms_ ? (size_t)((L_ + 1) & ~1u) * sizeof(uint64_t) : 0;
+        const size_t item_bytes = items_.size() * sizeof(SegMulItem);
+        const size_t bytes = head + item_bytes + tasks_.size() * sizeof(uint32_t);
+        uint64_t *d = nullptr;
+        int rc = dev_alloc((bytes + 7) / 8, &d);
+        if (rc != CSGN_OK) return rc;
+        DevTable t;
+        t.d = d;
+        uintptr_t addr = reinterpret_cast<uintptr_t>(out_->d) | reinterpret_cast<uintptr_t>(d);
+        std::vector<uint8_t> tab(bytes);
+        std::fill_n(reinterpret_cast<uint64_t *>(tab.data()), head / sizeof(uint64_t), ~0ull);
+        SegMulItem *it = reinterpret_cast<SegMulItem *>(tab.data() + head);
+        for (size_t i = 0; i < items_.size(); ++i) {
+            it[i] = items_[i];
+            if (!it[i].a) it[i].a = d;
+            addr |= reinterpret_cast<uintptr_t>(it[i].a) | reinterpret_cast<uintptr_t>(it[i].b);
+        }
+        memcpy(tab.data() + head + item_bytes, tasks_.data(), tasks_.size() * sizeof(uint32_t));
+        rc = stage_into(d, tab.data(), bytes);
+        if (rc != CSGN_OK) return rc;
+        const SegMulItem *d_items = reinterpret_cast<const SegMulItem *>(reinterpret_cast<const uint8_t *>(d) + head);
+        const cudaError_t e = launch_seg_mul(out_->d, L_, !(L_ & 1u) && (addr & 15u) == 0, d_items,
+                                             reinterpret_cast<const uint32_t *>(d_items + items_.size()),
+                                             (uint32_t)(tasks_.size() - 1), g.stream);
+        return e == cudaSuccess ? CSGN_OK : cuda_fail(e, "grouped multiply kernel");
+    }
+
+private:
+    void add(const SegMulItem &m, uint64_t words) {
+        items_.push_back(m);
+        in_task_ += words;
+        if (in_task_ >= target_) {
+            tasks_.push_back((uint32_t)items_.size());
+            in_task_ = 0;
+        }
+    }
+
+    const uint32_t L_;
+    const uint64_t large_, target_;
+    csgn_buf *const out_;
+    uint64_t pos_ = 0, in_task_ = 0;   // output block of the next piece; words in the open task
+    bool terms_ = false;
+    cudaError_t e_ = cudaSuccess;
+    std::vector<SegMulItem> items_;
+    std::vector<uint32_t> tasks_ = std::vector<uint32_t>(1, 0);
 };
 
 // out = src[0] || src[1] || ... (words[p] words from src[p]) in one launch of the piece copy.
@@ -120,62 +215,118 @@ int csgn_seg_mul(const csgn_buf *a, const uint64_t *a_off, const csgn_buf *b, co
     acquire_read(a);
     acquire_read(b);
     acquire_write(c);
-    // work items: small products whole or cut into row ranges of about one task each, packed into tasks in element
-    // order; large products: one launch_mul each
-    const uint64_t large = large_bytes() / 8;
+    const uint64_t large = large_words();
     uint64_t small_words = 0;
     for (uint64_t k = 0; k < n; ++k) {
         const uint64_t w = (oo[k + 1] - oo[k]) * L;
         if (w < large) small_words += w;
     }
-    const uint64_t target = task_words(small_words);
-    std::vector<SegMulItem> items;
-    std::vector<uint32_t> tasks(1, 0);
-    uint64_t in_task = 0;
-    cudaError_t e = cudaSuccess;
-    for (uint64_t k = 0; k < n && e == cudaSuccess; ++k) {
-        const uint64_t t1 = a_off[k + 1] - a_off[k], t2 = b_off[k + 1] - b_off[k];
-        if (t1 == 0 || t2 == 0) continue;
-        if (t1 * t2 * L >= large) {
-            e = launch_mul(a->d + a_off[k] * L, t1, b->d + b_off[k] * L, t2, L, c->d + oo[k] * L, g.stream);
-            continue;
-        }
-        const uint64_t row = t2 * L, step = std::max<uint64_t>(1, target / row);
-        for (uint64_t r = 0; r < t1; r += step) {
-            const uint64_t rows = std::min(step, t1 - r);
-            items.push_back({a_off[k] + r, b_off[k], oo[k] + r * t2, (uint32_t)t2, (uint32_t)rows});
-            in_task += rows * row;
-            if (in_task >= target) {
-                tasks.push_back((uint32_t)items.size());
-                in_task = 0;
-            }
-        }
-    }
-    if (tasks.back() != items.size()) tasks.push_back((uint32_t)items.size());
-    if (e == cudaSuccess && !items.empty()) {
-        if (items.size() >= UINT32_MAX) {
-            csgn_buf_free(c);
-            return fail(CSGN_ERR_INVALID_ARGUMENT, "too many work items");
-        }
-        std::vector<uint8_t> tab(items.size() * sizeof(SegMulItem) + tasks.size() * sizeof(uint32_t));
-        memcpy(tab.data(), items.data(), items.size() * sizeof(SegMulItem));
-        memcpy(tab.data() + items.size() * sizeof(SegMulItem), tasks.data(), tasks.size() * sizeof(uint32_t));
-        DevTable t;
-        rc = stage_to_device(tab.data(), tab.size(), &t.d);
-        if (rc != CSGN_OK) {
-            csgn_buf_free(c);
-            return rc;
-        }
-        const SegMulItem *d_items = static_cast<const SegMulItem *>(t.d);
-        e = launch_seg_mul(a->d, b->d, c->d, L, d_items, reinterpret_cast<const uint32_t *>(d_items + items.size()),
-                           (uint32_t)(tasks.size() - 1), g.stream);
-    }
-    if (e != cudaSuccess) {
+    SegMulWork work(L, small_words, c);
+    for (uint64_t k = 0; k < n; ++k)
+        work.product(a->d + a_off[k] * L, a_off[k + 1] - a_off[k], b->d + b_off[k] * L, b_off[k + 1] - b_off[k]);
+    rc = work.launch();
+    if (rc != CSGN_OK) {
         csgn_buf_free(c);
-        return cuda_fail(e, "grouped multiply kernel");
+        return rc;
     }
     memcpy(out_off, oo.data(), (n + 1) * sizeof(uint64_t));
     *out = c;
+    return CSGN_OK;
+}
+
+int csgn_seg_mul_sum(const csgn_buf *const *a, const uint64_t *const *a_off, const csgn_buf *const *b,
+                     const uint64_t *const *b_off, uint32_t n_products, const csgn_buf *const *c,
+                     const uint64_t *const *c_off, uint32_t n_terms, uint64_t n, uint64_t *out_off, csgn_buf **out) {
+    NEED_INIT();
+    if (!out || !out_off) return fail(CSGN_ERR_INVALID_ARGUMENT, "null argument");
+    if (n_products == 0 && n_terms == 0) return fail(CSGN_ERR_INVALID_ARGUMENT, "no products and no terms");
+    if (n_products && (!a || !a_off || !b || !b_off)) return fail(CSGN_ERR_INVALID_ARGUMENT, "null product arrays");
+    if (n_terms && (!c || !c_off)) return fail(CSGN_ERR_INVALID_ARGUMENT, "null term arrays");
+    // operand j: the left operands of the products, their right operands, then the terms
+    const uint64_t p = n_products, m = p * 2 + n_terms;
+    auto op = [&](uint64_t j) { return j < p ? a[j] : j < 2 * p ? b[j - p] : c[j - 2 * p]; };
+    auto off = [&](uint64_t j) { return j < p ? a_off[j] : j < 2 * p ? b_off[j - p] : c_off[j - 2 * p]; };
+    auto name = [&](uint64_t j) {
+        char s[48];
+        snprintf(s, sizeof s, "%s %llu", j < p ? "left operand" : j < 2 * p ? "right operand" : "term",
+                 (unsigned long long)(j < p ? j : j < 2 * p ? j - p : j - 2 * p));
+        return std::string(s);
+    };
+    for (uint64_t j = 0; j < m; ++j)
+        if (!op(j)) return fail(CSGN_ERR_INVALID_ARGUMENT, "null %s", name(j).c_str());
+    const uint32_t L = op(0)->L;
+    for (uint64_t j = 1; j < m; ++j)
+        if (op(j)->L != L)
+            return fail(CSGN_ERR_SHAPE_MISMATCH, "words per block differ (%s: %u vs %s: %u)", name(0).c_str(), L,
+                        name(j).c_str(), op(j)->L);
+    for (uint64_t j = 0; j < m; ++j) {
+        const int rc = check_offsets(op(j), off(j), n, name(j).c_str());
+        if (rc != CSGN_OK) return rc;
+    }
+    std::vector<uint64_t> oo(n + 1, 0);
+    for (uint64_t k = 0; k < n; ++k) {
+        uint64_t o = oo[k];
+        for (uint64_t i = 0; i < p; ++i) {
+            const uint64_t t1 = a_off[i][k + 1] - a_off[i][k], t2 = b_off[i][k + 1] - b_off[i][k];
+            if (t2 && t1 > UINT64_MAX / t2)
+                return fail(CSGN_ERR_INVALID_ARGUMENT, "product %llu of element %llu overflows", (unsigned long long)i,
+                            (unsigned long long)k);
+            if (o + t1 * t2 < o) return fail(CSGN_ERR_INVALID_ARGUMENT, "output block count overflows");
+            o += t1 * t2;
+        }
+        for (uint64_t i = 0; i < n_terms; ++i) {
+            const uint64_t t = c_off[i][k + 1] - c_off[i][k];
+            if (o + t < o) return fail(CSGN_ERR_INVALID_ARGUMENT, "output block count overflows");
+            o += t;
+        }
+        oo[k + 1] = o;
+    }
+    int rc = check_blocks(oo[n], L);
+    if (rc != CSGN_OK) return rc;
+    // every distinct buffer once; the automatic lane follows the two largest
+    std::vector<const csgn_buf *> bufs;
+    for (uint64_t j = 0; j < m; ++j) bufs.push_back(op(j));
+    std::sort(bufs.begin(), bufs.end());
+    bufs.erase(std::unique(bufs.begin(), bufs.end()), bufs.end());
+    std::stable_sort(bufs.begin(), bufs.end(),
+                     [](const csgn_buf *x, const csgn_buf *y) { return x->n_blocks > y->n_blocks; });
+    AutoLane lane(bufs[0], bufs.size() > 1 ? bufs[1] : nullptr);
+    for (const csgn_buf *x : bufs) {
+        rc = need_dense(x);
+        if (rc != CSGN_OK) return rc;
+    }
+    csgn_buf *res = nullptr;
+    rc = new_buf(oo[n], L, 0, &res);
+    if (rc != CSGN_OK) return rc;
+    for (const csgn_buf *x : bufs) acquire_read(x);
+    acquire_write(res);
+    const uint64_t large = large_words();
+    uint64_t small_words = 0;
+    for (uint64_t k = 0; k < n; ++k) {
+        for (uint64_t i = 0; i < p; ++i) {
+            const uint64_t w = (a_off[i][k + 1] - a_off[i][k]) * (b_off[i][k + 1] - b_off[i][k]) * L;
+            if (w < large) small_words += w;
+        }
+        for (uint64_t i = 0; i < n_terms; ++i) {
+            const uint64_t w = (c_off[i][k + 1] - c_off[i][k]) * L;
+            if (w < large) small_words += w;
+        }
+    }
+    // output order: element by element, its products first, then its terms
+    SegMulWork work(L, small_words, res);
+    for (uint64_t k = 0; k < n; ++k) {
+        for (uint64_t i = 0; i < p; ++i)
+            work.product(a[i]->d + a_off[i][k] * L, a_off[i][k + 1] - a_off[i][k], b[i]->d + b_off[i][k] * L,
+                         b_off[i][k + 1] - b_off[i][k]);
+        for (uint64_t i = 0; i < n_terms; ++i) work.term(c[i]->d + c_off[i][k] * L, c_off[i][k + 1] - c_off[i][k]);
+    }
+    rc = work.launch();
+    if (rc != CSGN_OK) {
+        csgn_buf_free(res);
+        return rc;
+    }
+    memcpy(out_off, oo.data(), (n + 1) * sizeof(uint64_t));
+    *out = res;
     return CSGN_OK;
 }
 
@@ -295,7 +446,7 @@ int csgn_seg_decrypt_count_async(const csgn_buf *c, const uint64_t *c_off, uint6
     acquire_read(c);
     CU(cudaMemsetAsync(device_counts, 0, n * sizeof(uint64_t), g.stream));
     // tasks: runs of consecutive small elements cut into pieces of about `target` blocks; large elements: one fold each
-    const uint64_t large = large_bytes() / 8;
+    const uint64_t large = large_words();
     uint64_t small_words = 0;
     for (uint64_t k = 0; k < n; ++k) {
         const uint64_t w = (c_off[k + 1] - c_off[k]) * L;

@@ -54,15 +54,20 @@ cudaError_t launch_concat(const uint64_t *a, uint64_t n_words_a, const uint64_t 
 cudaError_t launch_piece_copy(const void *const *src, const uint64_t *dst, uint32_t n_pieces, uint64_t total_units,
                               bool units16, void *out, cudaStream_t stream);
 
-// Ciphertext arrays (segments.cu).  Grouped multiply: work item k multiplies rows [a, a + rows) of its left operand
-// by the t2 blocks starting at block b of the right operand, into the rows*t2 blocks at block `out` of the output
-// (all in blocks of L words); a warp task is a run of consecutive items [task[t], task[t+1]).  One launch.
+// Ciphertext arrays (segments.cu).  Grouped multiply: work item k multiplies the `rows` blocks at device address a
+// (its left operand's first row) by the t2 blocks at device address b (its right operand), into the rows*t2 blocks at
+// block `out` of the output (blocks of L words); the operands may lie in any buffers.  A plain (copy) term is an item
+// whose left operand is one all-ones block: AND with ~0 is the identity on every word.  A warp task is a run of
+// consecutive items [task[t], task[t+1]).  units16: L is even and every operand, the output and the items are 16-byte
+// aligned.  One launch.
 struct SegMulItem {
-    uint64_t a, b, out;
+    const uint64_t *a, *b;
+    uint64_t out;
     uint32_t t2, rows;
 };
-cudaError_t launch_seg_mul(const uint64_t *a, const uint64_t *b, uint64_t *out, uint32_t L, const SegMulItem *items,
-                           const uint32_t *tasks, uint32_t n_tasks, cudaStream_t stream);
+static_assert(sizeof(SegMulItem) == 32, "SegMulItem is read as one 32-byte record");
+cudaError_t launch_seg_mul(uint64_t *out, uint32_t L, bool units16, const SegMulItem *items, const uint32_t *tasks,
+                           uint32_t n_tasks, cudaStream_t stream);
 // Segmented decrypt: a warp task walks blocks [first, end), which belong to elements [elem, elem_last] (element e =
 // blocks [off[e], off[e+1]), off on the device), and adds each element's satisfied-block count to counts[e] (zeroed
 // by the caller in stream order).  One launch.

@@ -440,6 +440,30 @@ class CiphertextArray:
         """csgn_seg_concat: element k = self_k + other_k (block concatenation, the homomorphic XOR)."""
         return self._binary(_lib().csgn_seg_concat, other)
 
+    @staticmethod
+    def sum_of_products(products, terms=()):
+        """csgn_seg_mul_sum: element k = A0_k*B0_k + A1_k*B1_k + ... + C0_k + ... for `products` [(A0, B0), ...] and
+        `terms` [C0, ...], every output word written once (one gate of a circuit in one call)."""
+        products = [(x, y) for x, y in products]
+        terms = list(terms)
+        arrays = [x for pr in products for x in pr] + terms
+        if not arrays:
+            raise ValueError("sum_of_products needs at least one product or term")
+        n, ctx = len(arrays[0]), arrays[0].ctx
+        for x in arrays[1:]:
+            if len(x) != n:
+                raise ValueError("arrays of %d and %d elements" % (n, len(x)))
+            if (x.ctx.N, x.ctx.D) != (ctx.N, ctx.D):
+                raise ValueError("arrays of Context(%d,%d) and Context(%d,%d)" % (ctx.N, ctx.D, x.ctx.N, x.ctx.D))
+        h = lambda xs: handle_array([x.storage for x in xs]) if xs else None                          # noqa: E731
+        o = lambda xs: (_vp * len(xs))(*[x.offsets.ctypes.data for x in xs]) if xs else None          # noqa: E731
+        left, right = [x for x, _ in products], [y for _, y in products]
+        out_off = np.empty(n + 1, dtype=np.uint64)
+        out = _vp()
+        check(_lib().csgn_seg_mul_sum(h(left), o(left), h(right), o(right), len(products), h(terms), o(terms), len(terms),
+                                      n, out_off.ctypes.data_as(_vp), ctypes.byref(out)))
+        return CiphertextArray(Ciphertext(out, ctx), out_off)
+
     def gather(self, idx):
         """csgn_seg_gather: element j = self_{idx[j]} (any order, repeats allowed)."""
         ix = np.ascontiguousarray(np.asarray(idx, dtype=np.uint64).reshape(-1))

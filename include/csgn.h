@@ -253,6 +253,15 @@ int csgn_seg_mul(const csgn_buf *a, const uint64_t *a_off, const csgn_buf *b, co
 /* element k = a_k || b_k (src/Ciphertext.cpp:107-122): the element-wise homomorphic XOR. */
 int csgn_seg_concat(const csgn_buf *a, const uint64_t *a_off, const csgn_buf *b, const uint64_t *b_off, uint64_t n,
                     uint64_t *out_off, csgn_buf **out);
+/* element k = a[0]_k*b[0]_k || ... || a[p-1]_k*b[p-1]_k || c[0]_k || ... || c[q-1]_k   (p = n_products, q = n_terms)
+ * the element-wise homomorphic XOR of p ANDs and q plain terms, every output word written once: one gate of a circuit
+ * (carry x*y + (x+y)*c, majority x*y + x*z + y*z, multiplexer s*a + s*b + b) in one call and one launch.  The words
+ * of element k are those of (a[0]*b[0] + ... ) + c[0] + ... built with csgn_seg_mul and csgn_seg_concat, in that
+ * block order; a product is empty when either operand element is empty.  p + q >= 1, every buffer has the same L, and
+ * a buffer may appear any number of times (x*x, x*y + x). */
+int csgn_seg_mul_sum(const csgn_buf *const *a, const uint64_t *const *a_off, const csgn_buf *const *b,
+                     const uint64_t *const *b_off, uint32_t n_products, const csgn_buf *const *c,
+                     const uint64_t *const *c_off, uint32_t n_terms, uint64_t n, uint64_t *out_off, csgn_buf **out);
 /* element j = src_{idx[j]}, j < m: any order, repeats allowed; idx[j] < n_src is checked. */
 int csgn_seg_gather(const csgn_buf *src, const uint64_t *src_off, uint64_t n_src, const uint64_t *idx, uint64_t m,
                     uint64_t *out_off, csgn_buf **out);

@@ -7,10 +7,15 @@
           both as a fraction of a device-to-device copy (torch) of the same bytes measured in the same run
   adder   the 8-bit ripple-carry adder over 4096 lanes, end to end (encrypt, circuit, decrypt) on arrays and with
           per-element Ciphertext calls (csgn_mul_batch for the products)
+  gates   the carry step C' = X*Y + T*C of a 12-bit ripple-carry adder over 4096 lanes (carry 2^i - 1 blocks per lane,
+          ~2.7 GB at the last step) as three calls (csgn_seg_mul twice, csgn_seg_concat) and as one csgn_seg_mul_sum:
+          time and launches per step, output bytes per second as a fraction of a device-to-device copy of the same
+          bytes; then the whole 12-bit adder (circuit and decrypt) both ways
   sweep   elements whose product is 64 KB .. 64 MB, ~1 GB per call: the grouped kernel against one launch_mul per
           element (CSGN_SEG_LARGE_BYTES), which sets the large-element threshold of capi_seg.cu
 
-Timing: CUDA events around enough calls to fill >= 1 s after a warm-up call; inputs of the mixed and sweep runs are
+Under CSGN_LIBRARY=<older libcsgn.so> (an A/B run) sections that need entry points the older build lacks are skipped.
+Timing: CUDA events, recorded on the stream the library runs on, around enough calls to fill >= 1 s after a warm-up call; inputs of the mixed and sweep runs are
 larger than the 126 MB L2.  Usage: python tools/seg_bench.py [--out FILE] [--quick]"""
 import argparse
 import ctypes
@@ -65,7 +70,7 @@ def gpu_header():
     q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.sm,clocks.max.sm", "--format=csv,noheader"],
                        stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
     log("gpu: %s" % q.stdout.strip().splitlines()[0] if q.returncode == 0 else "gpu: nvidia-smi unavailable")
-    log("torch %s, %s" % (torch.__version__, eng.version()))
+    log("torch %s, %s, %s" % (torch.__version__, eng.version(), os.environ.get("CSGN_LIBRARY", "libcsgn.so of this tree")))
 
 
 def one_block_operands(n, ctx, rng):
@@ -219,6 +224,82 @@ def adder(ctx, key, rng, lanes):
         " | speed-up %.1fx" % (lanes, ctx.N, ctx.D, t_arr * 1e3, l_arr, t_el * 1e3, l_el, t_el / t_arr))
 
 
+def gates(ctx, key, rng, lanes, bits):
+    SP = eng.CiphertextArray.sum_of_products
+    xb, yb = rng.integers(0, 1 << bits, lanes), rng.integers(0, 1 << bits, lanes)
+    plain = np.concatenate([np.concatenate([(v >> i) & 1 for i in range(bits)]) for v in (xb, yb)]).astype(np.uint8)
+    allb = key.encrypt_array(plain, seed=7)
+    rows = [allb.gather(np.arange(r * lanes, (r + 1) * lanes)) for r in range(2 * bits)]
+    T = [rows[i] + rows[bits + i] for i in range(bits)]
+
+    def adder(one_call):
+        C = rows[0] * rows[bits]
+        S = [T[0]]
+        for i in range(1, bits):
+            S.append(T[i] + C)
+            C = SP([(rows[i], rows[bits + i]), (T[i], C)]) if one_call else rows[i] * rows[bits + i] + T[i] * C
+        return S, C
+
+    def decrypted(S, C):
+        return [key.decrypt_array(s)[0] for s in S] + [key.decrypt_array(C)[0]]
+
+    S3, C3 = adder(False)
+    S1, C1 = adder(True)
+    assert np.array_equal(C1.offsets, C3.offsets), "carry offsets differ"
+    assert C1.storage.checksum() == C3.storage.checksum(), "carry words differ"
+    got = decrypted(S1, C1)
+    assert all(np.array_equal(p, q) for p, q in zip(decrypted(S3, C3), got)), "the two adders disagree"
+    val = sum(got[i].astype(np.int64) << i for i in range(bits))
+    assert np.array_equal(val, (xb + yb) % (1 << bits)) and np.array_equal(got[bits], (xb + yb) >> bits), "adder wrong"
+    # the last carry step: C' = X*Y + T*C with the carry of bit bits-2
+    C = rows[0] * rows[bits]
+    for i in range(1, bits - 1):
+        C = SP([(rows[i], rows[bits + i]), (T[i], C)])
+    X, Y, Tl = rows[bits - 1], rows[2 * bits - 1], T[bits - 1]
+    out_bytes = C1.storage.n_blocks * ctx.L * 8
+    del S3, C3, S1
+    torch.cuda.empty_cache()
+    cp = copy_rate(out_bytes)
+    keep = []
+
+    def three():
+        keep[:] = [X * Y + Tl * C]
+
+    def one():
+        keep[:] = [SP([(X, Y), (Tl, C)])]
+    assert SP([(X, Y), (Tl, C)]).storage.checksum() == C1.storage.checksum()
+    del C1
+    res = {}
+    for name, fn in (("three calls", three), ("one call", one), ("three calls", three), ("one call", one)):
+        t, _ = timed(fn)
+        res.setdefault(name, []).append(t)
+        res[name + " launches"] = launches(fn)
+        keep.clear()
+    log("gates: carry step %d of a %d-bit adder, %d lanes, Context(%d,%d): carry in %d -> out %d blocks per lane, "
+        "output %.2f GB; device-to-device copy of the same bytes %.0f GB/s" % (
+            bits - 1, bits, lanes, ctx.N, ctx.D, (1 << (bits - 1)) - 1, (1 << bits) - 1, out_bytes / 1e9, cp / 1e9))
+    for name in ("three calls", "one call"):
+        t = min(res[name])
+        log("gates: carry step, %-11s %8.3f ms (runs %s)  %d launches  %6.0f GB/s of output  %.2f of copy" % (
+            name, t * 1e3, " / ".join("%.3f" % (x * 1e3) for x in res[name]), res[name + " launches"],
+            out_bytes / t / 1e9, out_bytes / t / cp))
+    log("gates: carry step, three calls / one call %.2fx" % (min(res["three calls"]) / min(res["one call"])))
+    del C
+    torch.cuda.empty_cache()
+    whole = {}
+    for name, flag in (("three calls", False), ("one call", True), ("three calls", False), ("one call", True)):
+        def run():
+            decrypted(*adder(flag))
+        t, _ = timed(run, min_s=2.0, min_reps=2)
+        whole.setdefault(name, []).append(t)
+        whole[name + " launches"] = launches(run)
+        torch.cuda.empty_cache()
+    log("gates: whole %d-bit adder (circuit + decrypt of %d arrays), %d lanes: three-call carries %8.2f ms (%d launches) | "
+        "one-call carries %8.2f ms (%d launches) | %.2fx" % (
+            bits, bits + 1, lanes, min(whole["three calls"]) * 1e3, whole["three calls launches"],
+            min(whole["one call"]) * 1e3, whole["one call launches"], min(whole["three calls"]) / min(whole["one call"])))
+
+
 def sweep(ctx, total_bytes, sizes_kb):
     L = ctx.L
     for kb in sizes_kb:
@@ -252,11 +333,15 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default="")
     ap.add_argument("--quick", action="store_true", help="small sizes (a check of the script, not a measurement)")
-    ap.add_argument("--only", default="small,mixed,adder,sweep")
+    ap.add_argument("--only", default="small,mixed,adder,gates,sweep")
     args = ap.parse_args()
     torch.cuda.set_device(0)
     eng.init(0)
-    st = torch.cuda.current_stream()
+    # One NON-default torch stream for the library's work, torch's copies and the timing events.  (torch's default
+    # stream has the handle 0, and csgn_set_stream(0) selects the library's own non-blocking stream, which events
+    # recorded on torch's default stream would not wait for.)
+    st = torch.cuda.Stream()
+    torch.cuda.set_stream(st)
     eng.set_stream(st.cuda_stream)
     gpu_header()
     rng = np.random.default_rng(1)
@@ -269,6 +354,11 @@ def main():
         mixed(ctx, key, rng, (64 << 20) if args.quick else (1 << 30))
     if "adder" in only:
         adder(ctx, key, rng, 256 if args.quick else 4096)
+    if "gates" in only:
+        if hasattr(eng._lib(), "csgn_seg_mul_sum"):
+            gates(ctx, key, rng, 256 if args.quick else 4096, 8 if args.quick else 12)
+        else:
+            log("gates: skipped, %s has no csgn_seg_mul_sum" % os.environ.get("CSGN_LIBRARY", "this build"))
     if "sweep" in only:
         sweep(ctx, (64 << 20) if args.quick else (1 << 30),
               [64, 256] if args.quick else [64, 256, 1024, 4096, 16384, 65536])

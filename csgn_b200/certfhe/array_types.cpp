@@ -3,6 +3,7 @@
 //   CiphertextArray(vector)   -> csgn_concat_n
 //   operator* / operator+     -> csgn_seg_mul / csgn_seg_concat
 //   sumOfProducts             -> csgn_seg_mul_sum
+//   compactSumOfProducts, compact, Ciphertext::compact -> csgn_seg_mul_sum_compact (min_bits = D)
 //   gather                    -> csgn_seg_gather
 //   applyPermutation          -> csgn_permute on the storage (a permutation acts on every block by itself)
 //   encryptArray / decryptArray -> csgn_encrypt_batch / csgn_seg_decrypt
@@ -87,22 +88,23 @@ CiphertextArray CiphertextArray::operator+(const CiphertextArray &c) const {
     return CiphertextArray(out, off, context);
 }
 
-CiphertextArray CiphertextArray::sumOfProducts(const std::vector<std::pair<CiphertextArray, CiphertextArray>> &products,
-                                               const std::vector<CiphertextArray> &terms) {
+CiphertextArray CiphertextArray::gate(const std::vector<std::pair<CiphertextArray, CiphertextArray>> &products,
+                                      const std::vector<CiphertextArray> &terms, bool compact) {
+    const std::string who = compact ? "CiphertextArray::compactSumOfProducts" : "CiphertextArray::sumOfProducts";
     std::vector<const CiphertextArray *> all;
     for (size_t i = 0; i < products.size(); ++i) {
         all.push_back(&products[i].first);
         all.push_back(&products[i].second);
     }
     for (size_t i = 0; i < terms.size(); ++i) all.push_back(&terms[i]);
-    if (all.empty()) throw Error("CiphertextArray::sumOfProducts: no products and no terms");
+    if (all.empty()) throw Error(who + ": no products and no terms");
     const CiphertextArray &x0 = *all[0];
     for (size_t i = 1; i < all.size(); ++i) {
         if (all[i]->size() != x0.size())
-            throw Error("CiphertextArray::sumOfProducts: arrays of " + to_string(x0.size()) + " and " +
+            throw Error(who + ": arrays of " + to_string(x0.size()) + " and " +
                         to_string(all[i]->size()) + " elements");
         if (all[i]->context.getN() != x0.context.getN() || all[i]->context.getD() != x0.context.getD())
-            throw Error("CiphertextArray::sumOfProducts: arrays of different contexts");
+            throw Error(who + ": arrays of different contexts");
     }
     std::vector<const csgn_buf *> a, b, c;
     std::vector<const uint64_t *> ao, bo, co;
@@ -118,11 +120,30 @@ CiphertextArray CiphertextArray::sumOfProducts(const std::vector<std::pair<Ciphe
     }
     std::vector<uint64_t> off(x0.size() + 1);
     csgn_buf *out = nullptr;
-    glue::check(csgn_seg_mul_sum(a.data(), ao.data(), b.data(), bo.data(), (uint32_t)products.size(), c.data(), co.data(),
-                                 (uint32_t)terms.size(), x0.size(), off.data(), &out),
-                "csgn_seg_mul_sum");
+    if (compact)
+        glue::check(csgn_seg_mul_sum_compact(a.data(), ao.data(), b.data(), bo.data(), (uint32_t)products.size(),
+                                             c.data(), co.data(), (uint32_t)terms.size(), x0.size(),
+                                             (uint32_t)x0.context.getD(), off.data(), &out),
+                    "csgn_seg_mul_sum_compact");
+    else
+        glue::check(csgn_seg_mul_sum(a.data(), ao.data(), b.data(), bo.data(), (uint32_t)products.size(), c.data(),
+                                     co.data(), (uint32_t)terms.size(), x0.size(), off.data(), &out),
+                    "csgn_seg_mul_sum");
     return CiphertextArray(out, off, x0.context);
 }
+
+CiphertextArray CiphertextArray::sumOfProducts(const std::vector<std::pair<CiphertextArray, CiphertextArray>> &products,
+                                               const std::vector<CiphertextArray> &terms) {
+    return gate(products, terms, false);
+}
+
+CiphertextArray CiphertextArray::compactSumOfProducts(
+    const std::vector<std::pair<CiphertextArray, CiphertextArray>> &products, const std::vector<CiphertextArray> &terms) {
+    return gate(products, terms, true);
+}
+
+CiphertextArray CiphertextArray::compact() const { return gate({}, {*this}, true); }
+
 
 CiphertextArray CiphertextArray::gather(const std::vector<uint64_t> &idx) const {
     std::vector<uint64_t> off(idx.size() + 1);
@@ -139,6 +160,25 @@ CiphertextArray CiphertextArray::applyPermutation(const Permutation &permutation
     else
         glue::check(csgn_permute(storage.get(), permutation.deviceMap(context.getN()), 0, &out), "csgn_permute");
     return CiphertextArray(out, offsets, context);
+}
+
+Ciphertext Ciphertext::compact() const {
+    const csgn_buf *b = deviceBuffer();   // writes a pending product; the call makes a lazy sum dense
+    if (!b) return *this;
+    if (!certFHEcontext) throw Error("Ciphertext::compact: no context");
+    const csgn_buf *one[1] = {b};
+    const uint64_t off[2] = {0, csgn_buf_blocks(b)};
+    const uint64_t *offs[1] = {off};
+    uint64_t out_off[2];
+    csgn_buf *res = nullptr;
+    glue::check(csgn_seg_mul_sum_compact(nullptr, nullptr, nullptr, nullptr, 0, one, offs, 1, 1,
+                                         (uint32_t)certFHEcontext->getD(), out_off, &res),
+                "csgn_seg_mul_sum_compact");
+    Ciphertext out;
+    out.certFHEcontext = new Context(*certFHEcontext);
+    out.dev = adopt(res);
+    out.sharded = sharded;
+    return out;
 }
 
 CiphertextArray SecretKey::encryptArray(const unsigned char *bits, uint64_t n, uint64_t seed) {

@@ -250,6 +250,10 @@ public:
     // through pinned staging (csgn_buf_save / csgn_buf_load).  The reference has no serialisation.
     void save(const std::string &path) const;
     static Ciphertext load(const std::string &path);
+    // The blocks with at least D set bits, in order (csgn_seg_mul_sum_compact): no key of the context can satisfy
+    // the others, so the satisfied-block count is the same under every key.  A pending product or lazy sum is made
+    // dense first; an empty ciphertext stays empty.
+    Ciphertext compact() const;
     // A sharded ciphertext as one file per rank, `<prefix>.shard<rank>of<world>` (csgn_buf_save_shard): every rank
     // writes / reads its own blocks, no collective.  loadSharded returns a ciphertext marked sharded.
     void saveSharded(const std::string &prefix) const;
@@ -320,6 +324,8 @@ class CiphertextArray {
     std::vector<uint64_t> offsets;   // n + 1 block offsets
     Context context;
     CiphertextArray(csgn_buf *storage, const std::vector<uint64_t> &offsets, const Context &context);
+    static CiphertextArray gate(const std::vector<std::pair<CiphertextArray, CiphertextArray>> &products,
+                                const std::vector<CiphertextArray> &terms, bool compact);
     friend class SecretKey;
 
 public:
@@ -341,6 +347,13 @@ public:
     // or contexts, or when both lists are empty.
     static CiphertextArray sumOfProducts(const std::vector<std::pair<CiphertextArray, CiphertextArray>> &products,
                                          const std::vector<CiphertextArray> &terms = {});
+    // sumOfProducts keeping only the blocks with at least D set bits (csgn_seg_mul_sum_compact, min_bits = D of the
+    // context): no key of the context can satisfy the others, so every element decrypts as before, with the same
+    // satisfied-block count, under every key.  Throws as sumOfProducts does.  compact() drops them from this array.
+    static CiphertextArray compactSumOfProducts(
+        const std::vector<std::pair<CiphertextArray, CiphertextArray>> &products,
+        const std::vector<CiphertextArray> &terms = {});
+    CiphertextArray compact() const;
 
     const std::vector<uint64_t> &getOffsets() const;
     const csgn_buf *deviceBuffer() const;

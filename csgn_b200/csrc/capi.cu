@@ -666,6 +666,18 @@ int stage_to_device(const void *host, size_t bytes, void **out) {
     return CSGN_OK;
 }
 
+int read_back(void *host, const void *d, size_t bytes) {
+    if (bytes == 0) return CSGN_OK;
+    StagingSlot *sl = bytes <= kStagingMaxOne ? take_staging(bytes) : nullptr;
+    cudaError_t e = cudaMemcpyAsync(sl ? sl->p : host, d, bytes, cudaMemcpyDeviceToHost, g.stream);
+    if (e == cudaSuccess && sl) e = cudaEventRecord(sl->done, g.stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(g.stream);
+    if (e != cudaSuccess) return cuda_fail(e, "table read-back");
+    note_synced(g.stream);
+    if (sl) memcpy(host, sl->p, bytes);
+    return CSGN_OK;
+}
+
 }  // namespace detail
 }  // namespace csgn
 

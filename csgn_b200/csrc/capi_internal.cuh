@@ -196,6 +196,8 @@ bool folds_overlap();
 int stage_to_device(const void *host, size_t bytes, void **out);
 // The same copy into device memory `d` the caller already holds (a table that contains its own device address).
 int stage_into(void *d, const void *host, size_t bytes);
+// `bytes` of device memory `d` to `host` on the current stream, through the pinned staging, and wait for the copy.
+int read_back(void *host, const void *d, size_t bytes);
 
 // Scope of one batch call: item i runs with the work stream set to way i % n, where way 0 is the caller's own stream
 // and ways 1.. are the library's side lanes, forked from the caller's stream on construction; join() makes the

@@ -55,15 +55,24 @@ struct DevTable {
 // (items whose left operand is the all-ones block at the head of the staged table).  Small pieces become items packed
 // into tasks of about task_words(small_words) words; a long term is cut into items of about one task each.  A piece of
 // large_words() or more goes straight into its position: launch_mul for a product, a device-to-device copy for a term.
+// The compacting form (out null, then compact()) has no large pieces, since launch_mul and the copy write every block:
+// every piece becomes items of about one task, a long row being cut into column ranges.
 class SegMulWork {
 public:
     SegMulWork(uint32_t L, uint64_t small_words, csgn_buf *out)
-        : L_(L), large_(large_words()), target_(task_words(small_words)), out_(out) {}
+        : L_(L), large_(out ? large_words() : UINT64_MAX), target_(task_words(small_words)), out_(out) {}
 
     void product(const uint64_t *a, uint64_t t1, const uint64_t *b, uint64_t t2) {
         if (t1 && t2 && e_ == cudaSuccess) {
             if (t1 * t2 * L_ >= large_) {
                 e_ = launch_mul(a, t1, b, t2, L_, out_->d + pos_ * L_, g.stream);
+            } else if (!out_ && t2 * L_ > target_) {
+                const uint64_t cols = std::max<uint64_t>(1, target_ / L_);
+                for (uint64_t r = 0; r < t1; ++r)
+                    for (uint64_t j = 0; j < t2; j += cols) {
+                        const uint64_t m = std::min(cols, t2 - j);
+                        add({a + r * L_, b + j * L_, pos_ + r * t2 + j, (uint32_t)m, 1}, m * L_);
+                    }
             } else {
                 const uint64_t row = t2 * L_, step = std::max<uint64_t>(1, target_ / row);
                 for (uint64_t r = 0; r < t1; r += step) {
@@ -95,18 +104,94 @@ public:
     int launch() {
         if (e_ != cudaSuccess) return cuda_fail(e_, "grouped multiply kernel");
         if (items_.empty()) return CSGN_OK;
+        Table tb;
+        int rc = stage(0, &tb);
+        if (rc != CSGN_OK) return rc;
+        const bool units16 = tb.units16 && (reinterpret_cast<uintptr_t>(out_->d) & 15u) == 0;
+        const cudaError_t e = launch_seg_mul(out_->d, L_, units16, tb.items, tb.tasks, n_tasks(), g.stream);
+        return e == cudaSuccess ? CSGN_OK : cuda_fail(e, "grouped multiply kernel");
+    }
+
+    // The compacting form: count the blocks of at least min_bits set bits of every item (one launch), read the counts
+    // back (the call's one host synchronisation), allocate exactly those blocks and write them (a second launch), each
+    // item from the total of the items before it, which keeps the blocks of every element in order.  oo: the offsets
+    // of the n elements without compaction.  out_off and *out on success only.
+    int compact(uint32_t min_bits, const std::vector<uint64_t> &oo, uint64_t *out_off, csgn_buf **out) {
+        const uint64_t n = oo.size() - 1;
+        const size_t ni = items_.size();
+        std::vector<uint64_t> off(n + 1, 0), base(ni);
+        csgn_buf *res = nullptr;
+        if (ni == 0) {
+            const int rc = new_buf(0, L_, 0, &res);
+            if (rc != CSGN_OK) return rc;
+        } else {
+            // after the table: the items' output bases (uint64), then their counts (uint32)
+            Table tb;
+            int rc = stage(ni * (sizeof(uint64_t) + sizeof(uint32_t)), &tb);
+            if (rc != CSGN_OK) return rc;
+            uint64_t *d_base = reinterpret_cast<uint64_t *>(tb.extra);
+            uint32_t *d_live = reinterpret_cast<uint32_t *>(d_base + ni);
+            cudaError_t e = launch_seg_mul_live(nullptr, L_, tb.units16, tb.items, tb.tasks, n_tasks(), min_bits,
+                                                d_live, nullptr, g.stream);
+            if (e != cudaSuccess) return cuda_fail(e, "grouped multiply kernel (count)");
+            std::vector<uint32_t> live(ni);
+            rc = read_back(live.data(), d_live, ni * sizeof(uint32_t));
+            if (rc != CSGN_OK) return rc;
+            uint64_t total = 0;
+            for (size_t i = 0, k = 0; i < ni; ++i) {
+                while (oo[k + 1] <= items_[i].out) ++k;           // element of item i (items are non-empty)
+                base[i] = total;
+                total += live[i];
+                off[k + 1] += live[i];
+            }
+            for (uint64_t k = 0; k < n; ++k) off[k + 1] += off[k];
+            rc = new_buf(total, L_, 0, &res);
+            if (rc != CSGN_OK) return rc;
+            acquire_write(res);
+            if (total) {
+                rc = stage_into(d_base, base.data(), ni * sizeof(uint64_t));
+                if (rc == CSGN_OK) {
+                    const bool units16 = tb.units16 && (reinterpret_cast<uintptr_t>(res->d) & 15u) == 0;
+                    e = launch_seg_mul_live(res->d, L_, units16, tb.items, tb.tasks, n_tasks(), min_bits, nullptr,
+                                            d_base, g.stream);
+                    if (e != cudaSuccess) rc = cuda_fail(e, "grouped multiply kernel (write)");
+                }
+                if (rc != CSGN_OK) {
+                    csgn_buf_free(res);
+                    return rc;
+                }
+            }
+        }
+        memcpy(out_off, off.data(), (n + 1) * sizeof(uint64_t));
+        *out = res;
+        return CSGN_OK;
+    }
+
+private:
+    // The staged table on the device, released in stream order after the launches that read it.
+    struct Table {
+        DevTable t;
+        const SegMulItem *items = nullptr;
+        const uint32_t *tasks = nullptr;
+        uint8_t *extra = nullptr;   // `extra` bytes after the table, 8-byte aligned, left to the caller
+        bool units16 = false;       // 16-byte units fit the operands and the table (not yet the output)
+    };
+
+    uint32_t n_tasks() const { return (uint32_t)(tasks_.size() - 1); }
+
+    // table: [the all-ones block, L words rounded up to 16 bytes, when there are terms] [items] [task bounds]
+    int stage(size_t extra, Table *tb) {
         if (tasks_.back() != items_.size()) tasks_.push_back((uint32_t)items_.size());
         if (items_.size() >= UINT32_MAX) return fail(CSGN_ERR_INVALID_ARGUMENT, "too many work items");
-        // table: [the all-ones block, L words rounded up to 16 bytes, when there are terms] [items] [task bounds]
         const size_t head = terms_ ? (size_t)((L_ + 1) & ~1u) * sizeof(uint64_t) : 0;
         const size_t item_bytes = items_.size() * sizeof(SegMulItem);
         const size_t bytes = head + item_bytes + tasks_.size() * sizeof(uint32_t);
+        const size_t words = (bytes + 7) / 8;
         uint64_t *d = nullptr;
-        int rc = dev_alloc((bytes + 7) / 8, &d);
+        int rc = dev_alloc(words + (extra + 7) / 8, &d);
         if (rc != CSGN_OK) return rc;
-        DevTable t;
-        t.d = d;
-        uintptr_t addr = reinterpret_cast<uintptr_t>(out_->d) | reinterpret_cast<uintptr_t>(d);
+        tb->t.d = d;
+        uintptr_t addr = reinterpret_cast<uintptr_t>(d);
         std::vector<uint8_t> tab(bytes);
         std::fill_n(reinterpret_cast<uint64_t *>(tab.data()), head / sizeof(uint64_t), ~0ull);
         SegMulItem *it = reinterpret_cast<SegMulItem *>(tab.data() + head);
@@ -118,14 +203,13 @@ public:
         memcpy(tab.data() + head + item_bytes, tasks_.data(), tasks_.size() * sizeof(uint32_t));
         rc = stage_into(d, tab.data(), bytes);
         if (rc != CSGN_OK) return rc;
-        const SegMulItem *d_items = reinterpret_cast<const SegMulItem *>(reinterpret_cast<const uint8_t *>(d) + head);
-        const cudaError_t e = launch_seg_mul(out_->d, L_, !(L_ & 1u) && (addr & 15u) == 0, d_items,
-                                             reinterpret_cast<const uint32_t *>(d_items + items_.size()),
-                                             (uint32_t)(tasks_.size() - 1), g.stream);
-        return e == cudaSuccess ? CSGN_OK : cuda_fail(e, "grouped multiply kernel");
+        tb->items = reinterpret_cast<const SegMulItem *>(reinterpret_cast<const uint8_t *>(d) + head);
+        tb->tasks = reinterpret_cast<const uint32_t *>(tb->items + items_.size());
+        tb->extra = reinterpret_cast<uint8_t *>(d + words);
+        tb->units16 = !(L_ & 1u) && (addr & 15u) == 0;
+        return CSGN_OK;
     }
 
-private:
     void add(const SegMulItem &m, uint64_t words) {
         items_.push_back(m);
         in_task_ += words;
@@ -180,6 +264,109 @@ int gather_into_new(uint64_t blocks, uint32_t L, const std::vector<const uint64_
         return rc;
     }
     *out = c;
+    return CSGN_OK;
+}
+
+// csgn_seg_mul_sum, and with compact csgn_seg_mul_sum_compact: the same checks, items and output order, plus
+// 1 <= min_bits <= 64 L.
+int mul_sum(const csgn_buf *const *a, const uint64_t *const *a_off, const csgn_buf *const *b,
+            const uint64_t *const *b_off, uint32_t n_products, const csgn_buf *const *c, const uint64_t *const *c_off,
+            uint32_t n_terms, uint64_t n, bool compact, uint32_t min_bits, uint64_t *out_off, csgn_buf **out) {
+    if (!out || !out_off) return fail(CSGN_ERR_INVALID_ARGUMENT, "null argument");
+    if (n_products == 0 && n_terms == 0) return fail(CSGN_ERR_INVALID_ARGUMENT, "no products and no terms");
+    if (n_products && (!a || !a_off || !b || !b_off)) return fail(CSGN_ERR_INVALID_ARGUMENT, "null product arrays");
+    if (n_terms && (!c || !c_off)) return fail(CSGN_ERR_INVALID_ARGUMENT, "null term arrays");
+    // operand j: the left operands of the products, their right operands, then the terms
+    const uint64_t p = n_products, m = p * 2 + n_terms;
+    auto op = [&](uint64_t j) { return j < p ? a[j] : j < 2 * p ? b[j - p] : c[j - 2 * p]; };
+    auto off = [&](uint64_t j) { return j < p ? a_off[j] : j < 2 * p ? b_off[j - p] : c_off[j - 2 * p]; };
+    auto name = [&](uint64_t j) {
+        char s[48];
+        snprintf(s, sizeof s, "%s %llu", j < p ? "left operand" : j < 2 * p ? "right operand" : "term",
+                 (unsigned long long)(j < p ? j : j < 2 * p ? j - p : j - 2 * p));
+        return std::string(s);
+    };
+    for (uint64_t j = 0; j < m; ++j)
+        if (!op(j)) return fail(CSGN_ERR_INVALID_ARGUMENT, "null %s", name(j).c_str());
+    const uint32_t L = op(0)->L;
+    for (uint64_t j = 1; j < m; ++j)
+        if (op(j)->L != L)
+            return fail(CSGN_ERR_SHAPE_MISMATCH, "words per block differ (%s: %u vs %s: %u)", name(0).c_str(), L,
+                        name(j).c_str(), op(j)->L);
+    if (compact && (min_bits < 1 || min_bits > 64ull * L))
+        return fail(CSGN_ERR_INVALID_ARGUMENT, "min_bits = %u outside [1, %llu] (64 bits of %u words)", min_bits,
+                    64ull * L, L);
+    for (uint64_t j = 0; j < m; ++j) {
+        const int rc = check_offsets(op(j), off(j), n, name(j).c_str());
+        if (rc != CSGN_OK) return rc;
+    }
+    std::vector<uint64_t> oo(n + 1, 0);
+    for (uint64_t k = 0; k < n; ++k) {
+        uint64_t o = oo[k];
+        for (uint64_t i = 0; i < p; ++i) {
+            const uint64_t t1 = a_off[i][k + 1] - a_off[i][k], t2 = b_off[i][k + 1] - b_off[i][k];
+            if (t2 && t1 > UINT64_MAX / t2)
+                return fail(CSGN_ERR_INVALID_ARGUMENT, "product %llu of element %llu overflows", (unsigned long long)i,
+                            (unsigned long long)k);
+            if (o + t1 * t2 < o) return fail(CSGN_ERR_INVALID_ARGUMENT, "output block count overflows");
+            o += t1 * t2;
+        }
+        for (uint64_t i = 0; i < n_terms; ++i) {
+            const uint64_t t = c_off[i][k + 1] - c_off[i][k];
+            if (o + t < o) return fail(CSGN_ERR_INVALID_ARGUMENT, "output block count overflows");
+            o += t;
+        }
+        oo[k + 1] = o;
+    }
+    int rc = check_blocks(oo[n], L);
+    if (rc != CSGN_OK) return rc;
+    // every distinct buffer once; the automatic lane follows the two largest
+    std::vector<const csgn_buf *> bufs;
+    for (uint64_t j = 0; j < m; ++j) bufs.push_back(op(j));
+    std::sort(bufs.begin(), bufs.end());
+    bufs.erase(std::unique(bufs.begin(), bufs.end()), bufs.end());
+    std::stable_sort(bufs.begin(), bufs.end(),
+                     [](const csgn_buf *x, const csgn_buf *y) { return x->n_blocks > y->n_blocks; });
+    AutoLane lane(bufs[0], bufs.size() > 1 ? bufs[1] : nullptr);
+    for (const csgn_buf *x : bufs) {
+        rc = need_dense(x);
+        if (rc != CSGN_OK) return rc;
+    }
+    csgn_buf *res = nullptr;
+    if (!compact) {
+        rc = new_buf(oo[n], L, 0, &res);
+        if (rc != CSGN_OK) return rc;
+    }
+    for (const csgn_buf *x : bufs) acquire_read(x);
+    if (res) acquire_write(res);
+    const uint64_t large = compact ? UINT64_MAX : large_words();
+    uint64_t small_words = 0;
+    for (uint64_t k = 0; k < n; ++k) {
+        for (uint64_t i = 0; i < p; ++i) {
+            const uint64_t w = (a_off[i][k + 1] - a_off[i][k]) * (b_off[i][k + 1] - b_off[i][k]) * L;
+            if (w < large) small_words += w;
+        }
+        for (uint64_t i = 0; i < n_terms; ++i) {
+            const uint64_t w = (c_off[i][k + 1] - c_off[i][k]) * L;
+            if (w < large) small_words += w;
+        }
+    }
+    // output order: element by element, its products first, then its terms
+    SegMulWork work(L, small_words, res);
+    for (uint64_t k = 0; k < n; ++k) {
+        for (uint64_t i = 0; i < p; ++i)
+            work.product(a[i]->d + a_off[i][k] * L, a_off[i][k + 1] - a_off[i][k], b[i]->d + b_off[i][k] * L,
+                         b_off[i][k + 1] - b_off[i][k]);
+        for (uint64_t i = 0; i < n_terms; ++i) work.term(c[i]->d + c_off[i][k] * L, c_off[i][k + 1] - c_off[i][k]);
+    }
+    if (compact) return work.compact(min_bits, oo, out_off, out);
+    rc = work.launch();
+    if (rc != CSGN_OK) {
+        csgn_buf_free(res);
+        return rc;
+    }
+    memcpy(out_off, oo.data(), (n + 1) * sizeof(uint64_t));
+    *out = res;
     return CSGN_OK;
 }
 
@@ -238,96 +425,15 @@ int csgn_seg_mul_sum(const csgn_buf *const *a, const uint64_t *const *a_off, con
                      const uint64_t *const *b_off, uint32_t n_products, const csgn_buf *const *c,
                      const uint64_t *const *c_off, uint32_t n_terms, uint64_t n, uint64_t *out_off, csgn_buf **out) {
     NEED_INIT();
-    if (!out || !out_off) return fail(CSGN_ERR_INVALID_ARGUMENT, "null argument");
-    if (n_products == 0 && n_terms == 0) return fail(CSGN_ERR_INVALID_ARGUMENT, "no products and no terms");
-    if (n_products && (!a || !a_off || !b || !b_off)) return fail(CSGN_ERR_INVALID_ARGUMENT, "null product arrays");
-    if (n_terms && (!c || !c_off)) return fail(CSGN_ERR_INVALID_ARGUMENT, "null term arrays");
-    // operand j: the left operands of the products, their right operands, then the terms
-    const uint64_t p = n_products, m = p * 2 + n_terms;
-    auto op = [&](uint64_t j) { return j < p ? a[j] : j < 2 * p ? b[j - p] : c[j - 2 * p]; };
-    auto off = [&](uint64_t j) { return j < p ? a_off[j] : j < 2 * p ? b_off[j - p] : c_off[j - 2 * p]; };
-    auto name = [&](uint64_t j) {
-        char s[48];
-        snprintf(s, sizeof s, "%s %llu", j < p ? "left operand" : j < 2 * p ? "right operand" : "term",
-                 (unsigned long long)(j < p ? j : j < 2 * p ? j - p : j - 2 * p));
-        return std::string(s);
-    };
-    for (uint64_t j = 0; j < m; ++j)
-        if (!op(j)) return fail(CSGN_ERR_INVALID_ARGUMENT, "null %s", name(j).c_str());
-    const uint32_t L = op(0)->L;
-    for (uint64_t j = 1; j < m; ++j)
-        if (op(j)->L != L)
-            return fail(CSGN_ERR_SHAPE_MISMATCH, "words per block differ (%s: %u vs %s: %u)", name(0).c_str(), L,
-                        name(j).c_str(), op(j)->L);
-    for (uint64_t j = 0; j < m; ++j) {
-        const int rc = check_offsets(op(j), off(j), n, name(j).c_str());
-        if (rc != CSGN_OK) return rc;
-    }
-    std::vector<uint64_t> oo(n + 1, 0);
-    for (uint64_t k = 0; k < n; ++k) {
-        uint64_t o = oo[k];
-        for (uint64_t i = 0; i < p; ++i) {
-            const uint64_t t1 = a_off[i][k + 1] - a_off[i][k], t2 = b_off[i][k + 1] - b_off[i][k];
-            if (t2 && t1 > UINT64_MAX / t2)
-                return fail(CSGN_ERR_INVALID_ARGUMENT, "product %llu of element %llu overflows", (unsigned long long)i,
-                            (unsigned long long)k);
-            if (o + t1 * t2 < o) return fail(CSGN_ERR_INVALID_ARGUMENT, "output block count overflows");
-            o += t1 * t2;
-        }
-        for (uint64_t i = 0; i < n_terms; ++i) {
-            const uint64_t t = c_off[i][k + 1] - c_off[i][k];
-            if (o + t < o) return fail(CSGN_ERR_INVALID_ARGUMENT, "output block count overflows");
-            o += t;
-        }
-        oo[k + 1] = o;
-    }
-    int rc = check_blocks(oo[n], L);
-    if (rc != CSGN_OK) return rc;
-    // every distinct buffer once; the automatic lane follows the two largest
-    std::vector<const csgn_buf *> bufs;
-    for (uint64_t j = 0; j < m; ++j) bufs.push_back(op(j));
-    std::sort(bufs.begin(), bufs.end());
-    bufs.erase(std::unique(bufs.begin(), bufs.end()), bufs.end());
-    std::stable_sort(bufs.begin(), bufs.end(),
-                     [](const csgn_buf *x, const csgn_buf *y) { return x->n_blocks > y->n_blocks; });
-    AutoLane lane(bufs[0], bufs.size() > 1 ? bufs[1] : nullptr);
-    for (const csgn_buf *x : bufs) {
-        rc = need_dense(x);
-        if (rc != CSGN_OK) return rc;
-    }
-    csgn_buf *res = nullptr;
-    rc = new_buf(oo[n], L, 0, &res);
-    if (rc != CSGN_OK) return rc;
-    for (const csgn_buf *x : bufs) acquire_read(x);
-    acquire_write(res);
-    const uint64_t large = large_words();
-    uint64_t small_words = 0;
-    for (uint64_t k = 0; k < n; ++k) {
-        for (uint64_t i = 0; i < p; ++i) {
-            const uint64_t w = (a_off[i][k + 1] - a_off[i][k]) * (b_off[i][k + 1] - b_off[i][k]) * L;
-            if (w < large) small_words += w;
-        }
-        for (uint64_t i = 0; i < n_terms; ++i) {
-            const uint64_t w = (c_off[i][k + 1] - c_off[i][k]) * L;
-            if (w < large) small_words += w;
-        }
-    }
-    // output order: element by element, its products first, then its terms
-    SegMulWork work(L, small_words, res);
-    for (uint64_t k = 0; k < n; ++k) {
-        for (uint64_t i = 0; i < p; ++i)
-            work.product(a[i]->d + a_off[i][k] * L, a_off[i][k + 1] - a_off[i][k], b[i]->d + b_off[i][k] * L,
-                         b_off[i][k + 1] - b_off[i][k]);
-        for (uint64_t i = 0; i < n_terms; ++i) work.term(c[i]->d + c_off[i][k] * L, c_off[i][k + 1] - c_off[i][k]);
-    }
-    rc = work.launch();
-    if (rc != CSGN_OK) {
-        csgn_buf_free(res);
-        return rc;
-    }
-    memcpy(out_off, oo.data(), (n + 1) * sizeof(uint64_t));
-    *out = res;
-    return CSGN_OK;
+    return mul_sum(a, a_off, b, b_off, n_products, c, c_off, n_terms, n, false, 0, out_off, out);
+}
+
+int csgn_seg_mul_sum_compact(const csgn_buf *const *a, const uint64_t *const *a_off, const csgn_buf *const *b,
+                             const uint64_t *const *b_off, uint32_t n_products, const csgn_buf *const *c,
+                             const uint64_t *const *c_off, uint32_t n_terms, uint64_t n, uint32_t min_bits,
+                             uint64_t *out_off, csgn_buf **out) {
+    NEED_INIT();
+    return mul_sum(a, a_off, b, b_off, n_products, c, c_off, n_terms, n, true, min_bits, out_off, out);
 }
 
 int csgn_seg_concat(const csgn_buf *a, const uint64_t *a_off, const csgn_buf *b, const uint64_t *b_off, uint64_t n,

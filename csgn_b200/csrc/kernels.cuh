@@ -68,6 +68,12 @@ struct SegMulItem {
 static_assert(sizeof(SegMulItem) == 32, "SegMulItem is read as one 32-byte record");
 cudaError_t launch_seg_mul(uint64_t *out, uint32_t L, bool units16, const SegMulItem *items, const uint32_t *tasks,
                            uint32_t n_tasks, cudaStream_t stream);
+// The two passes of a compacting grouped multiply over the same items (a block survives when its L words hold at least
+// min_bits set bits).  With `live`: live[k] = surviving blocks of item k, nothing else written.  Without: the surviving
+// blocks of item k, in order, to blocks base[k], base[k] + 1, ... of `out`.  One launch each.
+cudaError_t launch_seg_mul_live(uint64_t *out, uint32_t L, bool units16, const SegMulItem *items,
+                                const uint32_t *tasks, uint32_t n_tasks, uint32_t min_bits, uint32_t *live,
+                                const uint64_t *base, cudaStream_t stream);
 // Segmented decrypt: a warp task walks blocks [first, end), which belong to elements [elem, elem_last] (element e =
 // blocks [off[e], off[e+1]), off on the device), and adds each element's satisfied-block count to counts[e] (zeroed
 // by the caller in stream order).  One launch.

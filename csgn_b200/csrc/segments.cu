@@ -28,23 +28,93 @@ __device__ __forceinline__ uint4 vand(const uint4 x, const uint4 y) {
     return make_uint4(x.x & y.x, x.y & y.y, x.z & y.z, x.w & y.w);
 }
 __device__ __forceinline__ uint2 vand(const uint2 x, const uint2 y) { return make_uint2(x.x & y.x, x.y & y.y); }
+__device__ __forceinline__ uint32_t vpopc(const uint4 x) { return __popc(x.x) + __popc(x.y) + __popc(x.z) + __popc(x.w); }
+__device__ __forceinline__ uint32_t vpopc(const uint2 x) { return __popc(x.x) + __popc(x.y); }
+
+// Modes of the grouped multiply: kSegPlain writes every block at its item's `out`; kSegCount writes, per item, the
+// number of its blocks with at least min_bits set bits (live[it]); kSegWriteLive writes only those blocks, in order,
+// from block base[it] on.
+enum SegMode { kSegPlain, kSegCount, kSegWriteLive };
 
 // ---------------------------------------------------------------------------------------
 // grouped multiply: a warp task is a run of items; an item is the `rows` blocks at address a (rows of one element's
 // left operand, or the all-ones block of a plain term) times the t2 blocks at address b, written to block `out` on.
 // Lane l holds unit w = l % U of block j = l / U of each warp step (U < 32), or units l, l+32, ... of one block
 // (U >= 32).
+// The counting modes walk an item's blocks in warp steps that every lane takes (no early return, no per-lane loop
+// bound), because each step votes with the full mask: a lane with no block (past t2, or beyond the last whole block of
+// a step) counts 0 set bits and is not live.
+// The counting modes ask for 3 resident CTAs per SM: left to its own register target, ptxas spills in them.
 // ---------------------------------------------------------------------------------------
-template <typename VT>
-__global__ void __launch_bounds__(kSegThreads)
+template <typename VT, SegMode MODE>
+__global__ void __launch_bounds__(kSegThreads, MODE == kSegPlain ? 0 : 3)
 seg_mul_kernel(VT *__restrict__ out, const uint32_t U, const SegMulItem *__restrict__ items,
-               const uint32_t *__restrict__ tasks, const uint32_t n_tasks) {
+               const uint32_t *__restrict__ tasks, const uint32_t n_tasks, const uint32_t min_bits,
+               uint32_t *__restrict__ live, const uint64_t *__restrict__ base) {
     const uint32_t lane = threadIdx.x & 31u;
     const uint32_t G = U >= 32u ? 1u : 32u / U;                // blocks per warp step
     const uint32_t w0 = U >= 32u ? lane : lane % U;
     const uint32_t j0 = U >= 32u ? 0u : lane / U;
     const uint32_t warps = gridDim.x * (blockDim.x >> 5);
     pdl_enter();
+    if constexpr (MODE != kSegPlain) {
+        // group of this lane (U < 32): lanes [gl, gl + U); the scan just before gl and at its last lane give its total
+        const uint32_t gl = j0 * U, glast = min(gl + U - 1u, 31u);
+        const uint32_t below = (1u << gl) - 1u;                // leaders of the groups before this one
+        for (uint32_t t = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); t < n_tasks; t += warps) {
+            const uint32_t it_end = __ldg(tasks + t + 1);
+            for (uint32_t it = __ldg(tasks + t); it < it_end; ++it) {
+                const SegMulItem m = items[it];
+                const VT *a = reinterpret_cast<const VT *>(m.a), *b = reinterpret_cast<const VT *>(m.b);
+                uint64_t pos = MODE == kSegWriteLive ? __ldg(base + it) : 0;   // next surviving block of this item
+                uint32_t running = 0;
+                for (uint32_t r = 0; r < m.rows; ++r) {
+                    const VT *arow = a + (uint64_t)r * U;
+                    if (U < 32u) {
+                        VT x = {};
+                        if (j0 < G) x = __ldg(arow + w0);
+                        for (uint32_t js = 0; js < m.t2; js += G) {
+                            const uint32_t j = js + j0;
+                            const bool has = j0 < G && j < m.t2;
+                            VT v = {};
+                            if (has) v = vand(x, __ldg(b + (uint64_t)j * U + w0));
+                            // inclusive scan of the lanes' set bits; a group's total is a difference of two scans
+                            uint32_t s = vpopc(v);
+#pragma unroll
+                            for (uint32_t d = 1; d < 32u; d <<= 1) {
+                                const uint32_t y = __shfl_up_sync(0xffffffffu, s, d);
+                                if (lane >= d) s += y;
+                            }
+                            const uint32_t hi = __shfl_sync(0xffffffffu, s, glast);
+                            const uint32_t lo = __shfl_sync(0xffffffffu, s, gl ? gl - 1u : 0u);
+                            const bool alive = has && hi - (gl ? lo : 0u) >= min_bits;
+                            const uint32_t vote = __ballot_sync(0xffffffffu, alive && w0 == 0u);
+                            if (MODE == kSegWriteLive && alive)
+                                __stcs(out + (pos + running + __popc(vote & below)) * U + w0, v);
+                            running += __popc(vote);
+                        }
+                    } else {
+                        for (uint32_t j = 0; j < m.t2; ++j) {
+                            const VT *brow = b + (uint64_t)j * U;
+                            uint32_t s = 0;
+                            for (uint32_t w = w0; w < U; w += 32u) s += vpopc(vand(__ldg(arow + w), __ldg(brow + w)));
+                            if (__reduce_add_sync(0xffffffffu, s) >= min_bits) {   // the same verdict on every lane
+                                if (MODE == kSegWriteLive) {                     // read again (L1 / L2), then store
+                                    VT *o = out + (pos + running) * U;
+#pragma unroll 4
+                                    for (uint32_t w = w0; w < U; w += 32u)
+                                        __stcs(o + w, vand(__ldg(arow + w), __ldg(brow + w)));
+                                }
+                                ++running;
+                            }
+                        }
+                    }
+                }
+                if (MODE == kSegCount && lane == 0u) live[it] = running;
+            }
+        }
+        return;
+    }
     if (j0 >= G) return;                                       // lanes beyond the last whole block of a step
     for (uint32_t t = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); t < n_tasks; t += warps) {
         const uint32_t it_end = __ldg(tasks + t + 1);
@@ -135,10 +205,29 @@ cudaError_t launch_seg_mul(uint64_t *out, uint32_t L, bool units16, const SegMul
     if (n_tasks == 0) return cudaSuccess;
     count_launch();
     if (units16)
-        return launch_kernel(seg_mul_kernel<uint4>, seg_grid(n_tasks), kSegThreads, 0, stream,
-                             reinterpret_cast<uint4 *>(out), L / 2, items, tasks, n_tasks);
-    return launch_kernel(seg_mul_kernel<uint2>, seg_grid(n_tasks), kSegThreads, 0, stream,
-                         reinterpret_cast<uint2 *>(out), L, items, tasks, n_tasks);
+        return launch_kernel(seg_mul_kernel<uint4, kSegPlain>, seg_grid(n_tasks), kSegThreads, 0, stream,
+                             reinterpret_cast<uint4 *>(out), L / 2, items, tasks, n_tasks, 0u, (uint32_t *)nullptr,
+                             (const uint64_t *)nullptr);
+    return launch_kernel(seg_mul_kernel<uint2, kSegPlain>, seg_grid(n_tasks), kSegThreads, 0, stream,
+                         reinterpret_cast<uint2 *>(out), L, items, tasks, n_tasks, 0u, (uint32_t *)nullptr,
+                         (const uint64_t *)nullptr);
+}
+
+cudaError_t launch_seg_mul_live(uint64_t *out, uint32_t L, bool units16, const SegMulItem *items,
+                                const uint32_t *tasks, uint32_t n_tasks, uint32_t min_bits, uint32_t *live,
+                                const uint64_t *base, cudaStream_t stream) {
+    if (n_tasks == 0) return cudaSuccess;
+    count_launch();
+    const uint32_t grid = seg_grid(n_tasks);
+    if (units16)
+        return live ? launch_kernel(seg_mul_kernel<uint4, kSegCount>, grid, kSegThreads, 0, stream,
+                                    reinterpret_cast<uint4 *>(out), L / 2, items, tasks, n_tasks, min_bits, live, base)
+                    : launch_kernel(seg_mul_kernel<uint4, kSegWriteLive>, grid, kSegThreads, 0, stream,
+                                    reinterpret_cast<uint4 *>(out), L / 2, items, tasks, n_tasks, min_bits, live, base);
+    return live ? launch_kernel(seg_mul_kernel<uint2, kSegCount>, grid, kSegThreads, 0, stream,
+                                reinterpret_cast<uint2 *>(out), L, items, tasks, n_tasks, min_bits, live, base)
+                : launch_kernel(seg_mul_kernel<uint2, kSegWriteLive>, grid, kSegThreads, 0, stream,
+                                reinterpret_cast<uint2 *>(out), L, items, tasks, n_tasks, min_bits, live, base);
 }
 
 cudaError_t launch_seg_decrypt(const uint64_t *v, uint32_t L, const uint64_t *mask, const uint64_t *off,

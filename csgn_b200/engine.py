@@ -280,6 +280,11 @@ class Ciphertext:
         check(_lib().csgn_permute(self._h, perm._h, 1 if strict_ref_truncate else 0, ctypes.byref(h)))
         return Ciphertext(h, self.ctx)
 
+    def compact(self):
+        """A new ciphertext without the blocks that have fewer than D set bits (see CiphertextArray.compact): the same
+        satisfied-block count under every key of the context."""
+        return CiphertextArray(self, [0, self.n_blocks]).compact().storage
+
     def permute_into(self, perm, out):
         check(_lib().csgn_permute_into(self._h, perm._h, out._h))
         return out
@@ -441,9 +446,11 @@ class CiphertextArray:
         return self._binary(_lib().csgn_seg_concat, other)
 
     @staticmethod
-    def sum_of_products(products, terms=()):
+    def sum_of_products(products, terms=(), compact=False):
         """csgn_seg_mul_sum: element k = A0_k*B0_k + A1_k*B1_k + ... + C0_k + ... for `products` [(A0, B0), ...] and
-        `terms` [C0, ...], every output word written once (one gate of a circuit in one call)."""
+        `terms` [C0, ...], every output word written once (one gate of a circuit in one call).  compact=True
+        (csgn_seg_mul_sum_compact with min_bits = D): only the blocks with at least D set bits, which are the only
+        blocks any key of the context can satisfy, so every decryption is unchanged."""
         products = [(x, y) for x, y in products]
         terms = list(terms)
         arrays = [x for pr in products for x in pr] + terms
@@ -460,9 +467,17 @@ class CiphertextArray:
         left, right = [x for x, _ in products], [y for _, y in products]
         out_off = np.empty(n + 1, dtype=np.uint64)
         out = _vp()
-        check(_lib().csgn_seg_mul_sum(h(left), o(left), h(right), o(right), len(products), h(terms), o(terms), len(terms),
-                                      n, out_off.ctypes.data_as(_vp), ctypes.byref(out)))
+        args = (h(left), o(left), h(right), o(right), len(products), h(terms), o(terms), len(terms), n)
+        if compact:
+            check(_lib().csgn_seg_mul_sum_compact(*args, ctx.D, out_off.ctypes.data_as(_vp), ctypes.byref(out)))
+        else:
+            check(_lib().csgn_seg_mul_sum(*args, out_off.ctypes.data_as(_vp), ctypes.byref(out)))
         return CiphertextArray(Ciphertext(out, ctx), out_off)
+
+    def compact(self):
+        """The array without the blocks that have fewer than D set bits (no key of the context satisfies them): every
+        element keeps its other blocks in order and decrypts as before under every key."""
+        return CiphertextArray.sum_of_products([], [self], compact=True)
 
     def gather(self, idx):
         """csgn_seg_gather: element j = self_{idx[j]} (any order, repeats allowed)."""

@@ -262,6 +262,16 @@ int csgn_seg_concat(const csgn_buf *a, const uint64_t *a_off, const csgn_buf *b,
 int csgn_seg_mul_sum(const csgn_buf *const *a, const uint64_t *const *a_off, const csgn_buf *const *b,
                      const uint64_t *const *b_off, uint32_t n_products, const csgn_buf *const *c,
                      const uint64_t *const *c_off, uint32_t n_terms, uint64_t n, uint64_t *out_off, csgn_buf **out);
+/* csgn_seg_mul_sum with only the blocks that have at least min_bits set bits (min_bits = D of the context: no key can
+ * satisfy the others, so every element's satisfied-block count is unchanged under every key).  Element k is the stable
+ * subsequence of element k of csgn_seg_mul_sum's result.  n_products = 0 with one term compacts an existing array.
+ * The sizes depend on the data: the call returns after the counting pass, like csgn_seg_decrypt.  The checks are
+ * those of csgn_seg_mul_sum, plus 1 <= min_bits <= 64*L.  A block's pad bits count (the library leaves them zero);
+ * an element with no surviving block is empty. */
+int csgn_seg_mul_sum_compact(const csgn_buf *const *a, const uint64_t *const *a_off, const csgn_buf *const *b,
+                             const uint64_t *const *b_off, uint32_t n_products, const csgn_buf *const *c,
+                             const uint64_t *const *c_off, uint32_t n_terms, uint64_t n, uint32_t min_bits,
+                             uint64_t *out_off, csgn_buf **out);
 /* element j = src_{idx[j]}, j < m: any order, repeats allowed; idx[j] < n_src is checked. */
 int csgn_seg_gather(const csgn_buf *src, const uint64_t *src_off, uint64_t n_src, const uint64_t *idx, uint64_t m,
                     uint64_t *out_off, csgn_buf **out);

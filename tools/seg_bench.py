@@ -11,6 +11,10 @@
           ~2.7 GB at the last step) as three calls (csgn_seg_mul twice, csgn_seg_concat) and as one csgn_seg_mul_sum:
           time and launches per step, output bytes per second as a fraction of a device-to-device copy of the same
           bytes; then the whole 12-bit adder (circuit and decrypt) both ways
+  compact the carry gate with compaction (csgn_seg_mul_sum_compact, min_bits = D: only blocks that some key could
+          satisfy are kept): the 12-bit adder over 4096 lanes with plain and with compacting carry gates, the 32-bit adder
+          compacted (uncompacted its last carry would hold 2^32 - 1 blocks per lane), and compact() on its own over the
+          uncompacted 12-bit carry -- time, bytes written by the carry gates, and blocks held per lane after every gate
   sweep   elements whose product is 64 KB .. 64 MB, ~1 GB per call: the grouped kernel against one launch_mul per
           element (CSGN_SEG_LARGE_BYTES), which sets the large-element threshold of capi_seg.cu
 
@@ -300,6 +304,72 @@ def gates(ctx, key, rng, lanes, bits):
             min(whole["one call"]) * 1e3, whole["one call launches"], min(whole["three calls"]) / min(whole["one call"])))
 
 
+def compact_adder(ctx, key, rng, lanes, bits, compact):
+    """-> (run, check): run() computes the carries of a `bits`-bit adder over `lanes` lanes (carry gates compacting or
+    not) and returns (sum arrays, last carry, blocks per lane after every carry gate, bytes the carry gates wrote)"""
+    SP = eng.CiphertextArray.sum_of_products
+    xb, yb = rng.integers(0, 1 << bits, lanes), rng.integers(0, 1 << bits, lanes)
+    plain = np.concatenate([np.concatenate([(v >> i) & 1 for i in range(bits)]) for v in (xb, yb)]).astype(np.uint8)
+    allb = key.encrypt_array(plain, seed=11)
+    rows = [allb.gather(np.arange(r * lanes, (r + 1) * lanes)) for r in range(2 * bits)]
+    T = [rows[i] + rows[bits + i] for i in range(bits)]
+    word_bytes = ctx.L * 8
+
+    def run():
+        C = SP([(rows[0], rows[bits])], compact=compact)
+        S, held, written = [T[0]], [C.storage.n_blocks / lanes], C.storage.n_blocks * word_bytes
+        for i in range(1, bits):
+            S.append(T[i] + C)
+            C = SP([(rows[i], rows[bits + i]), (T[i], C)], compact=compact)
+            held.append(C.storage.n_blocks / lanes)
+            written += C.storage.n_blocks * word_bytes
+        return S, C, held, written
+
+    def check(S, C):
+        got = [key.decrypt_array(x)[0] for x in S] + [key.decrypt_array(C)[0]]
+        val = sum(got[i].astype(np.int64) << i for i in range(bits))
+        assert np.array_equal(val, (xb + yb) % (1 << bits)) and np.array_equal(got[bits], (xb + yb) >> bits), \
+            "%d-bit adder wrong" % bits
+    return run, check
+
+
+def compaction(ctx, key, rng, lanes):
+    keep = []
+    for bits, modes in ((12, (False, True)), (32, (True,))):
+        for compact in modes:
+            run, check = compact_adder(ctx, key, np.random.default_rng(bits), lanes, bits, compact)
+            S, C, held, written = run()
+            check(S, C)
+            del S, C
+            torch.cuda.empty_cache()
+
+            def carries():
+                keep[:] = [run()]
+            t, reps = timed(carries, min_s=2.0, min_reps=2)
+            keep.clear()
+            torch.cuda.empty_cache()
+            log("compact: %d-bit adder carries, %d lanes, Context(%d,%d), %s: %8.2f ms (%d runs)  %.3f GB written by "
+                "the carry gates" % (bits, lanes, ctx.N, ctx.D, "compacting gates" if compact else "plain gates   ",
+                                     t * 1e3, reps, written / 1e9))
+            log("compact: %d-bit %s blocks per lane after each carry gate: %s" % (
+                bits, "compacted" if compact else "plain    ", " ".join("%.1f" % h for h in held)))
+    # compact() on its own over the uncompacted 12-bit carry
+    run, _ = compact_adder(ctx, key, np.random.default_rng(12), lanes, 12, False)
+    _, C, _, _ = run()
+    small = C.compact()
+
+    def compact_once():
+        keep[:] = [C.compact()]
+    t, reps = timed(compact_once)
+    keep.clear()
+    log("compact: compact() of the uncompacted 12-bit carry (%.2f GB, %.1f blocks per lane) -> %.1f blocks per lane: "
+        "%8.3f ms (%d calls)  %.3f GB written  %.0f GB/s read" % (
+            C.storage.n_blocks * ctx.L * 8 / 1e9, C.storage.n_blocks / lanes, small.storage.n_blocks / lanes, t * 1e3,
+            reps, small.storage.n_blocks * ctx.L * 8 / 1e9, C.storage.n_blocks * ctx.L * 8 / t / 1e9))
+    del C, small
+    torch.cuda.empty_cache()
+
+
 def sweep(ctx, total_bytes, sizes_kb):
     L = ctx.L
     for kb in sizes_kb:
@@ -333,7 +403,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default="")
     ap.add_argument("--quick", action="store_true", help="small sizes (a check of the script, not a measurement)")
-    ap.add_argument("--only", default="small,mixed,adder,gates,sweep")
+    ap.add_argument("--only", default="small,mixed,adder,gates,compact,sweep")
     args = ap.parse_args()
     torch.cuda.set_device(0)
     eng.init(0)
@@ -359,6 +429,11 @@ def main():
             gates(ctx, key, rng, 256 if args.quick else 4096, 8 if args.quick else 12)
         else:
             log("gates: skipped, %s has no csgn_seg_mul_sum" % os.environ.get("CSGN_LIBRARY", "this build"))
+    if "compact" in only:
+        if hasattr(eng._lib(), "csgn_seg_mul_sum_compact"):
+            compaction(ctx, key, rng, 256 if args.quick else 4096)
+        else:
+            log("compact: skipped, %s has no csgn_seg_mul_sum_compact" % os.environ.get("CSGN_LIBRARY", "this build"))
     if "sweep" in only:
         sweep(ctx, (64 << 20) if args.quick else (1 << 30),
               [64, 256] if args.quick else [64, 256, 1024, 4096, 16384, 65536])

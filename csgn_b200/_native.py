@@ -84,6 +84,7 @@ SIGNATURES = {
     "csgn_seg_mul_sum_compact": (ctypes.c_int, [ctypes.POINTER(_vp), ctypes.POINTER(_vp), ctypes.POINTER(_vp),
                                                 ctypes.POINTER(_vp), ctypes.c_uint32, ctypes.POINTER(_vp),
                                                 ctypes.POINTER(_vp), ctypes.c_uint32, _u64, ctypes.c_uint32, _vp, _vpp]),
+    "csgn_seg_cancel": (ctypes.c_int, [_vp, _vp, _u64, _vp, _vpp]),
     "csgn_seg_gather": (ctypes.c_int, [_vp, _vp, _u64, _vp, _u64, _vp, _vpp]),
     "csgn_concat_n": (ctypes.c_int, [ctypes.POINTER(_vp), _u64, _vpp]),
     "csgn_seg_decrypt_count_async": (ctypes.c_int, [_vp, _vp, _u64, _vp, _vp]),

@@ -4,6 +4,7 @@
 //   operator* / operator+     -> csgn_seg_mul / csgn_seg_concat
 //   sumOfProducts             -> csgn_seg_mul_sum
 //   compactSumOfProducts, compact, Ciphertext::compact -> csgn_seg_mul_sum_compact (min_bits = D)
+//   cancel, Ciphertext::cancel -> csgn_seg_cancel
 //   gather                    -> csgn_seg_gather
 //   applyPermutation          -> csgn_permute on the storage (a permutation acts on every block by itself)
 //   encryptArray / decryptArray -> csgn_encrypt_batch / csgn_seg_decrypt
@@ -144,6 +145,13 @@ CiphertextArray CiphertextArray::compactSumOfProducts(
 
 CiphertextArray CiphertextArray::compact() const { return gate({}, {*this}, true); }
 
+CiphertextArray CiphertextArray::cancel() const {
+    std::vector<uint64_t> off(size() + 1);
+    csgn_buf *out = nullptr;
+    glue::check(csgn_seg_cancel(storage.get(), offsets.data(), size(), off.data(), &out), "csgn_seg_cancel");
+    return CiphertextArray(out, off, context);
+}
+
 
 CiphertextArray CiphertextArray::gather(const std::vector<uint64_t> &idx) const {
     std::vector<uint64_t> off(idx.size() + 1);
@@ -174,6 +182,21 @@ Ciphertext Ciphertext::compact() const {
     glue::check(csgn_seg_mul_sum_compact(nullptr, nullptr, nullptr, nullptr, 0, one, offs, 1, 1,
                                          (uint32_t)certFHEcontext->getD(), out_off, &res),
                 "csgn_seg_mul_sum_compact");
+    Ciphertext out;
+    out.certFHEcontext = new Context(*certFHEcontext);
+    out.dev = adopt(res);
+    out.sharded = sharded;
+    return out;
+}
+
+Ciphertext Ciphertext::cancel() const {
+    const csgn_buf *b = deviceBuffer();   // writes a pending product; the call makes a lazy sum dense
+    if (!b) return *this;
+    if (!certFHEcontext) throw Error("Ciphertext::cancel: no context");
+    const uint64_t off[2] = {0, csgn_buf_blocks(b)};
+    uint64_t out_off[2];
+    csgn_buf *res = nullptr;
+    glue::check(csgn_seg_cancel(b, off, 1, out_off, &res), "csgn_seg_cancel");
     Ciphertext out;
     out.certFHEcontext = new Context(*certFHEcontext);
     out.dev = adopt(res);

@@ -254,6 +254,11 @@ public:
     // the others, so the satisfied-block count is the same under every key.  A pending product or lazy sum is made
     // dense first; an empty ciphertext stays empty.
     Ciphertext compact() const;
+    // The first occurrence, in order, of every block value that occurs an odd number of times (csgn_seg_cancel): equal
+    // blocks are satisfied by the same keys, so the decryption is unchanged under every key, while the satisfied-block
+    // count changes by an even number (unlike compact()).  x*x cancels to x.  A pending product or lazy sum is made
+    // dense first; an empty ciphertext stays empty.
+    Ciphertext cancel() const;
     // A sharded ciphertext as one file per rank, `<prefix>.shard<rank>of<world>` (csgn_buf_save_shard): every rank
     // writes / reads its own blocks, no collective.  loadSharded returns a ciphertext marked sharded.
     void saveSharded(const std::string &prefix) const;
@@ -354,6 +359,10 @@ public:
         const std::vector<std::pair<CiphertextArray, CiphertextArray>> &products,
         const std::vector<CiphertextArray> &terms = {});
     CiphertextArray compact() const;
+    // Every element reduced to the first occurrence, in order, of each block value that occurs an odd number of times
+    // in it (csgn_seg_cancel): x*x -> x, a + a -> empty.  Every element decrypts as before under every key; its
+    // satisfied-block count changes by an even number.  The usual gate is compactSumOfProducts(...).cancel().
+    CiphertextArray cancel() const;
 
     const std::vector<uint64_t> &getOffsets() const;
     const csgn_buf *deviceBuffer() const;

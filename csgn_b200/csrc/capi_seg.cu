@@ -436,6 +436,105 @@ int csgn_seg_mul_sum_compact(const csgn_buf *const *a, const uint64_t *const *a_
     return mul_sum(a, a_off, b, b_off, n_products, c, c_off, n_terms, n, true, min_bits, out_off, out);
 }
 
+// Every element is cut into tasks of about one task's words (segments.cu, SegCancelTask); element k gets a hash region
+// of the power of two >= 2 T_k slots.  One staged allocation holds the task table, the tasks' output bases, then the
+// scratch of the three passes: slots and parity bits (zeroed by one memset), first (0x7f bytes), rep, and the tasks'
+// survivor counts.
+int csgn_seg_cancel(const csgn_buf *c, const uint64_t *c_off, uint64_t n, uint64_t *out_off, csgn_buf **out) {
+    NEED_INIT();
+    if (!c || !out || !out_off) return fail(CSGN_ERR_INVALID_ARGUMENT, "null argument");
+    int rc = check_offsets(c, c_off, n, "ciphertext array");
+    if (rc != CSGN_OK) return rc;
+    const uint32_t L = c->L;
+    const uint64_t T = c->n_blocks;
+    const uint64_t target = std::max<uint64_t>(1, task_words(T * L) / L);
+    std::vector<SegCancelTask> tasks;
+    std::vector<uint64_t> owner;   // element of every task
+    uint64_t slots = 0;
+    for (uint64_t k = 0; k < n; ++k) {
+        const uint64_t t = c_off[k + 1] - c_off[k];
+        if (t > kCancelMaxBlocks)
+            return fail(CSGN_ERR_INVALID_ARGUMENT, "element %llu holds %llu blocks, more than the 2^30 of one element",
+                        (unsigned long long)k, (unsigned long long)t);
+        if (t == 0) continue;
+        uint64_t cap = 2;
+        while (cap < 2 * t) cap <<= 1;
+        for (uint64_t i = 0; i < t; i += target) {
+            tasks.push_back({c_off[k], slots, (uint32_t)i, (uint32_t)std::min(t, i + target), (uint32_t)(cap - 1), 0});
+            owner.push_back(k);
+        }
+        slots += cap;
+    }
+    const uint64_t nt = tasks.size();
+    if (nt >= UINT32_MAX) return fail(CSGN_ERR_INVALID_ARGUMENT, "too many work items");
+    AutoLane lane(c);
+    rc = need_dense(c);
+    if (rc != CSGN_OK) return rc;
+    acquire_read(c);
+    std::vector<uint64_t> off(n + 1, 0);
+    csgn_buf *res = nullptr;
+    if (nt == 0) {   // no blocks
+        rc = new_buf(0, L, 0, &res);
+        if (rc != CSGN_OK) return rc;
+        memcpy(out_off, off.data(), (n + 1) * sizeof(uint64_t));
+        *out = res;
+        return CSGN_OK;
+    }
+    // words: tasks, bases, then slots + parity (uint32 each, zeroed together), first, rep, live
+    const uint64_t w_tab = nt * sizeof(SegCancelTask) / 8, w_zero = slots / 2 + (T + 63) / 64, w_t = (T + 1) / 2;
+    uint64_t *d = nullptr;
+    rc = dev_alloc(w_tab + nt + w_zero + 2 * w_t + (nt + 1) / 2, &d);
+    if (rc != CSGN_OK) return rc;
+    DevTable scratch;
+    scratch.d = d;
+    const SegCancelTask *d_tasks = reinterpret_cast<const SegCancelTask *>(d);
+    uint64_t *d_base = d + w_tab, *zero = d_base + nt;
+    SegCancelScratch s;
+    s.slots = reinterpret_cast<uint32_t *>(zero);
+    s.parity = s.slots + slots;
+    s.first = reinterpret_cast<int32_t *>(zero + w_zero);
+    s.rep = reinterpret_cast<int32_t *>(zero + w_zero + w_t);
+    uint32_t *d_live = reinterpret_cast<uint32_t *>(zero + w_zero + 2 * w_t);
+    rc = stage_into(d, tasks.data(), nt * sizeof(SegCancelTask));
+    if (rc != CSGN_OK) return rc;
+    CU(cudaMemsetAsync(zero, 0, w_zero * sizeof(uint64_t), g.stream));
+    CU(cudaMemsetAsync(s.first, 0x7f, T * sizeof(int32_t), g.stream));
+    const bool units16 = !(L & 1u) && (reinterpret_cast<uintptr_t>(c->d) & 15u) == 0;
+    cudaError_t e = launch_seg_cancel_insert(c->d, L, units16, d_tasks, (uint32_t)nt, s, g.stream);
+    if (e == cudaSuccess) e = launch_seg_cancel_count(d_tasks, (uint32_t)nt, s, d_live, g.stream);
+    if (e != cudaSuccess) return cuda_fail(e, "cancellation kernel");
+    std::vector<uint32_t> live(nt);
+    rc = read_back(live.data(), d_live, nt * sizeof(uint32_t));
+    if (rc != CSGN_OK) return rc;
+    // every task's base is the total of the tasks before it, which keeps the survivors of every element in order
+    std::vector<uint64_t> base(nt);
+    uint64_t total = 0;
+    for (uint64_t t = 0; t < nt; ++t) {
+        base[t] = total;
+        total += live[t];
+        off[owner[t] + 1] += live[t];
+    }
+    for (uint64_t k = 0; k < n; ++k) off[k + 1] += off[k];
+    rc = new_buf(total, L, 0, &res);
+    if (rc != CSGN_OK) return rc;
+    acquire_write(res);
+    if (total) {
+        rc = stage_into(d_base, base.data(), nt * sizeof(uint64_t));
+        if (rc == CSGN_OK) {
+            const bool out16 = units16 && (reinterpret_cast<uintptr_t>(res->d) & 15u) == 0;
+            e = launch_seg_cancel_write(c->d, L, out16, d_tasks, (uint32_t)nt, s, d_base, res->d, g.stream);
+            if (e != cudaSuccess) rc = cuda_fail(e, "cancellation kernel (write)");
+        }
+        if (rc != CSGN_OK) {
+            csgn_buf_free(res);
+            return rc;
+        }
+    }
+    memcpy(out_off, off.data(), (n + 1) * sizeof(uint64_t));
+    *out = res;
+    return CSGN_OK;
+}
+
 int csgn_seg_concat(const csgn_buf *a, const uint64_t *a_off, const csgn_buf *b, const uint64_t *b_off, uint64_t n,
                     uint64_t *out_off, csgn_buf **out) {
     NEED_INIT();

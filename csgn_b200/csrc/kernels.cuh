@@ -83,6 +83,34 @@ struct SegDecTask {
 };
 cudaError_t launch_seg_decrypt(const uint64_t *v, uint32_t L, const uint64_t *mask, const uint64_t *off,
                                const SegDecTask *tasks, uint32_t n_tasks, uint64_t *counts, cudaStream_t stream);
+// Cancellation (csgn_seg_cancel): a warp task is the blocks [first, end) of one element, whose first block is block
+// `elem` of the array and whose open-addressing region is slots [slot, slot + slot_mask + 1) (a power of two).  Three
+// passes over the same tasks, one launch each:
+//   insert  every block finds its value's representative r (a slot holds an element-relative block index + 1, taken by
+//           atomicCAS; equality is decided on all L words) and stores rep[b] = b - r; first[r] = min of b - r over the
+//           value's blocks (atomicMin; the caller sets first to 0x7f7f7f7f), parity bit r ^= 1 (atomicXor; zeroed by the
+//           caller, as are the slots);
+//   count   live[t] = blocks b of task t with first[r] == b - r and parity bit r set (one plain store per task);
+//   write   those blocks of task t, in order, to blocks base[t], base[t] + 1, ... of `out`.
+// Blocks are numbered in the whole array; an element holds at most kCancelMaxBlocks blocks, so b - r fits an int32.
+struct SegCancelTask {
+    uint64_t elem, slot;
+    uint32_t first, end, slot_mask, pad;
+};
+static_assert(sizeof(SegCancelTask) == 32, "SegCancelTask is read as one 32-byte record");
+struct SegCancelScratch {
+    uint32_t *slots;
+    int32_t *first, *rep;
+    uint32_t *parity;
+};
+constexpr uint64_t kCancelMaxBlocks = 1ull << 30;
+cudaError_t launch_seg_cancel_insert(const uint64_t *v, uint32_t L, bool units16, const SegCancelTask *tasks,
+                                     uint32_t n_tasks, const SegCancelScratch &s, cudaStream_t stream);
+cudaError_t launch_seg_cancel_count(const SegCancelTask *tasks, uint32_t n_tasks, const SegCancelScratch &s,
+                                    uint32_t *live, cudaStream_t stream);
+cudaError_t launch_seg_cancel_write(const uint64_t *v, uint32_t L, bool units16, const SegCancelTask *tasks,
+                                    uint32_t n_tasks, const SegCancelScratch &s, const uint64_t *base, uint64_t *out,
+                                    cudaStream_t stream);
 
 // out[0] = sum of in[0..n): the partial counts of a ciphertext held as several segments (a lazy sum)
 cudaError_t launch_sum_words(const uint64_t *in, uint32_t n, uint64_t *out, cudaStream_t stream);

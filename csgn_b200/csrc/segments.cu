@@ -6,6 +6,8 @@
 //                      or a sum of products and plain terms a0_k*b0_k || ... || c0_k || ... (operands in any buffers;
 //                      a term is a product with one all-ones block)
 //   segmented decrypt  counts[k] = satisfied blocks of element k           (reference src/SecretKey.cpp:126-140)
+//   cancellation       element k = the first occurrence, in order, of every block value that occurs an odd number of
+//                      times in element k (insert into a hash table per element, count, write)
 //
 // (the element-wise concat / gather / pack copy is misc.cu's streaming copy over a piece table.)
 //
@@ -192,6 +194,176 @@ seg_decrypt_kernel(const VT *__restrict__ v, const uint32_t U, const uint32_t lo
     }
 }
 
+// ---------------------------------------------------------------------------------------
+// cancellation: groups of G lanes (G the power of two >= U, up to 32) take one block each per warp step, as in the
+// segmented decrypt.  A block's hash is the splitmix64 finaliser of the sum of its words' finalised values (each word
+// offset by its position), so the lanes of a group add their parts in any order; the hash only chooses the first slot
+// to probe.  Linear probing from there: an empty slot is taken by atomicCAS; a taken slot's occupant is compared word
+// for word, and an equal occupant is the representative.  Equal blocks walk the same slots, and a slot is taken once,
+// so every value of an element has exactly one representative whatever the order of the warps.  With G < 32 the group
+// leader probes alone and compares serially (groups probe different numbers of slots, so no warp vote runs there);
+// with G = 32 (WARP_BLOCK) the warp holds one block, every lane takes every probe, and lane 0's atomicCAS is broadcast.
+// The insert pass asks for 4 resident CTAs per SM: left to its own register target, ptxas spills in the probe loops.
+// ---------------------------------------------------------------------------------------
+__device__ __forceinline__ uint64_t mix64(uint64_t x) {
+    x ^= x >> 30;
+    x *= 0xbf58476d1ce4e5b9ull;
+    x ^= x >> 27;
+    x *= 0x94d049bb133111ebull;
+    return x ^ (x >> 31);
+}
+__device__ __forceinline__ uint64_t word_hash(uint64_t x, uint64_t w) { return mix64(x + (w + 1) * 0x9e3779b97f4a7c15ull); }
+__device__ __forceinline__ uint64_t unit_hash(const uint2 u, uint32_t w) {
+    return word_hash((uint64_t)u.y << 32 | u.x, w);
+}
+__device__ __forceinline__ uint64_t unit_hash(const uint4 u, uint32_t w) {
+    return word_hash((uint64_t)u.y << 32 | u.x, 2ull * w) + word_hash((uint64_t)u.w << 32 | u.z, 2ull * w + 1);
+}
+__device__ __forceinline__ bool veq(const uint2 x, const uint2 y) { return x.x == y.x && x.y == y.y; }
+__device__ __forceinline__ bool veq(const uint4 x, const uint4 y) {
+    return x.x == y.x && x.y == y.y && x.z == y.z && x.w == y.w;
+}
+
+// Block b (of the whole array) survives when it is the first of its value's blocks and the value occurs an odd number
+// of times in its element.
+__device__ __forceinline__ bool cancel_survives(const uint64_t b, const SegCancelScratch &s) {
+    const int32_t d = __ldg(s.rep + b);
+    const uint64_t r = b - (uint64_t)(int64_t)d;
+    return __ldg(s.first + r) == d && ((__ldg(s.parity + (r >> 5)) >> (r & 31u)) & 1u);
+}
+
+template <typename VT, bool WARP_BLOCK>
+__global__ void __launch_bounds__(kSegThreads, 4)
+seg_cancel_insert_kernel(const VT *__restrict__ v, const uint32_t U, const uint32_t log2g,
+                         const SegCancelTask *__restrict__ tasks, const uint32_t n_tasks, const SegCancelScratch s) {
+    const uint32_t lane = threadIdx.x & 31u;
+    const uint32_t G = 1u << log2g, sub = lane & (G - 1u), grp = lane >> log2g, B = 32u >> log2g;
+    const uint32_t warps = gridDim.x * (blockDim.x >> 5);
+    pdl_enter();
+    for (uint32_t t = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); t < n_tasks; t += warps) {
+        const SegCancelTask task = tasks[t];
+        const VT *ev = v + task.elem * U;                      // the element's first block
+        uint32_t *slots = s.slots + task.slot;
+        for (uint32_t i0 = task.first; i0 < task.end; i0 += B) {
+            const uint32_t i = i0 + grp;                       // element-relative block of this lane's group
+            const bool live = i < task.end;
+            const VT *p = ev + (uint64_t)i * U;
+            uint64_t h = 0;
+            if (live)
+                for (uint32_t w = sub; w < U; w += G) h += unit_hash(__ldg(p + w), w);
+            // the group's sum on each of its lanes; every lane takes every step with the full mask
+#pragma unroll
+            for (uint32_t d = 1; d < 32u; d <<= 1) {
+                const uint64_t y = __shfl_xor_sync(0xffffffffu, h, d);
+                if (d < G) h += y;
+            }
+            h = mix64(h);
+            uint32_t slot = (uint32_t)h & task.slot_mask, r = 0;
+            bool records;                                      // the lane that records the block's representative
+            if (!WARP_BLOCK) {
+                records = live && sub == 0u;
+                while (records) {
+                    const uint32_t occ = atomicCAS(slots + slot, 0u, i + 1u);
+                    if (occ == 0u) {
+                        r = i;
+                        break;
+                    }
+                    const VT *q = ev + (uint64_t)(occ - 1u) * U;
+                    bool eq = true;
+                    for (uint32_t w = 0; w < U && eq; ++w) eq = veq(__ldg(p + w), __ldg(q + w));
+                    if (eq) {
+                        r = occ - 1u;
+                        break;
+                    }
+                    slot = (slot + 1u) & task.slot_mask;
+                }
+            } else {                                           // one block per warp step: the whole warp probes
+                for (;;) {
+                    uint32_t occ = 0;
+                    if (lane == 0u) occ = atomicCAS(slots + slot, 0u, i + 1u);
+                    occ = __shfl_sync(0xffffffffu, occ, 0);
+                    if (occ == 0u) {
+                        r = i;
+                        break;
+                    }
+                    const VT *q = ev + (uint64_t)(occ - 1u) * U;
+                    bool eq = true;
+                    for (uint32_t w = lane; w < U; w += 32u) eq &= veq(__ldg(p + w), __ldg(q + w));
+                    if (__all_sync(0xffffffffu, eq)) {
+                        r = occ - 1u;
+                        break;
+                    }
+                    slot = (slot + 1u) & task.slot_mask;
+                }
+                records = lane == 0u;
+            }
+            if (records) {
+                const uint64_t b = task.elem + i, rb = task.elem + r;
+                const int32_t d = (int32_t)i - (int32_t)r;
+                s.rep[b] = d;
+                atomicMin(s.first + rb, d);
+                atomicXor(s.parity + (rb >> 5), 1u << (rb & 31u));
+            }
+        }
+    }
+}
+
+// One block per lane; the survivors of a task are counted with one ballot per warp step and stored once.
+__global__ void __launch_bounds__(kSegThreads)
+seg_cancel_count_kernel(const SegCancelTask *__restrict__ tasks, const uint32_t n_tasks, const SegCancelScratch s,
+                        uint32_t *__restrict__ live) {
+    const uint32_t lane = threadIdx.x & 31u;
+    const uint32_t warps = gridDim.x * (blockDim.x >> 5);
+    pdl_enter();
+    for (uint32_t t = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); t < n_tasks; t += warps) {
+        const SegCancelTask task = tasks[t];
+        uint32_t running = 0;
+        for (uint32_t i0 = task.first; i0 < task.end; i0 += 32u) {
+            const uint32_t i = i0 + lane;
+            const bool keep = i < task.end && cancel_survives(task.elem + i, s);
+            running += __popc(__ballot_sync(0xffffffffu, keep));
+        }
+        if (lane == 0u) live[t] = running;
+    }
+}
+
+// Groups of G lanes as in the insert pass; a surviving block's rank is the number of surviving group leaders below
+// its own in the step's ballot, after the task's running count.
+template <typename VT>
+__global__ void __launch_bounds__(kSegThreads)
+seg_cancel_write_kernel(const VT *__restrict__ v, VT *__restrict__ out, const uint32_t U, const uint32_t log2g,
+                        const SegCancelTask *__restrict__ tasks, const uint32_t n_tasks, const SegCancelScratch s,
+                        const uint64_t *__restrict__ base) {
+    const uint32_t lane = threadIdx.x & 31u;
+    const uint32_t G = 1u << log2g, sub = lane & (G - 1u), grp = lane >> log2g, B = 32u >> log2g;
+    const uint32_t below = (1u << (grp * G)) - 1u;             // lanes of the groups before this one
+    const uint32_t warps = gridDim.x * (blockDim.x >> 5);
+    pdl_enter();
+    for (uint32_t t = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); t < n_tasks; t += warps) {
+        const SegCancelTask task = tasks[t];
+        const uint64_t pos = __ldg(base + t);
+        uint32_t running = 0;
+        for (uint32_t i0 = task.first; i0 < task.end; i0 += B) {
+            const uint32_t i = i0 + grp;
+            const bool keep = i < task.end && cancel_survives(task.elem + i, s);
+            const uint32_t vote = __ballot_sync(0xffffffffu, keep && sub == 0u);
+            if (keep) {
+                const VT *p = v + (task.elem + i) * U;
+                VT *o = out + (pos + running + __popc(vote & below)) * U;
+                for (uint32_t w = sub; w < U; w += G) __stcs(o + w, __ldg(p + w));
+            }
+            running += __popc(vote);
+        }
+    }
+}
+
+// log2 of the group width G of the decrypt and cancellation kernels: the power of two >= U, up to 32
+uint32_t group_log2(uint32_t U) {
+    uint32_t log2g = 0;
+    while (log2g < 5 && (1u << log2g) < U) ++log2g;
+    return log2g;
+}
+
 uint32_t seg_grid(uint32_t n_tasks) {
     const uint32_t warps_per_cta = kSegThreads / 32;
     const uint64_t want = ((uint64_t)n_tasks + warps_per_cta - 1) / warps_per_cta;
@@ -235,8 +407,7 @@ cudaError_t launch_seg_decrypt(const uint64_t *v, uint32_t L, const uint64_t *ma
     if (n_tasks == 0) return cudaSuccess;
     const bool units16 = !(L & 1u) && ((reinterpret_cast<uintptr_t>(v) | reinterpret_cast<uintptr_t>(mask)) & 15u) == 0;
     const uint32_t U = units16 ? L / 2 : L;
-    uint32_t log2g = 0;
-    while (log2g < 5 && (1u << log2g) < U) ++log2g;
+    const uint32_t log2g = group_log2(U);
     count_launch();
     if (units16)
         return launch_kernel(seg_decrypt_kernel<uint4>, seg_grid(n_tasks), kSegThreads, 0, stream,
@@ -245,6 +416,48 @@ cudaError_t launch_seg_decrypt(const uint64_t *v, uint32_t L, const uint64_t *ma
     return launch_kernel(seg_decrypt_kernel<uint2>, seg_grid(n_tasks), kSegThreads, 0, stream,
                          reinterpret_cast<const uint2 *>(v), U, log2g, reinterpret_cast<const uint2 *>(mask), off, tasks,
                          n_tasks, counts);
+}
+
+cudaError_t launch_seg_cancel_insert(const uint64_t *v, uint32_t L, bool units16, const SegCancelTask *tasks,
+                                     uint32_t n_tasks, const SegCancelScratch &s, cudaStream_t stream) {
+    if (n_tasks == 0) return cudaSuccess;
+    const uint32_t U = units16 ? L / 2 : L, log2g = group_log2(U);
+    const uint32_t grid = seg_grid(n_tasks);
+    count_launch();
+    if (units16) {
+        const uint4 *v4 = reinterpret_cast<const uint4 *>(v);
+        return log2g == 5 ? launch_kernel(seg_cancel_insert_kernel<uint4, true>, grid, kSegThreads, 0, stream, v4, U,
+                                          log2g, tasks, n_tasks, s)
+                          : launch_kernel(seg_cancel_insert_kernel<uint4, false>, grid, kSegThreads, 0, stream, v4, U,
+                                          log2g, tasks, n_tasks, s);
+    }
+    const uint2 *v2 = reinterpret_cast<const uint2 *>(v);
+    return log2g == 5 ? launch_kernel(seg_cancel_insert_kernel<uint2, true>, grid, kSegThreads, 0, stream, v2, U, log2g,
+                                      tasks, n_tasks, s)
+                      : launch_kernel(seg_cancel_insert_kernel<uint2, false>, grid, kSegThreads, 0, stream, v2, U,
+                                      log2g, tasks, n_tasks, s);
+}
+
+cudaError_t launch_seg_cancel_count(const SegCancelTask *tasks, uint32_t n_tasks, const SegCancelScratch &s,
+                                    uint32_t *live, cudaStream_t stream) {
+    if (n_tasks == 0) return cudaSuccess;
+    count_launch();
+    return launch_kernel(seg_cancel_count_kernel, seg_grid(n_tasks), kSegThreads, 0, stream, tasks, n_tasks, s, live);
+}
+
+cudaError_t launch_seg_cancel_write(const uint64_t *v, uint32_t L, bool units16, const SegCancelTask *tasks,
+                                    uint32_t n_tasks, const SegCancelScratch &s, const uint64_t *base, uint64_t *out,
+                                    cudaStream_t stream) {
+    if (n_tasks == 0) return cudaSuccess;
+    const uint32_t U = units16 ? L / 2 : L;
+    count_launch();
+    if (units16)
+        return launch_kernel(seg_cancel_write_kernel<uint4>, seg_grid(n_tasks), kSegThreads, 0, stream,
+                             reinterpret_cast<const uint4 *>(v), reinterpret_cast<uint4 *>(out), U, group_log2(U),
+                             tasks, n_tasks, s, base);
+    return launch_kernel(seg_cancel_write_kernel<uint2>, seg_grid(n_tasks), kSegThreads, 0, stream,
+                         reinterpret_cast<const uint2 *>(v), reinterpret_cast<uint2 *>(out), U, group_log2(U), tasks,
+                         n_tasks, s, base);
 }
 
 }  // namespace csgn

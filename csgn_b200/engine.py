@@ -285,6 +285,11 @@ class Ciphertext:
         satisfied-block count under every key of the context."""
         return CiphertextArray(self, [0, self.n_blocks]).compact().storage
 
+    def cancel(self):
+        """A new ciphertext keeping the first occurrence of every block value that occurs an odd number of times (see
+        CiphertextArray.cancel): the same decryption under every key, a satisfied-block count of the same parity."""
+        return CiphertextArray(self, [0, self.n_blocks]).cancel().storage
+
     def permute_into(self, perm, out):
         check(_lib().csgn_permute_into(self._h, perm._h, out._h))
         return out
@@ -478,6 +483,17 @@ class CiphertextArray:
         """The array without the blocks that have fewer than D set bits (no key of the context satisfies them): every
         element keeps its other blocks in order and decrypts as before under every key."""
         return CiphertextArray.sum_of_products([], [self], compact=True)
+
+    def cancel(self):
+        """csgn_seg_cancel: every element keeps, in order, the first occurrence of each block value that occurs an odd
+        number of times in it (x*x -> x, a + a -> empty).  Equal blocks are satisfied by the same keys, so every
+        element decrypts as before under every key; unlike compact(), its satisfied-block count changes (by an even
+        number).  The usual gate is sum_of_products(..., compact=True).cancel()."""
+        out_off = np.empty(len(self) + 1, dtype=np.uint64)
+        h = _vp()
+        check(_lib().csgn_seg_cancel(self.storage._h, self.offsets.ctypes.data_as(_vp), len(self),
+                                     out_off.ctypes.data_as(_vp), ctypes.byref(h)))
+        return CiphertextArray(Ciphertext(h, self.ctx), out_off)
 
     def gather(self, idx):
         """csgn_seg_gather: element j = self_{idx[j]} (any order, repeats allowed)."""

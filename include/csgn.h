@@ -272,6 +272,11 @@ int csgn_seg_mul_sum_compact(const csgn_buf *const *a, const uint64_t *const *a_
                              const uint64_t *const *b_off, uint32_t n_products, const csgn_buf *const *c,
                              const uint64_t *const *c_off, uint32_t n_terms, uint64_t n, uint32_t min_bits,
                              uint64_t *out_off, csgn_buf **out);
+/* element k = the first occurrence, in order, of every block value that occurs an odd number of times in element k.
+ * Equal blocks are satisfied by the same keys, so every decryption is unchanged under every key; satisfied-block
+ * counts change by an even number.  Sizes depend on the data: the call returns after its counting pass.  Equality is
+ * decided on all L words; the result depends on nothing else.  An element may hold at most 2^30 blocks. */
+int csgn_seg_cancel(const csgn_buf *c, const uint64_t *c_off, uint64_t n, uint64_t *out_off, csgn_buf **out);
 /* element j = src_{idx[j]}, j < m: any order, repeats allowed; idx[j] < n_src is checked. */
 int csgn_seg_gather(const csgn_buf *src, const uint64_t *src_off, uint64_t n_src, const uint64_t *idx, uint64_t m,
                     uint64_t *out_off, csgn_buf **out);

@@ -15,6 +15,12 @@
           satisfy are kept): the 12-bit adder over 4096 lanes with plain and with compacting carry gates, the 32-bit adder
           compacted (uncompacted its last carry would hold 2^32 - 1 blocks per lane), and compact() on its own over the
           uncompacted 12-bit carry -- time, bytes written by the carry gates, and blocks held per lane after every gate
+  cancel  cancellation (csgn_seg_cancel: per element, the first occurrence of every block value that occurs an odd
+          number of times): cancel() on its own over 4096 elements of 100 blocks with repeated values (time, blocks
+          per second, input bytes per second against a device-to-device copy), and the 6-bit multiplier (product mod
+          64) over 1024 lanes, random and all-ones, with every gate compacted, with and without cancellation -- time
+          and blocks per lane after every gate (without cancellation only where every gate stays under 40 GB and half
+          the free device memory)
   sweep   elements whose product is 64 KB .. 64 MB, ~1 GB per call: the grouped kernel against one launch_mul per
           element (CSGN_SEG_LARGE_BYTES), which sets the large-element threshold of capi_seg.cu
 
@@ -37,6 +43,7 @@ os.environ.setdefault("CSGN_TUNING", "1")      # CSGN_SEG_LARGE_BYTES is honoure
 import torch  # noqa: E402
 
 from csgn_b200 import engine as eng  # noqa: E402
+from oracle.pyoracle import pad_mask  # noqa: E402
 
 LINES = []
 
@@ -370,6 +377,112 @@ def compaction(ctx, key, rng, lanes):
     torch.cuda.empty_cache()
 
 
+class TooLarge(Exception):
+    pass
+
+
+def multiplier(X, Y, gate):
+    """Product mod 2^n of the bit arrays X[i], Y[i]: schoolbook rows, ripple-carry adds, every sum and carry one
+    gate(products, terms); None is an all-zero bit"""
+    n = len(X)
+    acc = [None] * n
+    for j in range(n):
+        pp = [None] * j + [gate([(X[i], Y[j])], []) for i in range(n - j)]
+        c, out = None, []
+        for k in range(n):
+            ops = [x for x in (acc[k], pp[k], c) if x is not None]
+            out.append(gate([], ops) if ops else None)
+            prods = [(ops[p], ops[q]) for p in range(len(ops)) for q in range(p + 1, len(ops))]
+            c = gate(prods, []) if prods else None
+        acc = out
+    return acc
+
+
+def cancellation(ctx, key, rng, n_elems, lanes, bits, budget_bytes):
+    L = ctx.L
+    # cancel() alone: about 100 blocks per element drawn from 70 values each, so most values repeat
+    per, vals_per = 100, 70
+    vals = torch.randint(-2**62, 2**62, (n_elems, vals_per, L), dtype=torch.int64, device="cuda")
+    idx = torch.randint(0, vals_per, (n_elems, per), device="cuda")
+    vals[:, :, L - 1] &= int(np.int64(np.uint64(pad_mask(ctx.N))))           # pad bits zero, as the library leaves them
+    words = torch.gather(vals, 1, idx.unsqueeze(-1).expand(-1, -1, L)).reshape(-1).contiguous()
+    X = eng.CiphertextArray(eng.Ciphertext.from_tensor(words, ctx), np.arange(n_elems + 1, dtype=np.uint64) * per)
+    blocks, nbytes = n_elems * per, n_elems * per * L * 8
+    cp = copy_rate(nbytes)
+    keep = []
+
+    def once():
+        keep[:] = [X.cancel()]
+    t, reps = timed(once)
+    kept = keep[0].storage.n_blocks
+    nl = launches(once)
+    keep.clear()
+    log("cancel: cancel() of %d elements x %d blocks (%d values each), Context(%d,%d), %.1f MB in (less than the 126 MB "
+        "L2: repeated calls may read it from there): "
+        "%8.3f ms (%d calls, %d launches)  %.0f M blocks/s  %.0f GB/s of input  %.2f of a device copy of the same bytes "
+        "(%.0f GB/s)  %d of %d blocks kept" % (n_elems, per, vals_per, ctx.N, ctx.D, nbytes / 1e6, t * 1e3, reps, nl,
+                                             blocks / t / 1e6, nbytes / t / 1e9, nbytes / t / cp, cp / 1e9, kept,
+                                             blocks))
+    del X, vals, idx, words
+    torch.cuda.empty_cache()
+
+    # the n-bit multiplier over `lanes` lanes, every gate compacted, with and without cancellation
+    SP = eng.CiphertextArray.sum_of_products
+    for lanes_kind in ("random", "all-ones"):
+        r = np.random.default_rng(bits)
+        if lanes_kind == "random":
+            xb, yb = r.integers(0, 1 << bits, lanes), r.integers(0, 1 << bits, lanes)
+        else:
+            xb = yb = np.full(lanes, (1 << bits) - 1)
+        plain = np.concatenate([np.concatenate([(v >> i) & 1 for i in range(bits)]) for v in (xb, yb)]).astype(np.uint8)
+        allb = key.encrypt_array(plain, seed=13)
+        rows = [allb.gather(np.arange(q * lanes, (q + 1) * lanes)) for q in range(2 * bits)]
+        for cancel in (True, False):
+            held = []
+
+            def gate(products, terms):
+                out = sum(int(np.dot(np.diff(a.offsets.astype(np.int64)), np.diff(b.offsets.astype(np.int64))))
+                          for a, b in products) + sum(int(c.offsets[-1]) for c in terms)
+                # the gate's product blocks, and the result before compaction in the worst case, next to what is held
+                limit = min(budget_bytes, eng.device_info()["hbm_free"] // 2)
+                if out * L * 8 > limit:
+                    raise TooLarge("a gate of %.1f GB before compaction, %.1f GB allowed" % (out * L * 8 / 1e9,
+                                                                                          limit / 1e9))
+                g = SP(products, terms, compact=True)
+                if cancel:
+                    g = g.cancel()
+                held.append(g.storage.n_blocks / lanes)
+                return g
+
+            def run():
+                held.clear()
+                return multiplier(rows[:bits], rows[bits:], gate)
+            name = "compact + cancel" if cancel else "compact alone   "
+            try:
+                P = run()
+            except TooLarge as e:
+                log("cancel: %d-bit multiplier, %d %s lanes, %s: does not fit (%s)" % (bits, lanes, lanes_kind, name, e))
+                torch.cuda.empty_cache()
+                continue
+            got = sum(key.decrypt_array(P[i])[0].astype(np.int64) << i for i in range(bits))
+            assert np.array_equal(got, (xb * yb) % (1 << bits)), "%d-bit multiplier wrong" % bits
+            out_bits = [P[i].storage.n_blocks / lanes for i in range(bits)]
+            del P
+            torch.cuda.empty_cache()
+
+            def circuit():
+                keep[:] = [run()]
+            t, reps = timed(circuit, min_s=2.0, min_reps=2)
+            keep.clear()
+            torch.cuda.empty_cache()
+            log("cancel: %d-bit multiplier (product mod 2^%d), %d %s lanes, Context(%d,%d), %s: %8.2f ms (%d runs), "
+                "%d gates, at most %.1f blocks per lane after a gate; output bits %s blocks per lane" % (
+                    bits, bits, lanes, lanes_kind, ctx.N, ctx.D, name, t * 1e3, reps, len(held), max(held),
+                    " ".join("%.1f" % h for h in out_bits)))
+            log("cancel: %d-bit %s lanes, %s, blocks per lane after each gate: %s" % (
+                bits, lanes_kind, name.strip(), " ".join("%.1f" % h for h in held)))
+
+
 def sweep(ctx, total_bytes, sizes_kb):
     L = ctx.L
     for kb in sizes_kb:
@@ -403,7 +516,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default="")
     ap.add_argument("--quick", action="store_true", help="small sizes (a check of the script, not a measurement)")
-    ap.add_argument("--only", default="small,mixed,adder,gates,compact,sweep")
+    ap.add_argument("--only", default="small,mixed,adder,gates,compact,cancel,sweep")
     args = ap.parse_args()
     torch.cuda.set_device(0)
     eng.init(0)
@@ -434,6 +547,12 @@ def main():
             compaction(ctx, key, rng, 256 if args.quick else 4096)
         else:
             log("compact: skipped, %s has no csgn_seg_mul_sum_compact" % os.environ.get("CSGN_LIBRARY", "this build"))
+    if "cancel" in only:
+        if hasattr(eng._lib(), "csgn_seg_cancel"):
+            cancellation(ctx, key, rng, 256 if args.quick else 4096, 128 if args.quick else 1024, 4 if args.quick else 6,
+                         40 << 30)
+        else:
+            log("cancel: skipped, %s has no csgn_seg_cancel" % os.environ.get("CSGN_LIBRARY", "this build"))
     if "sweep" in only:
         sweep(ctx, (64 << 20) if args.quick else (1 << 30),
               [64, 256] if args.quick else [64, 256, 1024, 4096, 16384, 65536])

@@ -89,6 +89,9 @@ SIGNATURES = {
     "csgn_concat_n": (ctypes.c_int, [ctypes.POINTER(_vp), _u64, _vpp]),
     "csgn_seg_decrypt_count_async": (ctypes.c_int, [_vp, _vp, _u64, _vp, _vp]),
     "csgn_seg_decrypt": (ctypes.c_int, [_vp, _vp, _u64, _vp, _vp, _vp]),
+    "csgn_seg_circuit": (ctypes.c_int, [ctypes.POINTER(_vp), ctypes.POINTER(_vp), ctypes.c_uint32, _u64, _vp, _u64,
+                                        ctypes.c_uint32, _vp, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_int, _u64,
+                                        ctypes.POINTER(_vp), ctypes.POINTER(_vp), _u64p]),
     "csgn_perm_create": (ctypes.c_int, [_u64, _vp, _vpp]),
     "csgn_perm_free": (ctypes.c_int, [_vp]),
     "csgn_permute": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vpp]),

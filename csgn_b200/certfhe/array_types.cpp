@@ -204,6 +204,60 @@ Ciphertext Ciphertext::cancel() const {
     return out;
 }
 
+Circuit::Circuit(uint32_t inputs) : inputs(inputs) {
+    if (inputs == 0) throw Error("Circuit: a circuit needs at least one input");
+}
+
+uint32_t Circuit::gate(const std::vector<std::pair<uint32_t, uint32_t>> &products, const std::vector<uint32_t> &terms) {
+    if (products.empty() && terms.empty()) throw Error("Circuit::gate: no products and no terms");
+    const uint32_t own = wires();
+    for (const auto &pr : products)
+        if (pr.first >= own || pr.second >= own) throw Error("Circuit::gate: an operand is not an earlier wire");
+    for (uint32_t w : terms)
+        if (w >= own) throw Error("Circuit::gate: a term is not an earlier wire");
+    netlist.push_back((uint32_t)products.size());
+    netlist.push_back((uint32_t)terms.size());
+    for (const auto &pr : products) {
+        netlist.push_back(pr.first);
+        netlist.push_back(pr.second);
+    }
+    netlist.insert(netlist.end(), terms.begin(), terms.end());
+    return inputs + gates++;
+}
+
+std::vector<CiphertextArray> Circuit::evaluate(const std::vector<CiphertextArray> &in,
+                                               const std::vector<uint32_t> &outputs, int64_t minBits, bool cancel,
+                                               uint64_t laneCapacity) {
+    if (in.size() != inputs) throw Error("Circuit::evaluate: wrong number of input arrays");
+    if (outputs.empty()) throw Error("Circuit::evaluate: no outputs");
+    const uint64_t n = in[0].size();
+    const Context &ctx = in[0].context;
+    std::vector<const csgn_buf *> bufs;
+    std::vector<const uint64_t *> offs;
+    for (const CiphertextArray &x : in) {
+        if (x.size() != n) throw Error("Circuit::evaluate: input arrays of different sizes");
+        if (x.context.getN() != ctx.getN() || x.context.getD() != ctx.getD())
+            throw Error("Circuit::evaluate: input arrays of different contexts");
+        bufs.push_back(x.storage.get());
+        offs.push_back(x.offsets.data());
+    }
+    for (uint32_t w : outputs)
+        if (w >= wires()) throw Error("Circuit::evaluate: an output is not a wire of the circuit");
+    if (minBits > 64 * (int64_t)csgn_words_per_block(ctx.getN())) throw Error("Circuit::evaluate: minBits out of range");
+    const uint32_t mb = minBits < 0 ? (uint32_t)ctx.getD() : (uint32_t)minBits;
+    std::vector<std::vector<uint64_t>> off(outputs.size(), std::vector<uint64_t>(n + 1));
+    std::vector<uint64_t *> off_p;
+    for (auto &o : off) off_p.push_back(o.data());
+    std::vector<csgn_buf *> res(outputs.size(), nullptr);
+    glue::check(csgn_seg_circuit(bufs.data(), offs.data(), inputs, n, netlist.data(), netlist.size(), gates,
+                                 outputs.data(), (uint32_t)outputs.size(), mb, cancel ? 1 : 0, laneCapacity,
+                                 off_p.data(), res.data(), &fallback),
+                "csgn_seg_circuit");
+    std::vector<CiphertextArray> out;
+    for (size_t j = 0; j < outputs.size(); ++j) out.push_back(CiphertextArray(res[j], off[j], ctx));
+    return out;
+}
+
 CiphertextArray SecretKey::encryptArray(const unsigned char *bits, uint64_t n, uint64_t seed) {
     if (!device_key) {
         glue::ensure_engine();

@@ -332,6 +332,7 @@ class CiphertextArray {
     static CiphertextArray gate(const std::vector<std::pair<CiphertextArray, CiphertextArray>> &products,
                                 const std::vector<CiphertextArray> &terms, bool compact);
     friend class SecretKey;
+    friend class Circuit;
 
 public:
     // Packs the ciphertexts into one array with one launch (csgn_concat_n); pending products and lazy sums are
@@ -366,6 +367,29 @@ public:
 
     const std::vector<uint64_t> &getOffsets() const;
     const csgn_buf *deviceBuffer() const;
+};
+
+// ---- Circuit (extension; include/csgn.h, "circuits") ----------------------------------------------------------------
+// A netlist of gates over CiphertextArrays, evaluated over every lane in one call (csgn_seg_circuit) instead of one
+// call per gate.  Wires 0 .. inputs - 1 are the inputs; gate() adds sum(u*v) + sum(terms) over earlier wires and
+// returns its wire.  Throws Error on a gate with no operands or an operand that is not an earlier wire.
+class Circuit {
+    uint32_t inputs, gates = 0;
+    std::vector<uint32_t> netlist;   // per gate: p, q, the p operand pairs, the q terms
+    uint64_t fallback = 0;
+
+public:
+    explicit Circuit(uint32_t inputs);
+    uint32_t gate(const std::vector<std::pair<uint32_t, uint32_t>> &products, const std::vector<uint32_t> &terms = {});
+    // The arrays of wires `outputs` over the lanes of `inputs` (one array per input wire, all of the same size and
+    // context): each gate compacted to minBits set bits (-1: D of the context; 0: no compaction) and, with cancel,
+    // cancelled, as compactSumOfProducts(...).cancel() would give.  laneCapacity: blocks per lane on the device (0: the
+    // library chooses).  Throws Error on mismatched sizes or contexts, or a bad output wire.
+    std::vector<CiphertextArray> evaluate(const std::vector<CiphertextArray> &inputs,
+                                          const std::vector<uint32_t> &outputs, int64_t minBits = -1,
+                                          bool cancel = false, uint64_t laneCapacity = 0);
+    uint64_t lastFallback() const { return fallback; }   // lanes of the last evaluate() evaluated gate by gate
+    uint32_t wires() const { return inputs + gates; }
 };
 
 // ---- Timer (reference src/Timer.h:13-74) -------------------------------------------------

@@ -1,5 +1,6 @@
 // capi_internal.cuh -- shared by the translation units that implement include/csgn.h (capi.cu: library, buffers,
-// the hot path, batches; capi_comm.cu: the peer communicator; capi_io.cu: save / load; capi_seg.cu: ciphertext arrays): the handle types, the
+// the hot path, batches; capi_comm.cu: the peer communicator; capi_io.cu: save / load; capi_seg.cu: ciphertext arrays;
+// capi_circuit.cu: circuits over ciphertext arrays): the handle types, the
 // process-wide state and the small helpers every entry point uses.  Internal: not part of the C ABI.
 #pragma once
 
@@ -198,6 +199,22 @@ int stage_to_device(const void *host, size_t bytes, void **out);
 int stage_into(void *d, const void *host, size_t bytes);
 // `bytes` of device memory `d` to `host` on the current stream, through the pinned staging, and wait for the copy.
 int read_back(void *host, const void *d, size_t bytes);
+
+// A device table, released in stream order after the launches that read it.
+struct DevTable {
+    void *d = nullptr;
+    ~DevTable() { dev_free(d); }
+};
+
+// Ciphertext arrays (capi_seg.cu), shared with the circuits (capi_circuit.cu).  The offsets of an n-element array
+// over `buf` (off[0] == 0, non-decreasing, off[n] == its blocks); `what` names the array in the message.
+int check_offsets(const csgn_buf *buf, const uint64_t *off, uint64_t n, const char *what);
+// An output of `total` blocks of L words stays addressable in bytes.
+int check_blocks(uint64_t total, uint32_t L);
+// Allocate an output of `blocks` blocks and fill it with src[0] (words[0] words) || src[1] || ... in one launch of the
+// piece copy (none without pieces); *out only on success.
+int gather_into_new(uint64_t blocks, uint32_t L, const std::vector<const uint64_t *> &src,
+                    const std::vector<uint64_t> &words, csgn_buf **out);
 
 // Scope of one batch call: item i runs with the work stream set to way i % n, where way 0 is the caller's own stream
 // and ways 1.. are the library's side lanes, forked from the caller's stream on construction; join() makes the

@@ -26,6 +26,11 @@ uint64_t task_words(uint64_t total_words) {
     return std::min(kSegTaskMaxWords, std::max(kSegTaskMinWords, total_words / (2 * warps)));
 }
 
+}  // namespace
+
+namespace csgn {
+namespace detail {
+
 int check_offsets(const csgn_buf *buf, const uint64_t *off, uint64_t n, const char *what) {
     if (!off) return fail(CSGN_ERR_INVALID_ARGUMENT, "%s: null offsets", what);
     if (off[0] != 0)
@@ -45,11 +50,48 @@ int check_blocks(uint64_t total, uint32_t L) {
     return CSGN_OK;
 }
 
-// A device table, released in stream order after the launches that read it.
-struct DevTable {
-    void *d = nullptr;
-    ~DevTable() { dev_free(d); }
-};
+// out = src[0] || src[1] || ... (words[p] words from src[p]) in one launch of the piece copy.
+int copy_pieces(const std::vector<const uint64_t *> &src, const std::vector<uint64_t> &words, csgn_buf *out) {
+    const size_t n = src.size();
+    if (n == 0) return CSGN_OK;
+    if (n >= UINT32_MAX) return fail(CSGN_ERR_INVALID_ARGUMENT, "more than 2^32 - 2 pieces to copy");
+    bool u16 = (reinterpret_cast<uintptr_t>(out->d) & 15u) == 0;
+    for (size_t p = 0; p < n && u16; ++p) u16 = (reinterpret_cast<uintptr_t>(src[p]) & 15u) == 0 && words[p] % 2 == 0;
+    // table: n + 1 destination offsets (units), then n source pointers
+    std::vector<uint64_t> tab(2 * n + 1);
+    for (size_t p = 0; p < n; ++p) {
+        tab[p + 1] = tab[p] + (u16 ? words[p] / 2 : words[p]);
+        tab[n + 1 + p] = (uint64_t)reinterpret_cast<uintptr_t>(src[p]);
+    }
+    DevTable t;
+    int rc = stage_to_device(tab.data(), tab.size() * sizeof(uint64_t), &t.d);
+    if (rc != CSGN_OK) return rc;
+    const uint64_t *d = static_cast<const uint64_t *>(t.d);
+    cudaError_t e = launch_piece_copy(reinterpret_cast<const void *const *>(d + n + 1), d, (uint32_t)n, tab[n], u16,
+                                      out->d, g.stream);
+    return e == cudaSuccess ? CSGN_OK : cuda_fail(e, "piece copy kernel");
+}
+
+// Allocate an output of `blocks` blocks and fill it from `src`/`words`; *out only on success.
+int gather_into_new(uint64_t blocks, uint32_t L, const std::vector<const uint64_t *> &src,
+                    const std::vector<uint64_t> &words, csgn_buf **out) {
+    csgn_buf *c = nullptr;
+    int rc = new_buf(blocks, L, 0, &c);
+    if (rc != CSGN_OK) return rc;
+    acquire_write(c);
+    rc = copy_pieces(src, words, c);
+    if (rc != CSGN_OK) {
+        csgn_buf_free(c);
+        return rc;
+    }
+    *out = c;
+    return CSGN_OK;
+}
+
+}  // namespace detail
+}  // namespace csgn
+
+namespace {
 
 // The work of one grouped multiply (seg_mul_kernel), added piece by piece in output order: products, and plain terms
 // (items whose left operand is the all-ones block at the head of the staged table).  Small pieces become items packed
@@ -228,44 +270,6 @@ private:
     std::vector<SegMulItem> items_;
     std::vector<uint32_t> tasks_ = std::vector<uint32_t>(1, 0);
 };
-
-// out = src[0] || src[1] || ... (words[p] words from src[p]) in one launch of the piece copy.
-int copy_pieces(const std::vector<const uint64_t *> &src, const std::vector<uint64_t> &words, csgn_buf *out) {
-    const size_t n = src.size();
-    if (n == 0) return CSGN_OK;
-    if (n >= UINT32_MAX) return fail(CSGN_ERR_INVALID_ARGUMENT, "more than 2^32 - 2 pieces to copy");
-    bool u16 = (reinterpret_cast<uintptr_t>(out->d) & 15u) == 0;
-    for (size_t p = 0; p < n && u16; ++p) u16 = (reinterpret_cast<uintptr_t>(src[p]) & 15u) == 0 && words[p] % 2 == 0;
-    // table: n + 1 destination offsets (units), then n source pointers
-    std::vector<uint64_t> tab(2 * n + 1);
-    for (size_t p = 0; p < n; ++p) {
-        tab[p + 1] = tab[p] + (u16 ? words[p] / 2 : words[p]);
-        tab[n + 1 + p] = (uint64_t)reinterpret_cast<uintptr_t>(src[p]);
-    }
-    DevTable t;
-    int rc = stage_to_device(tab.data(), tab.size() * sizeof(uint64_t), &t.d);
-    if (rc != CSGN_OK) return rc;
-    const uint64_t *d = static_cast<const uint64_t *>(t.d);
-    cudaError_t e = launch_piece_copy(reinterpret_cast<const void *const *>(d + n + 1), d, (uint32_t)n, tab[n], u16,
-                                      out->d, g.stream);
-    return e == cudaSuccess ? CSGN_OK : cuda_fail(e, "piece copy kernel");
-}
-
-// Allocate an output of `blocks` blocks and fill it from `src`/`words`; *out only on success.
-int gather_into_new(uint64_t blocks, uint32_t L, const std::vector<const uint64_t *> &src,
-                    const std::vector<uint64_t> &words, csgn_buf **out) {
-    csgn_buf *c = nullptr;
-    int rc = new_buf(blocks, L, 0, &c);
-    if (rc != CSGN_OK) return rc;
-    acquire_write(c);
-    rc = copy_pieces(src, words, c);
-    if (rc != CSGN_OK) {
-        csgn_buf_free(c);
-        return rc;
-    }
-    *out = c;
-    return CSGN_OK;
-}
 
 // csgn_seg_mul_sum, and with compact csgn_seg_mul_sum_compact: the same checks, items and output order, plus
 // 1 <= min_bits <= 64 L.

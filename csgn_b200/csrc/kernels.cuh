@@ -112,6 +112,31 @@ cudaError_t launch_seg_cancel_write(const uint64_t *v, uint32_t L, bool units16,
                                     uint32_t n_tasks, const SegCancelScratch &s, const uint64_t *base, uint64_t *out,
                                     cudaStream_t stream);
 
+// Circuits (circuit.cu, csgn_seg_circuit): one warp per lane evaluates every gate of a netlist over that lane.  Wire w
+// < n_inputs of lane k is element k of input w (in_base[w] + in_off[w * (n + 1) + k] blocks); gate g, whose p, q,
+// operand pairs and terms start at gates[gate_at[g]], defines wire n_inputs + g.  After gate g the wires
+// frees[free_at[g] .. free_at[g + 1]) are dead.  A lane's gate wires live in its slice of `arena` (cap blocks from
+// block k * cap); wires[] holds kCircuitWireBytes per wire per resident warp.  For every lane and output j,
+// res[2 (k n_out + j)] and [+1] are the block position in the lane's slice and the block count of wire outputs[j]
+// (gate wires only); fallback[k] = 1 when the lane did not fit (its res entries are then meaningless).  `next` is a
+// zeroed lane counter.  One launch.
+struct CircuitArgs {
+    const uint32_t *gates, *gate_at, *frees, *free_at, *outputs;
+    const uint64_t *in_base, *in_off;
+    uint64_t *arena, *res;
+    void *wires;
+    uint32_t *fallback;
+    unsigned long long *next;
+    uint64_t n, cap;
+    uint32_t n_inputs, n_gates, n_outputs, min_bits, cancel;
+};
+constexpr uint32_t kCircuitWireBytes = 16;
+// The largest gate output (after compaction) that the kernel cancels; a larger one sends its lane to the fallback.
+constexpr uint32_t kCircuitCancelBlocks = 1024;
+// Resident warps of the circuit kernel for these arguments (the size of its wire tables).
+uint32_t circuit_warps(uint64_t n, bool units16, bool cancel);
+cudaError_t launch_circuit(const CircuitArgs &a, uint32_t L, bool units16, cudaStream_t stream);
+
 // out[0] = sum of in[0..n): the partial counts of a ciphertext held as several segments (a lazy sum)
 cudaError_t launch_sum_words(const uint64_t *in, uint32_t n, uint64_t *out, cudaStream_t stream);
 

@@ -17,6 +17,7 @@
 #include "kernels.cuh"
 #include "launch.cuh"
 #include "fold.cuh"
+#include "seg_device.cuh"
 
 #include <algorithm>
 
@@ -25,13 +26,6 @@ namespace {
 
 constexpr int kSegThreads = 256;
 constexpr int kSegCtasPerSm = 8;
-
-__device__ __forceinline__ uint4 vand(const uint4 x, const uint4 y) {
-    return make_uint4(x.x & y.x, x.y & y.y, x.z & y.z, x.w & y.w);
-}
-__device__ __forceinline__ uint2 vand(const uint2 x, const uint2 y) { return make_uint2(x.x & y.x, x.y & y.y); }
-__device__ __forceinline__ uint32_t vpopc(const uint4 x) { return __popc(x.x) + __popc(x.y) + __popc(x.z) + __popc(x.w); }
-__device__ __forceinline__ uint32_t vpopc(const uint2 x) { return __popc(x.x) + __popc(x.y); }
 
 // Modes of the grouped multiply: kSegPlain writes every block at its item's `out`; kSegCount writes, per item, the
 // number of its blocks with at least min_bits set bits (live[it]); kSegWriteLive writes only those blocks, in order,
@@ -204,25 +198,8 @@ seg_decrypt_kernel(const VT *__restrict__ v, const uint32_t U, const uint32_t lo
 // leader probes alone and compares serially (groups probe different numbers of slots, so no warp vote runs there);
 // with G = 32 (WARP_BLOCK) the warp holds one block, every lane takes every probe, and lane 0's atomicCAS is broadcast.
 // The insert pass asks for 4 resident CTAs per SM: left to its own register target, ptxas spills in the probe loops.
+// (The hash and the unit helpers are in seg_device.cuh, shared with the circuit kernel.)
 // ---------------------------------------------------------------------------------------
-__device__ __forceinline__ uint64_t mix64(uint64_t x) {
-    x ^= x >> 30;
-    x *= 0xbf58476d1ce4e5b9ull;
-    x ^= x >> 27;
-    x *= 0x94d049bb133111ebull;
-    return x ^ (x >> 31);
-}
-__device__ __forceinline__ uint64_t word_hash(uint64_t x, uint64_t w) { return mix64(x + (w + 1) * 0x9e3779b97f4a7c15ull); }
-__device__ __forceinline__ uint64_t unit_hash(const uint2 u, uint32_t w) {
-    return word_hash((uint64_t)u.y << 32 | u.x, w);
-}
-__device__ __forceinline__ uint64_t unit_hash(const uint4 u, uint32_t w) {
-    return word_hash((uint64_t)u.y << 32 | u.x, 2ull * w) + word_hash((uint64_t)u.w << 32 | u.z, 2ull * w + 1);
-}
-__device__ __forceinline__ bool veq(const uint2 x, const uint2 y) { return x.x == y.x && x.y == y.y; }
-__device__ __forceinline__ bool veq(const uint4 x, const uint4 y) {
-    return x.x == y.x && x.y == y.y && x.z == y.z && x.w == y.w;
-}
 
 // Block b (of the whole array) survives when it is the first of its value's blocks and the value occurs an odd number
 // of times in its element.

@@ -511,6 +511,66 @@ class CiphertextArray:
         return CiphertextArray(self.storage.applyPermutation(perm), self.offsets.copy())
 
 
+class Circuit:
+    """A netlist of gates over ciphertext arrays, evaluated over every lane in one call (csgn_seg_circuit).  Wires 0 ..
+    n_inputs - 1 are the inputs; gate(products, terms) adds the gate sum(u*v for (u, v) in products) + sum(terms) over
+    earlier wires and returns its wire."""
+
+    def __init__(self, n_inputs):
+        if n_inputs < 1:
+            raise ValueError("a circuit needs at least one input")
+        self.n_inputs = int(n_inputs)
+        self.n_gates = 0
+        self._gates = []
+        self.last_fallback = None       # lanes of the last evaluate() that took the gate-by-gate path
+
+    @property
+    def n_wires(self):
+        return self.n_inputs + self.n_gates
+
+    def gate(self, products=(), terms=()):
+        products = [(int(u), int(v)) for u, v in products]
+        terms = [int(w) for w in terms]
+        if not products and not terms:
+            raise ValueError("a gate needs at least one product or term")
+        for w in [x for pr in products for x in pr] + terms:
+            if not 0 <= w < self.n_wires:
+                raise ValueError("wire %d is not below the gate's own wire %d" % (w, self.n_wires))
+        self._gates += [len(products), len(terms)] + [x for pr in products for x in pr] + terms
+        self.n_gates += 1
+        return self.n_wires - 1
+
+    def evaluate(self, inputs, outputs, min_bits=None, cancel=False, lane_capacity=0):
+        """The arrays of wires `outputs` over the lanes of `inputs` (one CiphertextArray per input wire, all of n
+        elements): each gate as sum_of_products, compacted to min_bits set bits (None: D of the context; 0: no
+        compaction) and, with cancel, cancelled.  lane_capacity: blocks per lane on the device (0: the library chooses);
+        lanes that do not fit are evaluated gate by gate (last_fallback counts them)."""
+        inputs = list(inputs)
+        outputs = [int(w) for w in outputs]
+        if len(inputs) != self.n_inputs:
+            raise ValueError("the circuit has %d inputs, got %d arrays" % (self.n_inputs, len(inputs)))
+        n, ctx = len(inputs[0]), inputs[0].ctx
+        for x in inputs[1:]:
+            if len(x) != n:
+                raise ValueError("arrays of %d and %d elements" % (n, len(x)))
+            if (x.ctx.N, x.ctx.D) != (ctx.N, ctx.D):
+                raise ValueError("arrays of Context(%d,%d) and Context(%d,%d)" % (ctx.N, ctx.D, x.ctx.N, x.ctx.D))
+        if not outputs:
+            raise ValueError("evaluate needs at least one output wire")
+        gates = np.asarray(self._gates, dtype=np.uint32)
+        outs = np.asarray(outputs, dtype=np.uint32)
+        out_offs = [np.empty(n + 1, dtype=np.uint64) for _ in outputs]
+        out = (_vp * len(outputs))()
+        fallback = ctypes.c_uint64(0)
+        check(_lib().csgn_seg_circuit(
+            handle_array([x.storage for x in inputs]), (_vp * len(inputs))(*[x.offsets.ctypes.data for x in inputs]),
+            len(inputs), n, gates.ctypes.data_as(_vp), gates.size, self.n_gates, outs.ctypes.data_as(_vp), outs.size,
+            ctx.D if min_bits is None else int(min_bits), 1 if cancel else 0, int(lane_capacity),
+            (_vp * len(outputs))(*[o.ctypes.data for o in out_offs]), out, ctypes.byref(fallback)))
+        self.last_fallback = fallback.value
+        return [CiphertextArray(Ciphertext(_vp(out[j]), ctx), out_offs[j]) for j in range(len(outputs))]
+
+
 class Result:
     """A decrypt whose count the host reads later (csgn_result)."""
 

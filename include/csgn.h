@@ -290,6 +290,25 @@ int csgn_seg_decrypt_count_async(const csgn_buf *c, const uint64_t *c_off, uint6
 int csgn_seg_decrypt(const csgn_buf *c, const uint64_t *c_off, uint64_t n, const csgn_key *key, uint8_t *bits,
                      uint64_t *counts);
 
+/* ---- circuits ----------------------------------------------------------------------------------------------------
+ * Evaluate a circuit over n lanes.
+ * Wires 0 .. n_inputs-1 are the input arrays.  Gate g defines wire n_inputs + g.
+ * gates[] is flat: for each gate, p, q, then p operand pairs (u0, v0, ...), then q terms (w0, ...).
+ * Every operand is a wire below the gate's own.
+ * Output j (offsets to out_off[j][0..n], array to out[j]) is, word for word, what evaluating the gates in order gives
+ * for wire outputs[j]: each gate with csgn_seg_mul_sum (min_bits == 0) or csgn_seg_mul_sum_compact(min_bits), followed
+ * by csgn_seg_cancel when `cancel` is set; an output that names an input wire is a copy of that input.  Lanes are
+ * independent, so the call evaluates every lane in ONE launch with one host synchronisation: a lane's gate wires live in
+ * an arena slice of lane_capacity blocks (0: the library chooses from free memory), each wire freed at its last use.
+ * Lanes that do not fit (or whose gate output to cancel exceeds a fixed table) are evaluated gate by gate with the calls
+ * above; *n_fallback (optional) reports how many.  The checks run on the host and allocate nothing on error: null
+ * arguments, the offsets of every input, equal L, gates_len against the gates it encodes, p + q >= 1, operands below
+ * the gate's wire, output indices, 0 <= min_bits <= 64*L. */
+int csgn_seg_circuit(const csgn_buf *const *in, const uint64_t *const *in_off, uint32_t n_inputs, uint64_t n,
+                     const uint32_t *gates, uint64_t gates_len, uint32_t n_gates,
+                     const uint32_t *outputs, uint32_t n_outputs, uint32_t min_bits, int cancel,
+                     uint64_t lane_capacity, uint64_t *const *out_off, csgn_buf **out, uint64_t *n_fallback);
+
 /* Permutation as a device source map: out_bit[i] = in_bit[perm[i]], i < N
  * (src/Ciphertext.cpp:33-34).  Fails unless perm is a bijection of [0,N). */
 int csgn_perm_create(uint64_t N, const uint64_t *perm, csgn_perm **out);

@@ -21,6 +21,11 @@
           64) over 1024 lanes, random and all-ones, with every gate compacted, with and without cancellation -- time
           and blocks per lane after every gate (without cancellation only where every gate stays under 40 GB and half
           the free device memory)
+  circuit whole circuits in one csgn_seg_circuit call against the gate-by-gate loop (sum_of_products(compact=True),
+          then cancel() when cancelling), alternating in the same run: the 12-bit and 32-bit adders over 4096 lanes and
+          the 6-bit multiplier over 1024 random and all-ones lanes, each with compaction alone and with compaction plus
+          cancellation -- time, launches, fallback lanes, the largest blocks per lane after a gate, and the loop's time
+          split into device time (torch.profiler) and host work plus synchronisation
   sweep   elements whose product is 64 KB .. 64 MB, ~1 GB per call: the grouped kernel against one launch_mul per
           element (CSGN_SEG_LARGE_BYTES), which sets the large-element threshold of capi_seg.cu
 
@@ -483,6 +488,91 @@ def cancellation(ctx, key, rng, n_elems, lanes, bits, budget_bytes):
                 bits, lanes_kind, name.strip(), " ".join("%.1f" % h for h in held)))
 
 
+def ripple_adder(X, Y, gate):
+    """Sum bits and final carry of the bit arrays X[i] + Y[i]: s_i = t + c with t = x_i + y_i, c' = x_i*y_i + t*c"""
+    S = [gate([], [X[0], Y[0]])]
+    c = gate([(X[0], Y[0])], [])
+    for i in range(1, len(X)):
+        t = gate([], [X[i], Y[i]])
+        S.append(gate([], [t, c]))
+        c = gate([(X[i], Y[i]), (t, c)], [])
+    return S + [c]
+
+
+def circuits(ctx, key, workloads):
+    """Each workload as ONE csgn_seg_circuit call and as the gate-by-gate loop (sum_of_products(compact=True), then
+    cancel() when cancelling), alternating in the same run; the outputs of both must agree word for word and decrypt to
+    the plaintext.  The loop's time is split into device time (kernels and copies, torch.profiler over one run) and the
+    rest (host work and synchronisation)."""
+    from torch.profiler import ProfilerActivity, profile
+    SP = eng.CiphertextArray.sum_of_products
+    for name, build, bits, lanes, kind in workloads:
+        r = np.random.default_rng(bits * 7 + lanes)
+        if kind == "random":
+            xb, yb = r.integers(0, 1 << bits, lanes), r.integers(0, 1 << bits, lanes)
+        else:
+            xb = yb = np.full(lanes, (1 << bits) - 1)
+        plain = np.concatenate([np.concatenate([(v >> i) & 1 for i in range(bits)]) for v in (xb, yb)]).astype(np.uint8)
+        allb = key.encrypt_array(plain, seed=17)
+        rows = [allb.gather(np.arange(q * lanes, (q + 1) * lanes)) for q in range(2 * bits)]
+        want = (xb + yb) if build is ripple_adder else (xb * yb) % (1 << bits)
+        C = eng.Circuit(2 * bits)
+        outs = [w for w in build(list(range(bits)), list(range(bits, 2 * bits)), C.gate) if w is not None]
+        for cancel in (False, True):
+            setting = "compact + cancel" if cancel else "compact alone"
+            held = []
+
+            def gate(products, terms):
+                g = SP(products, terms, compact=True)
+                if cancel:
+                    g = g.cancel()
+                held.append(g.storage.n_blocks / lanes)
+                return g
+            keep = []
+
+            def one_call():
+                keep[:] = C.evaluate(rows, outs, cancel=cancel)
+
+            def loop():
+                keep[:] = [w for w in build(rows[:bits], rows[bits:], gate) if w is not None]
+            one_call()
+            P1 = list(keep)
+            held.clear()
+            loop()
+            P2 = list(keep)
+            for a, b in zip(P1, P2):
+                assert np.array_equal(a.offsets, b.offsets) and a.storage.checksum() == b.storage.checksum(), name
+            got = sum(key.decrypt_array(P1[i])[0].astype(np.int64) << i for i in range(len(P1)))
+            assert np.array_equal(got, want), "%s: wrong result" % name
+            fallback, most = C.last_fallback, max(held)
+            del P1, P2
+            keep.clear()
+            n1, n2 = launches(one_call), launches(loop)
+            t1, t2 = [], []
+            for _ in range(5):                                 # alternating
+                t1.append(timed(one_call, min_s=0.4, min_reps=2)[0])
+                t2.append(timed(loop, min_s=0.4, min_reps=2)[0])
+            keep.clear()
+            torch.cuda.synchronize()
+            with profile(activities=[ProfilerActivity.CUDA]) as prof:
+                loop()
+                torch.cuda.synchronize()
+            dev = sum(e.device_time_total for e in prof.key_averages()                 # kernels and copies, us
+                      if e.device_type == torch.autograd.DeviceType.CUDA) / 1e6
+            keep.clear()
+            torch.cuda.empty_cache()
+            m1, m2 = float(np.median(t1)), float(np.median(t2))
+            log("circuit: %s, %d %s lanes, Context(%d,%d), %s, %d gates: one call %8.2f ms (%d launches, %d fallback "
+                "lanes) | gate by gate %8.2f ms (%d launches: %.2f ms on the device, %.2f ms host and synchronisation) | "
+                "one call / gate by gate %.3f | at most %.1f blocks per lane after a gate" % (
+                    name, lanes, kind, ctx.N, ctx.D, setting, C.n_gates, m1 * 1e3, n1, fallback, m2 * 1e3, n2,
+                    dev * 1e3, (m2 - dev) * 1e3, m1 / m2, most))
+            log("circuit: %s %s %s, runs (ms) one call %s | gate by gate %s" % (
+                name, kind, setting, " ".join("%.2f" % (x * 1e3) for x in t1), " ".join("%.2f" % (x * 1e3) for x in t2)))
+        del rows, allb
+        torch.cuda.empty_cache()
+
+
 def sweep(ctx, total_bytes, sizes_kb):
     L = ctx.L
     for kb in sizes_kb:
@@ -516,7 +606,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default="")
     ap.add_argument("--quick", action="store_true", help="small sizes (a check of the script, not a measurement)")
-    ap.add_argument("--only", default="small,mixed,adder,gates,compact,cancel,sweep")
+    ap.add_argument("--only", default="small,mixed,adder,gates,compact,cancel,circuit,sweep")
     args = ap.parse_args()
     torch.cuda.set_device(0)
     eng.init(0)
@@ -553,6 +643,15 @@ def main():
                          40 << 30)
         else:
             log("cancel: skipped, %s has no csgn_seg_cancel" % os.environ.get("CSGN_LIBRARY", "this build"))
+    if "circuit" in only:
+        if hasattr(eng._lib(), "csgn_seg_circuit"):
+            q = args.quick
+            circuits(ctx, key, [("12-bit adder", ripple_adder, 12, 256 if q else 4096, "random"),
+                                ("32-bit adder", ripple_adder, 8 if q else 32, 256 if q else 4096, "random"),
+                                ("6-bit multiplier", multiplier, 4 if q else 6, 128 if q else 1024, "random"),
+                                ("6-bit multiplier", multiplier, 4 if q else 6, 128 if q else 1024, "all-ones")])
+        else:
+            log("circuit: skipped, %s has no csgn_seg_circuit" % os.environ.get("CSGN_LIBRARY", "this build"))
     if "sweep" in only:
         sweep(ctx, (64 << 20) if args.quick else (1 << 30),
               [64, 256] if args.quick else [64, 256, 1024, 4096, 16384, 65536])

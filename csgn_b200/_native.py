@@ -92,6 +92,9 @@ SIGNATURES = {
     "csgn_seg_circuit": (ctypes.c_int, [ctypes.POINTER(_vp), ctypes.POINTER(_vp), ctypes.c_uint32, _u64, _vp, _u64,
                                         ctypes.c_uint32, _vp, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_int, _u64,
                                         ctypes.POINTER(_vp), ctypes.POINTER(_vp), _u64p]),
+    "csgn_encrypt_uint": (ctypes.c_int, [_vp, _vp, _u64, ctypes.c_uint32, _u64, _u64, ctypes.POINTER(_vp)]),
+    "csgn_decrypt_uint_async": (ctypes.c_int, [ctypes.POINTER(_vp), ctypes.POINTER(_vp), ctypes.c_uint32, _u64, _vp, _vp]),
+    "csgn_decrypt_uint": (ctypes.c_int, [ctypes.POINTER(_vp), ctypes.POINTER(_vp), ctypes.c_uint32, _u64, _vp, _vp]),
     "csgn_perm_create": (ctypes.c_int, [_u64, _vp, _vpp]),
     "csgn_perm_free": (ctypes.c_int, [_vp]),
     "csgn_permute": (ctypes.c_int, [_vp, _vp, ctypes.c_int, _vpp]),

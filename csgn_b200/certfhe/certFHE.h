@@ -35,6 +35,8 @@ struct csgn_result;
 namespace certFHE {
 
 class CiphertextArray;
+class EncryptedUInt;
+class UIntCircuit;
 
 // Raised where the reference would run into undefined behaviour or where the GPU
 // engine reports a failure.  The reference has no error channel at all; an uncaught
@@ -301,6 +303,11 @@ public:
     // decryption of every element of an array with one launch and one synchronisation (csgn_seg_decrypt).
     CiphertextArray encryptArray(const unsigned char *bits, uint64_t n, uint64_t seed);
     void decryptArray(const CiphertextArray &array, unsigned char *bits);
+    // Extension: n integers of `width` bits (1..64) as an EncryptedUInt, one launch (csgn_encrypt_uint); throws Error
+    // on a value that does not fit.  decryptUInt writes x.size() values with one launch and one synchronisation
+    // (csgn_decrypt_uint).
+    EncryptedUInt encryptUInt(const uint64_t *values, uint64_t n, uint32_t width, uint64_t seed);
+    void decryptUInt(const EncryptedUInt &x, uint64_t *values);
     void applyPermutation_inplace(const Permutation &permutation);
     SecretKey applyPermutation(const Permutation &permutation);
 
@@ -333,6 +340,7 @@ class CiphertextArray {
                                 const std::vector<CiphertextArray> &terms, bool compact);
     friend class SecretKey;
     friend class Circuit;
+    friend class UIntCircuit;
 
 public:
     // Packs the ciphertexts into one array with one launch (csgn_concat_n); pending products and lazy sums are
@@ -390,6 +398,90 @@ public:
                                           bool cancel = false, uint64_t laneCapacity = 0);
     uint64_t lastFallback() const { return fallback; }   // lanes of the last evaluate() evaluated gate by gate
     uint32_t wires() const { return inputs + gates; }
+    uint32_t inputCount() const { return inputs; }
+    const std::vector<uint32_t> &getNetlist() const { return netlist; }
+};
+
+// ---- encrypted integers (extension; include/csgn.h, "encrypted integers") ------------------------------------------
+// A vector of n encrypted W-bit unsigned integers: W CiphertextArrays of n elements, its bit planes, LSB first.  The
+// operators + - * (mod 2^W), < > (1-bit results) and & ^ | build a one-operation UIntCircuit and make one call, compacted
+// and cancelled; operands may differ in width (the shorter is zero-extended).  Throws Error on arrays of different sizes or contexts.
+class EncryptedUInt {
+    std::vector<CiphertextArray> planes;
+
+public:
+    explicit EncryptedUInt(const std::vector<CiphertextArray> &planes);
+    uint32_t width() const { return (uint32_t)planes.size(); }
+    uint64_t size() const { return planes[0].size(); }
+    const std::vector<CiphertextArray> &getPlanes() const { return planes; }
+    Context getContext() const { return planes[0].getContext(); }
+
+    EncryptedUInt operator+(const EncryptedUInt &b) const;
+    EncryptedUInt operator-(const EncryptedUInt &b) const;
+    EncryptedUInt operator*(const EncryptedUInt &b) const;
+    EncryptedUInt operator<(const EncryptedUInt &b) const;
+    EncryptedUInt operator>(const EncryptedUInt &b) const;
+    EncryptedUInt operator&(const EncryptedUInt &b) const;
+    EncryptedUInt operator^(const EncryptedUInt &b) const;
+    EncryptedUInt operator|(const EncryptedUInt &b) const;
+    // c ? x : y lane by lane (c of 1 bit)
+    static EncryptedUInt select(const EncryptedUInt &c, const EncryptedUInt &x, const EncryptedUInt &y);
+};
+
+// Integer netlists, built on the host and evaluated as ONE Circuit call; the netlists of the Python UIntCircuit,
+// wire for wire.  An integer is a vector of wires, LSB first.  Wires: operand i, bit j is input i*width + j; then the
+// `one` input (one = true: the caller passes an encryption of 1 per lane to evaluate); then the zero input (n empty
+// elements, supplied by evaluate).  Every operation is a sum of products plus terms; a gate that folds to one wire
+// (x + 0, x*1, a single term) adds no gate.  eq, le, ge and invert need `one` and throw Error without it.  Cancelled
+// results hold the blocks of their function's algebraic normal form: small for add, bitwise, select and shifts at any
+// width, about threefold per bit for sub, neg, comparisons, min, max and mul (practical up to about 8-12 bits).
+class UIntCircuit {
+public:
+    typedef std::vector<uint32_t> UInt;
+
+    UIntCircuit(uint32_t width, uint32_t operands, bool one = false);
+    const std::vector<UInt> &inputs() const { return in; }
+    uint32_t width() const { return w; }
+    const Circuit &circuit() const { return c; }
+    uint64_t lastFallback() const { return c.lastFallback(); }
+
+    UInt add(const UInt &a, const UInt &b);
+    UInt sub(const UInt &a, const UInt &b);
+    UInt neg(const UInt &a);
+    UInt lt(const UInt &a, const UInt &b);
+    UInt gt(const UInt &a, const UInt &b);
+    UInt ne(const UInt &a, const UInt &b);
+    UInt eq(const UInt &a, const UInt &b);
+    UInt le(const UInt &a, const UInt &b);
+    UInt ge(const UInt &a, const UInt &b);
+    UInt invert(const UInt &a);
+    UInt select(const UInt &s, const UInt &x, const UInt &y);
+    UInt min(const UInt &a, const UInt &b);
+    UInt max(const UInt &a, const UInt &b);
+    UInt mul(const UInt &a, const UInt &b);
+    UInt and_(const UInt &a, const UInt &b);
+    UInt xor_(const UInt &a, const UInt &b);
+    UInt or_(const UInt &a, const UInt &b);
+    UInt shl(const UInt &a, uint32_t k);
+    UInt shr(const UInt &a, uint32_t k);
+
+    // One csgn_seg_circuit call for every result.  operands: one EncryptedUInt per operand, of at most width() bits;
+    // one: the array that encrypts 1 in every lane, for a circuit built with one = true (null otherwise).
+    std::vector<EncryptedUInt> evaluate(const std::vector<EncryptedUInt> &operands, const std::vector<UInt> &results,
+                                        int64_t minBits = -1, bool cancel = false, uint64_t laneCapacity = 0,
+                                        const CiphertextArray *one = nullptr);
+
+private:
+    uint32_t w, operands;
+    bool has_one;
+    uint32_t one_w, zero_w;
+    std::vector<UInt> in;
+    Circuit c;
+
+    uint32_t gate(std::vector<std::pair<uint32_t, uint32_t>> products, std::vector<uint32_t> terms);
+    uint32_t notw(uint32_t x);
+    uint32_t borrow(uint32_t a, uint32_t b, uint32_t r, uint32_t t);
+    void pair(UInt &a, UInt &b) const;
 };
 
 // ---- Timer (reference src/Timer.h:13-74) -------------------------------------------------

@@ -1616,6 +1616,61 @@ int csgn_encrypt_batch(const csgn_key *key, const uint8_t *bits, uint64_t n, uin
     return CSGN_OK;
 }
 
+int csgn_encrypt_uint(const csgn_key *key, const uint64_t *values, uint64_t n, uint32_t width, uint64_t first_block,
+                      uint64_t seed, csgn_buf **out) {
+    NEED_INIT();
+    if (!key || !out || (n && !values)) return fail(CSGN_ERR_INVALID_ARGUMENT, "null argument");
+    if (width < 1 || width > 64) return fail(CSGN_ERR_INVALID_ARGUMENT, "width %u outside 1..64", width);
+    if (key->D == 0) return fail(CSGN_ERR_INVALID_ARGUMENT, "the key has no secret positions");
+    if (width < 64)
+        for (uint64_t k = 0; k < n; ++k)
+            if (values[k] >> width)
+                return fail(CSGN_ERR_INVALID_ARGUMENT, "values[%llu] = %llu does not fit in %u bits",
+                            (unsigned long long)k, (unsigned long long)values[k], width);
+    const uint32_t L = key->L;
+    if (n > UINT64_MAX / 64) return fail(CSGN_ERR_INVALID_ARGUMENT, "block count overflows");
+    int rc = check_blocks(width * n, L);
+    if (rc != CSGN_OK) return rc;
+    // one allocation for the width planes, laid one after another as the kernel writes them
+    csgn_slab *sl = new csgn_slab;
+    sl->cap_words = std::max<uint64_t>(1, width * n * L);
+    rc = dev_alloc(sl->cap_words, &sl->d);
+    if (rc != CSGN_OK) {
+        delete sl;
+        return rc;
+    }
+    if (n) {
+        DevTable v;
+        rc = stage_to_device(values, n * sizeof(uint64_t), &v.d);
+        const uint64_t rem = key->N % 64;
+        const uint64_t pad = rem ? ~0ull << (64 - rem) : ~0ull;
+        cudaError_t e = cudaSuccess;
+        if (rc == CSGN_OK)
+            e = launch_encrypt_uint(static_cast<const uint64_t *>(v.d), n, width, first_block, L, pad, key->d_mask,
+                                    key->d_positions, key->D, seed, sl->d, g.stream);
+        if (rc == CSGN_OK && e != cudaSuccess) rc = cuda_fail(e, "integer encryption");
+        if (rc != CSGN_OK) {
+            dev_free(sl->d);
+            delete sl;
+            return rc;
+        }
+    }
+    const uint64_t tick = g.tick++;
+    for (uint32_t j = 0; j < width; ++j) {
+        csgn_buf *b = new csgn_buf;
+        b->d = sl->d + j * n * L;
+        b->n_blocks = n;
+        b->L = L;
+        b->cap_words = 0;
+        b->owns = false;
+        b->slab = sl;
+        b->writer = {g.stream, tick};
+        out[j] = b;
+    }
+    sl->refs = width;
+    return CSGN_OK;
+}
+
 // ---------------------------------------------------------------------------
 // K4 permute
 // ---------------------------------------------------------------------------

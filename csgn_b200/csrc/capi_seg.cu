@@ -376,6 +376,27 @@ int mul_sum(const csgn_buf *const *a, const uint64_t *const *a_off, const csgn_b
 
 }  // namespace
 
+namespace {
+
+// The arguments of the integer decrypt: width 1..64, every plane an n-element array of the key's L.
+int check_uint_planes(const csgn_buf *const *planes, const uint64_t *const *plane_off, uint32_t width, uint64_t n,
+                      const csgn_key *key) {
+    if (!planes || !plane_off || !key) return fail(CSGN_ERR_INVALID_ARGUMENT, "null argument");
+    if (width < 1 || width > 64) return fail(CSGN_ERR_INVALID_ARGUMENT, "width %u outside 1..64", width);
+    if (n > UINT64_MAX / 8 / (width + 1)) return fail(CSGN_ERR_INVALID_ARGUMENT, "too many elements");
+    for (uint32_t j = 0; j < width; ++j) {
+        if (!planes[j]) return fail(CSGN_ERR_INVALID_ARGUMENT, "null plane %u", j);
+        if (planes[j]->L != key->L)
+            return fail(CSGN_ERR_SHAPE_MISMATCH, "plane %u has %u words per block, key expects %u", j, planes[j]->L,
+                        key->L);
+        int rc = check_offsets(planes[j], plane_off[j], n, "integer plane");
+        if (rc != CSGN_OK) return rc;
+    }
+    return CSGN_OK;
+}
+
+}  // namespace
+
 extern "C" {
 
 int csgn_seg_mul(const csgn_buf *a, const uint64_t *a_off, const csgn_buf *b, const uint64_t *b_off, uint64_t n,
@@ -736,6 +757,127 @@ int csgn_seg_decrypt(const csgn_buf *c, const uint64_t *c_off, uint64_t n, const
         if (counts) counts[k] = h[k];
     }
     return CSGN_OK;
+}
+
+int csgn_decrypt_uint_async(const csgn_buf *const *planes, const uint64_t *const *plane_off, uint32_t width,
+                            uint64_t n, const csgn_key *key, uint64_t *device_values) {
+    NEED_INIT();
+    if (n && !device_values) return fail(CSGN_ERR_INVALID_ARGUMENT, "null argument");
+    int rc = check_uint_planes(planes, plane_off, width, n, key);
+    if (rc != CSGN_OK || n == 0) return rc;
+    const uint32_t L = key->L;
+    bool units16 = true;
+    for (uint32_t j = 0; j < width; ++j) {
+        rc = need_dense(planes[j]);
+        if (rc != CSGN_OK) return rc;
+        acquire_read(planes[j]);
+        units16 = units16 && (reinterpret_cast<uintptr_t>(planes[j]->d) & 15u) == 0;
+    }
+    CU(cudaMemsetAsync(device_values, 0, n * sizeof(uint64_t), g.stream));
+    // As in csgn_seg_decrypt_count_async, plane by plane: runs of small elements cut into tasks of about `target`
+    // blocks, and every element of large_words() or more counted on its own into scratch.
+    const uint64_t large = large_words();
+    uint64_t small_words = 0;
+    for (uint32_t j = 0; j < width; ++j)
+        for (uint64_t k = 0; k < n; ++k) {
+            const uint64_t w = (plane_off[j][k + 1] - plane_off[j][k]) * L;
+            if (w < large) small_words += w;
+        }
+    const uint64_t target = std::max<uint64_t>(1, task_words(small_words) / L);
+    std::vector<SegDecTask> tasks;
+    std::vector<uint32_t> task_plane;
+    std::vector<uint64_t> large_entries;   // (element, plane) of every large element
+    std::vector<std::pair<const uint64_t *, uint64_t>> large_blocks;
+    for (uint32_t j = 0; j < width; ++j) {
+        const uint64_t *off = plane_off[j];
+        SegDecTask cur = {0, 0, 0, 0};
+        bool open = false;
+        auto close = [&]() {
+            if (open) {
+                tasks.push_back(cur);
+                task_plane.push_back(j);
+            }
+            open = false;
+        };
+        for (uint64_t k = 0; k < n; ++k) {
+            const uint64_t o0 = off[k], o1 = off[k + 1];
+            if (o0 == o1) continue;
+            if ((o1 - o0) * L >= large) {
+                close();
+                large_entries.push_back(k);
+                large_entries.push_back(j);
+                large_blocks.push_back({planes[j]->d + o0 * L, o1 - o0});
+                continue;
+            }
+            for (uint64_t p = o0; p < o1;) {
+                if (!open) {
+                    cur = {p, p, k, k};
+                    open = true;
+                }
+                const uint64_t take = std::min(o1 - p, target - (cur.end - cur.first));
+                cur.end = p + take;
+                cur.elem_last = k;
+                p += take;
+                if (cur.end - cur.first >= target) close();
+            }
+        }
+        close();
+    }
+    if (tasks.size() >= UINT32_MAX || large_blocks.size() >= UINT32_MAX)
+        return fail(CSGN_ERR_INVALID_ARGUMENT, "too many work items");
+    // one device table: width * (n + 1) offsets, the plane table, the tasks, the large entries, the tasks' planes
+    const uint64_t t_off = 0, t_planes = width * (n + 1), t_tasks = t_planes + 2 * width,
+                   t_large = t_tasks + 4 * tasks.size(), t_tplane = t_large + large_entries.size();
+    std::vector<uint64_t> tab(t_tplane + (task_plane.size() + 1) / 2);
+    for (uint32_t j = 0; j < width; ++j) memcpy(tab.data() + t_off + j * (n + 1), plane_off[j], (n + 1) * 8);
+    if (!tasks.empty()) memcpy(tab.data() + t_tasks, tasks.data(), tasks.size() * sizeof(SegDecTask));
+    if (!large_entries.empty()) memcpy(tab.data() + t_large, large_entries.data(), large_entries.size() * 8);
+    if (!task_plane.empty()) memcpy(tab.data() + t_tplane, task_plane.data(), task_plane.size() * sizeof(uint32_t));
+    uint64_t *d = nullptr;
+    rc = dev_alloc(tab.size(), &d);
+    if (rc != CSGN_OK) return rc;
+    DevTable t;
+    t.d = d;
+    for (uint32_t j = 0; j < width; ++j) {
+        tab[t_planes + 2 * j] = (uint64_t)reinterpret_cast<uintptr_t>(planes[j]->d);
+        tab[t_planes + 2 * j + 1] = (uint64_t)reinterpret_cast<uintptr_t>(d + t_off + j * (n + 1));
+    }
+    rc = stage_into(d, tab.data(), tab.size() * sizeof(uint64_t));
+    if (rc != CSGN_OK) return rc;
+    cudaError_t e = launch_seg_decrypt_uint(reinterpret_cast<const SegPlane *>(d + t_planes), units16, L, key->d_mask,
+                                            reinterpret_cast<const SegDecTask *>(d + t_tasks),
+                                            reinterpret_cast<const uint32_t *>(d + t_tplane), (uint32_t)tasks.size(),
+                                            device_values, g.stream);
+    if (e != cudaSuccess) return cuda_fail(e, "integer decrypt kernel");
+    if (!large_blocks.empty()) {
+        DevTable counts;
+        rc = dev_alloc(large_blocks.size(), reinterpret_cast<uint64_t **>(&counts.d));
+        if (rc != CSGN_OK) return rc;
+        uint64_t *c = static_cast<uint64_t *>(counts.d);
+        const uint64_t *hm = key->h_mask.empty() ? nullptr : key->h_mask.data();
+        for (size_t i = 0; i < large_blocks.size() && e == cudaSuccess; ++i)
+            e = launch_decrypt_count(large_blocks[i].first, large_blocks[i].second, L, key->d_mask, hm, fold_scratch(),
+                                     c + i, g.stream, nullptr, folds_overlap());
+        if (e == cudaSuccess)
+            e = launch_seg_uint_pack(c, d + t_large, (uint32_t)large_blocks.size(), device_values, g.stream);
+        if (e != cudaSuccess) return cuda_fail(e, "integer decrypt of large elements");
+    }
+    return CSGN_OK;
+}
+
+int csgn_decrypt_uint(const csgn_buf *const *planes, const uint64_t *const *plane_off, uint32_t width, uint64_t n,
+                      const csgn_key *key, uint64_t *values) {
+    NEED_INIT();
+    if (n && !values) return fail(CSGN_ERR_INVALID_ARGUMENT, "null argument");
+    int rc = check_uint_planes(planes, plane_off, width, n, key);   // before the allocation: nothing allocated on error
+    if (rc != CSGN_OK || n == 0) return rc;
+    uint64_t *d = nullptr;
+    rc = dev_alloc(n, &d);
+    if (rc != CSGN_OK) return rc;
+    rc = csgn_decrypt_uint_async(planes, plane_off, width, n, key, d);
+    if (rc == CSGN_OK) rc = read_back(values, d, n * sizeof(uint64_t));
+    dev_free(d);
+    return rc;
 }
 
 }  // extern "C"

@@ -12,6 +12,9 @@
 // the CPU restatement the tests compare against, bit for bit).  Three forms: short even blocks
 // (a warp builds 32 blocks, coalesced), long blocks (a warp builds one block), and a lane-per-block
 // form for odd L.  The work is ten Philox rounds per 16 bytes.
+//
+// Each form reads its plaintext bits from one of two sources: a byte per block (csgn_encrypt_batch), or the bit planes
+// of n integers laid one after another (csgn_encrypt_uint: block i encrypts bit i / n of values[i % n]).
 #include "kernels.cuh"
 #include "launch.cuh"
 
@@ -35,17 +38,29 @@ __device__ __forceinline__ uint4 philox4x32_10(uint32_t c0, uint32_t c1, uint32_
 
 constexpr uint32_t kTag = 0x43534731u;
 
+// Bit i of the planes of n integers: plane j = i / n (LSB first), element k = i - j*n.  The quotient comes from the
+// host's magic = floor((2^64 - 1) / n): umulhi(i, magic) is floor(i / n) or one less, and one step corrects it.
+__device__ __forceinline__ bool plane_bit(const UIntPlanes &p, uint64_t i) {
+    uint64_t j = __umul64hi(i, p.magic), k = i - j * p.n;
+    if (k >= p.n) {
+        ++j;
+        k -= p.n;
+    }
+    return (__ldg(p.values + k) >> j) & 1u;
+}
+
+template <bool PLANES>
 __global__ void __launch_bounds__(256)
 encrypt_batch_kernel(const uint8_t *__restrict__ bits, const uint64_t n, const uint64_t first_block,
                      const uint32_t L, const uint64_t pad_mask, const uint64_t *__restrict__ mask,
                      const uint64_t *__restrict__ positions, const uint32_t D, const uint32_t k0, const uint32_t k1,
-                     uint64_t *__restrict__ out) {
+                     uint64_t *__restrict__ out, const UIntPlanes planes) {
     pdl_enter();
     const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
         const uint64_t b = first_block + i;
         const uint32_t b_lo = (uint32_t)b, b_hi = (uint32_t)(b >> 32);
-        const bool one = __ldg(bits + i) & 1u;
+        const bool one = PLANES ? plane_bit(planes, i) : (__ldg(bits + i) & 1u);
         uint64_t hole = 0, hbit = 0, hole_word = 0;
         if (!one) {
             const uint4 r = philox4x32_10(b_lo, b_hi, 0xffffffffu, kTag, k0, k1);
@@ -83,12 +98,12 @@ encrypt_batch_kernel(const uint8_t *__restrict__ bits, const uint64_t n, const u
 // lane and step.  "Every other secret bit is 1" is a per-block AND across lanes: as in the decrypt
 // kernel, each step's ballot goes into a per-warp fail string and lane b reads block b's bits; the
 // lane then patches the hole word of its block.
-template <int L4C>
+template <int L4C, bool PLANES>
 __global__ void __launch_bounds__(256)
 encrypt_batch_units_kernel(const uint8_t *__restrict__ bits, const uint64_t n, const uint64_t first_block,
                            const uint32_t L4rt, const uint64_t pad_mask, const uint64_t *__restrict__ mask,
                            const uint64_t *__restrict__ positions, const uint32_t D, const uint32_t k0,
-                           const uint32_t k1, uint64_t *__restrict__ out) {
+                           const uint32_t k1, uint64_t *__restrict__ out, const UIntPlanes planes) {
     constexpr int kWarps = 8;
     __shared__ uint64_t sMask[64];               // 2*L4 <= 64 words
     __shared__ uint32_t sFail[kWarps][32];       // L4 <= 32 ballot words per warp
@@ -105,7 +120,7 @@ encrypt_batch_units_kernel(const uint8_t *__restrict__ bits, const uint64_t n, c
         // lane b prepares block b of the chunk: its bit and, for Enc(0), its hole
         const uint64_t my_i = chunk * 32u + lane;
         uint32_t my_hole = 0xffffffffu;
-        if (my_i < n && !(__ldg(bits + my_i) & 1u)) {
+        if (my_i < n && !(PLANES ? plane_bit(planes, my_i) : (__ldg(bits + my_i) & 1u))) {
             const uint64_t b = first_block + my_i;
             const uint4 r = philox4x32_10((uint32_t)b, (uint32_t)(b >> 32), 0xffffffffu, kTag, k0, k1);
             my_hole = (uint32_t)__ldg(positions + (r.x % D));
@@ -155,11 +170,12 @@ encrypt_batch_units_kernel(const uint8_t *__restrict__ bits, const uint64_t n, c
 
 // Long blocks (L >= 64 words, e.g. N=16383): one WARP builds one block, lanes striding over the
 // 16-byte units -- coalesced 512-byte stores per step; the "other secret bits" flag is a warp vote.
+template <bool PLANES>
 __global__ void __launch_bounds__(256)
 encrypt_batch_warp_kernel(const uint8_t *__restrict__ bits, const uint64_t n, const uint64_t first_block,
                           const uint32_t L, const uint64_t pad_mask, const uint64_t *__restrict__ mask,
                           const uint64_t *__restrict__ positions, const uint32_t D, const uint32_t k0,
-                          const uint32_t k1, uint64_t *__restrict__ out) {
+                          const uint32_t k1, uint64_t *__restrict__ out, const UIntPlanes planes) {
     pdl_enter();
     const uint32_t lane = threadIdx.x & 31u;
     const uint64_t warp_global = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -168,7 +184,7 @@ encrypt_batch_warp_kernel(const uint8_t *__restrict__ bits, const uint64_t n, co
     for (uint64_t i = warp_global; i < n; i += n_warps) {
         const uint64_t b = first_block + i;
         const uint32_t b_lo = (uint32_t)b, b_hi = (uint32_t)(b >> 32);
-        const bool one = __ldg(bits + i) & 1u;
+        const bool one = PLANES ? plane_bit(planes, i) : (__ldg(bits + i) & 1u);
         uint64_t hole = 0, hbit = 0;
         if (!one) {
             const uint4 r = philox4x32_10(b_lo, b_hi, 0xffffffffu, kTag, k0, k1);   // same value on every lane
@@ -204,16 +220,20 @@ encrypt_batch_warp_kernel(const uint8_t *__restrict__ bits, const uint64_t n, co
 
 }  // namespace
 
-cudaError_t launch_encrypt_batch(const uint8_t *bits, uint64_t n, uint64_t first_block, uint32_t L, uint64_t pad_mask,
-                                 const uint64_t *mask, const uint64_t *positions, uint32_t D, uint64_t seed,
-                                 uint64_t *out, cudaStream_t stream) {
+namespace {
+
+template <bool PLANES>
+cudaError_t launch_encrypt(const uint8_t *bits, const UIntPlanes &planes, uint64_t n, uint64_t first_block, uint32_t L,
+                           uint64_t pad_mask, const uint64_t *mask, const uint64_t *positions, uint32_t D, uint64_t seed,
+                           uint64_t *out, cudaStream_t stream) {
     if (n == 0) return cudaSuccess;
     count_launch();
+    const uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
     if (L >= 64) {
         const uint32_t wgrid = (uint32_t)std::max<uint64_t>(
             1, std::min<uint64_t>((n + 7) / 8, (uint64_t)device_props().sm_count * 8));
-        return launch_kernel(encrypt_batch_warp_kernel, wgrid, 256, 0, stream, bits, n, first_block, L, pad_mask, mask,
-                             positions, D, (uint32_t)seed, (uint32_t)(seed >> 32), out);
+        return launch_kernel(encrypt_batch_warp_kernel<PLANES>, wgrid, 256, 0, stream, bits, n, first_block, L, pad_mask,
+                             mask, positions, D, k0, k1, out, planes);
     }
     const bool aligned = (reinterpret_cast<uintptr_t>(out) & 15u) == 0;
     if (!(L & 1u) && L <= 64 && aligned && !env_long("CSGN_ENC_LANE", 0)) {
@@ -221,15 +241,31 @@ cudaError_t launch_encrypt_batch(const uint8_t *bits, uint64_t n, uint64_t first
         const uint32_t ugrid = (uint32_t)std::max<uint64_t>(
             1, std::min<uint64_t>((n_chunks + 7) / 8, (uint64_t)device_props().sm_count * 8));
         if (L == 20)
-            return launch_kernel(encrypt_batch_units_kernel<10>, ugrid, 256, 0, stream, bits, n, first_block, L / 2,
-                                 pad_mask, mask, positions, D, (uint32_t)seed, (uint32_t)(seed >> 32), out);
-        return launch_kernel(encrypt_batch_units_kernel<0>, ugrid, 256, 0, stream, bits, n, first_block, L / 2, pad_mask,
-                             mask, positions, D, (uint32_t)seed, (uint32_t)(seed >> 32), out);
+            return launch_kernel(encrypt_batch_units_kernel<10, PLANES>, ugrid, 256, 0, stream, bits, n, first_block,
+                                 L / 2, pad_mask, mask, positions, D, k0, k1, out, planes);
+        return launch_kernel(encrypt_batch_units_kernel<0, PLANES>, ugrid, 256, 0, stream, bits, n, first_block, L / 2,
+                             pad_mask, mask, positions, D, k0, k1, out, planes);
     }
     const uint32_t grid = (uint32_t)std::max<uint64_t>(
         1, std::min<uint64_t>((n + 255) / 256, (uint64_t)device_props().sm_count * 8));
-    return launch_kernel(encrypt_batch_kernel, grid, 256, 0, stream, bits, n, first_block, L, pad_mask, mask, positions,
-                         D, (uint32_t)seed, (uint32_t)(seed >> 32), out);
+    return launch_kernel(encrypt_batch_kernel<PLANES>, grid, 256, 0, stream, bits, n, first_block, L, pad_mask, mask,
+                         positions, D, k0, k1, out, planes);
+}
+
+}  // namespace
+
+cudaError_t launch_encrypt_batch(const uint8_t *bits, uint64_t n, uint64_t first_block, uint32_t L, uint64_t pad_mask,
+                                 const uint64_t *mask, const uint64_t *positions, uint32_t D, uint64_t seed,
+                                 uint64_t *out, cudaStream_t stream) {
+    return launch_encrypt<false>(bits, UIntPlanes{}, n, first_block, L, pad_mask, mask, positions, D, seed, out, stream);
+}
+
+cudaError_t launch_encrypt_uint(const uint64_t *values, uint64_t n, uint32_t width, uint64_t first_block, uint32_t L,
+                                uint64_t pad_mask, const uint64_t *mask, const uint64_t *positions, uint32_t D,
+                                uint64_t seed, uint64_t *out, cudaStream_t stream) {
+    const UIntPlanes planes = {values, n, n ? UINT64_MAX / n : 0};
+    return launch_encrypt<true>(nullptr, planes, (uint64_t)width * n, first_block, L, pad_mask, mask, positions, D,
+                                seed, out, stream);
 }
 
 }  // namespace csgn

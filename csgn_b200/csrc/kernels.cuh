@@ -83,6 +83,19 @@ struct SegDecTask {
 };
 cudaError_t launch_seg_decrypt(const uint64_t *v, uint32_t L, const uint64_t *mask, const uint64_t *off,
                                const SegDecTask *tasks, uint32_t n_tasks, uint64_t *counts, cudaStream_t stream);
+// The same over the bit planes of encrypted integers (csgn_decrypt_uint_async): plane j is the array at planes[j].v
+// with offsets planes[j].off (device), task t walks blocks of plane task_plane[t], and bit j of values[e] (zeroed by the
+// caller in stream order) is XORed with the parity of element e of plane j.  units16: L is even and every plane is
+// 16-byte aligned.  One launch.
+struct SegPlane {
+    const uint64_t *v, *off;
+};
+cudaError_t launch_seg_decrypt_uint(const SegPlane *planes, bool units16, uint32_t L, const uint64_t *mask,
+                                    const SegDecTask *tasks, const uint32_t *task_plane, uint32_t n_tasks,
+                                    uint64_t *values, cudaStream_t stream);
+// values[entries[2i]] ^= (counts[i] & 1) << entries[2i + 1], i < n: the plane elements counted on their own.  One launch.
+cudaError_t launch_seg_uint_pack(const uint64_t *counts, const uint64_t *entries, uint32_t n, uint64_t *values,
+                                 cudaStream_t stream);
 // Cancellation (csgn_seg_cancel): a warp task is the blocks [first, end) of one element, whose first block is block
 // `elem` of the array and whose open-addressing region is slots [slot, slot + slot_mask + 1) (a power of two).  Three
 // passes over the same tasks, one launch each:
@@ -172,6 +185,15 @@ constexpr uint32_t kPermSliceStride = 36;
 cudaError_t launch_encrypt_batch(const uint8_t *bits, uint64_t n, uint64_t first_block, uint32_t L, uint64_t pad_mask,
                                  const uint64_t *mask, const uint64_t *positions, uint32_t D, uint64_t seed,
                                  uint64_t *out, cudaStream_t stream);
+// The width*n blocks that launch_encrypt_batch builds from the bit planes of values[0..n) laid one after another
+// (LSB first): block j*n + k encrypts bit j of values[k].  One launch.
+struct UIntPlanes {
+    const uint64_t *values;
+    uint64_t n, magic;
+};
+cudaError_t launch_encrypt_uint(const uint64_t *values, uint64_t n, uint32_t width, uint64_t first_block, uint32_t L,
+                                uint64_t pad_mask, const uint64_t *mask, const uint64_t *positions, uint32_t D,
+                                uint64_t seed, uint64_t *out, cudaStream_t stream);
 
 // xor / wrapping sum / sum(w[i]*(2i+1)) of n_words words, accumulated into acc[0..2]
 // (device, must be zeroed by the caller).

@@ -5,7 +5,8 @@
 //   grouped multiply   element k = a_k * b_k, all-pairs AND, i-major      (reference src/Ciphertext.cpp:153-163),
 //                      or a sum of products and plain terms a0_k*b0_k || ... || c0_k || ... (operands in any buffers;
 //                      a term is a product with one all-ones block)
-//   segmented decrypt  counts[k] = satisfied blocks of element k           (reference src/SecretKey.cpp:126-140)
+//   segmented decrypt  counts[k] = satisfied blocks of element k           (reference src/SecretKey.cpp:126-140),
+//                      or over the bit planes of encrypted integers: bit j of values[k] = parity of element k of plane j
 //   cancellation       element k = the first occurrence, in order, of every block value that occurs an odd number of
 //                      times in element k (insert into a hash table per element, count, write)
 //
@@ -142,12 +143,15 @@ seg_mul_kernel(VT *__restrict__ out, const uint32_t U, const SegMulItem *__restr
 // segmented decrypt: groups of G lanes (G a power of two, >= U up to 32) evaluate one block each per warp step; the
 // group's verdict is one ballot.  Group leaders that hold the same element find each other with match.any and add
 // their verdicts with one more ballot: one atomic per (warp step, element), not one per block.
+// With PLANES the tasks walk the bit planes of encrypted integers: task t reads plane task_plane[t], whose storage and
+// offsets come from planes[], and XORs its elements' parities into bit j of counts[e] instead of adding the counts.
 // ---------------------------------------------------------------------------------------
-template <typename VT>
-__global__ void __launch_bounds__(kSegThreads)
+// The plane form holds the plane's addresses in registers: 6 resident CTAs per SM keep ptxas from spilling them.
+template <typename VT, bool PLANES>
+__global__ void __launch_bounds__(kSegThreads, PLANES ? 6 : 0)
 seg_decrypt_kernel(const VT *__restrict__ v, const uint32_t U, const uint32_t log2g, const VT *__restrict__ mask,
                    const uint64_t *__restrict__ off, const SegDecTask *__restrict__ tasks, const uint32_t n_tasks,
-                   uint64_t *counts) {
+                   uint64_t *counts, const SegPlane *__restrict__ planes, const uint32_t *__restrict__ task_plane) {
     const uint32_t lane = threadIdx.x & 31u;
     const uint32_t G = 1u << log2g, sub = lane & (G - 1u), grp = lane >> log2g, B = 32u >> log2g;
     const uint32_t gmask = G == 32u ? 0xffffffffu : ((1u << G) - 1u) << (grp * G);
@@ -155,6 +159,12 @@ seg_decrypt_kernel(const VT *__restrict__ v, const uint32_t U, const uint32_t lo
     pdl_enter();
     for (uint32_t t = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); t < n_tasks; t += warps) {
         const SegDecTask task = tasks[t];
+        uint32_t plane = 0;
+        if constexpr (PLANES) {
+            plane = __ldg(task_plane + t);
+            v = reinterpret_cast<const VT *>(planes[plane].v);
+            off = planes[plane].off;
+        }
         uint64_t e = task.elem;                                // element of this lane's block: never decreases
         for (uint64_t blk0 = task.first; blk0 < task.end; blk0 += B) {
             const uint64_t blk = blk0 + grp;
@@ -182,10 +192,27 @@ seg_decrypt_kernel(const VT *__restrict__ v, const uint32_t U, const uint32_t lo
             const uint64_t key = leader ? e : ~0ull;
             const uint32_t peers = __match_any_sync(0xffffffffu, key);
             const uint32_t sum = __popc(peers & __ballot_sync(0xffffffffu, leader && sat));
-            if (leader && sum && lane == (uint32_t)(__ffs(peers) - 1))
-                atomicAdd(reinterpret_cast<unsigned long long *>(counts + e), (unsigned long long)sum);
+            if constexpr (PLANES) {
+                if (leader && (sum & 1u) && lane == (uint32_t)(__ffs(peers) - 1))
+                    atomicXor(reinterpret_cast<unsigned long long *>(counts + e), 1ull << plane);
+            } else {
+                if (leader && sum && lane == (uint32_t)(__ffs(peers) - 1))
+                    atomicAdd(reinterpret_cast<unsigned long long *>(counts + e), (unsigned long long)sum);
+            }
         }
     }
+}
+
+// The parities of the plane elements that were counted on their own (launch_decrypt_count): entry i XORs bit
+// entries[2i + 1] of values[entries[2i]] with counts[i] & 1.  Several entries may name one value.
+__global__ void __launch_bounds__(kSegThreads)
+seg_uint_pack_kernel(const uint64_t *__restrict__ counts, const uint64_t *__restrict__ entries, const uint32_t n,
+                     uint64_t *values) {
+    pdl_enter();
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+        if (__ldg(counts + i) & 1u)
+            atomicXor(reinterpret_cast<unsigned long long *>(values + __ldg(entries + 2 * i)),
+                      1ull << __ldg(entries + 2 * i + 1));
 }
 
 // ---------------------------------------------------------------------------------------
@@ -387,12 +414,37 @@ cudaError_t launch_seg_decrypt(const uint64_t *v, uint32_t L, const uint64_t *ma
     const uint32_t log2g = group_log2(U);
     count_launch();
     if (units16)
-        return launch_kernel(seg_decrypt_kernel<uint4>, seg_grid(n_tasks), kSegThreads, 0, stream,
+        return launch_kernel(seg_decrypt_kernel<uint4, false>, seg_grid(n_tasks), kSegThreads, 0, stream,
                              reinterpret_cast<const uint4 *>(v), U, log2g, reinterpret_cast<const uint4 *>(mask), off,
-                             tasks, n_tasks, counts);
-    return launch_kernel(seg_decrypt_kernel<uint2>, seg_grid(n_tasks), kSegThreads, 0, stream,
+                             tasks, n_tasks, counts, (const SegPlane *)nullptr, (const uint32_t *)nullptr);
+    return launch_kernel(seg_decrypt_kernel<uint2, false>, seg_grid(n_tasks), kSegThreads, 0, stream,
                          reinterpret_cast<const uint2 *>(v), U, log2g, reinterpret_cast<const uint2 *>(mask), off, tasks,
-                         n_tasks, counts);
+                         n_tasks, counts, (const SegPlane *)nullptr, (const uint32_t *)nullptr);
+}
+
+cudaError_t launch_seg_decrypt_uint(const SegPlane *planes, bool units16, uint32_t L, const uint64_t *mask,
+                                    const SegDecTask *tasks, const uint32_t *task_plane, uint32_t n_tasks,
+                                    uint64_t *values, cudaStream_t stream) {
+    if (n_tasks == 0) return cudaSuccess;
+    units16 = units16 && !(L & 1u) && (reinterpret_cast<uintptr_t>(mask) & 15u) == 0;
+    const uint32_t U = units16 ? L / 2 : L;
+    const uint32_t log2g = group_log2(U);
+    count_launch();
+    if (units16)
+        return launch_kernel(seg_decrypt_kernel<uint4, true>, seg_grid(n_tasks), kSegThreads, 0, stream,
+                             (const uint4 *)nullptr, U, log2g, reinterpret_cast<const uint4 *>(mask),
+                             (const uint64_t *)nullptr, tasks, n_tasks, values, planes, task_plane);
+    return launch_kernel(seg_decrypt_kernel<uint2, true>, seg_grid(n_tasks), kSegThreads, 0, stream,
+                         (const uint2 *)nullptr, U, log2g, reinterpret_cast<const uint2 *>(mask),
+                         (const uint64_t *)nullptr, tasks, n_tasks, values, planes, task_plane);
+}
+
+cudaError_t launch_seg_uint_pack(const uint64_t *counts, const uint64_t *entries, uint32_t n, uint64_t *values,
+                                 cudaStream_t stream) {
+    if (n == 0) return cudaSuccess;
+    count_launch();
+    const uint32_t grid = std::min<uint32_t>((n + kSegThreads - 1) / kSegThreads, device_props().sm_count * 4);
+    return launch_kernel(seg_uint_pack_kernel, grid, kSegThreads, 0, stream, counts, entries, n, values);
 }
 
 cudaError_t launch_seg_cancel_insert(const uint64_t *v, uint32_t L, bool units16, const SegCancelTask *tasks,

@@ -571,6 +571,286 @@ class Circuit:
         return [CiphertextArray(Ciphertext(_vp(out[j]), ctx), out_offs[j]) for j in range(len(outputs))]
 
 
+class UIntCircuit:
+    """Integer netlists over encrypted integers (EncryptedUInt), built on the host and evaluated as ONE Circuit call.
+
+    An integer is a list of wire ids, LSB first.  Wires: operand i, bit j is input i*width + j; then the `one` input
+    (one=True: the caller supplies an encryption of 1 per lane, which only the key holder can make); then the zero
+    input, n empty elements, which the builder declares and evaluate() supplies (an empty ciphertext decrypts to 0).
+    Every operation is a sum of products plus terms over GF(2) (XOR of ANDs); a gate that folds to one wire (x + 0,
+    x*1, a single term) adds no gate.  Operands may differ in width: the shorter one is zero-extended, and the result
+    has the larger width.  certFHE::UIntCircuit builds the same netlists, wire for wire.
+
+    Size: with cancel=True a result holds, per lane, the blocks of its function's algebraic normal form over the input
+    blocks (whatever the netlist) that compaction keeps.  That form stays small for add, and, xor, or, select and the
+    shifts at any width, but grows about threefold per bit for sub, neg, the comparisons, min, max and mul (lt and ne
+    of two W-bit operands have 3^W - 1 monomials), so those are practical up to about 8-12 bits, and compositions of
+    them at fewer."""
+
+    def __init__(self, width, n_operands, one=False):
+        width, n_operands = int(width), int(n_operands)
+        if not 1 <= width <= 64:
+            raise ValueError("width %d outside 1..64" % width)
+        if n_operands < 0:
+            raise ValueError("negative operand count")
+        self.width, self.n_operands = width, n_operands
+        self.inputs = [[i * width + j for j in range(width)] for i in range(n_operands)]
+        self.one = n_operands * width if one else None
+        self.zero = n_operands * width + (1 if one else 0)
+        self.circuit = Circuit(self.zero + 1)
+
+    @property
+    def last_fallback(self):
+        return self.circuit.last_fallback
+
+    def netlist(self):
+        """(inputs, flat gates) as csgn_seg_circuit takes them: per gate p, q, p operand pairs, q terms."""
+        return self.circuit.n_inputs, list(self.circuit._gates)
+
+    # -- gates ----------------------------------------------------------------------------------------------------
+    def _gate(self, products, terms):
+        z, o = self.zero, self.one
+        terms = [w for w in terms if w != z]
+        prods = []
+        for u, v in products:
+            if u == z or v == z:
+                continue
+            if u == o:
+                terms.append(v)
+            elif v == o:
+                terms.append(u)
+            else:
+                prods.append((u, v))
+        if not prods and not terms:
+            return z
+        if not prods and len(terms) == 1:
+            return terms[0]
+        return self.circuit.gate(prods, terms)
+
+    def _not(self, w):
+        if self.one is None:
+            raise ValueError("NOT needs the `one` input: build the circuit with UIntCircuit(..., one=True)")
+        return self._gate([], [w, self.one])
+
+    def _pair(self, a, b):
+        a, b = list(a), list(b)
+        w = max(len(a), len(b))
+        return a + [self.zero] * (w - len(a)), b + [self.zero] * (w - len(b))
+
+    # -- operations -----------------------------------------------------------------------------------------------
+    def add(self, a, b):
+        """a + b mod 2^W: s = t + c, c' = a*b + t*c with t = a + b (no carry out of the top bit)."""
+        a, b = self._pair(a, b)
+        out, c = [], self.zero
+        for i in range(len(a)):
+            t = self._gate([], [a[i], b[i]])
+            out.append(self._gate([], [t, c]))
+            if i + 1 < len(a):
+                c = self._gate([(a[i], b[i]), (t, c)], [])
+        return out
+
+    def _borrow(self, a, b, r, t):
+        """borrow of a - b - r: a*b + t*r + b + r, which is (not a and b) or (not (a xor b) and r)"""
+        return self._gate([(a, b), (t, r)], [b, r])
+
+    def sub(self, a, b):
+        """a - b mod 2^W: d = t + r, borrow r' = a*b + t*r + b + r."""
+        a, b = self._pair(a, b)
+        out, r = [], self.zero
+        for i in range(len(a)):
+            t = self._gate([], [a[i], b[i]])
+            out.append(self._gate([], [t, r]))
+            if i + 1 < len(a):
+                r = self._borrow(a[i], b[i], r, t)
+        return out
+
+    def neg(self, a):
+        return self.sub([self.zero] * len(a), a)
+
+    def lt(self, a, b):
+        """[a < b] (unsigned, 1 bit): the borrow out of a - b."""
+        a, b = self._pair(a, b)
+        r = self.zero
+        for i in range(len(a)):
+            t = self._gate([], [a[i], b[i]]) if r != self.zero else self.zero
+            r = self._borrow(a[i], b[i], r, t)
+        return [r]
+
+    def gt(self, a, b):
+        return self.lt(b, a)
+
+    def ne(self, a, b):
+        """[a != b] (1 bit): OR over the bits of a + b, o' = o + t + o*t."""
+        a, b = self._pair(a, b)
+        o = self.zero
+        for i in range(len(a)):
+            t = self._gate([], [a[i], b[i]])
+            o = t if o == self.zero else self._gate([(o, t)], [o, t])
+        return [o]
+
+    def eq(self, a, b):
+        return [self._not(self.ne(a, b)[0])]
+
+    def le(self, a, b):
+        return [self._not(self.gt(a, b)[0])]
+
+    def ge(self, a, b):
+        return [self._not(self.lt(a, b)[0])]
+
+    def invert(self, a):
+        return [self._not(w) for w in a]
+
+    def select(self, s, x, y):
+        """s ? x : y per bit (s one bit): s*x + s*y + y."""
+        if len(s) != 1:
+            raise ValueError("select needs a 1-bit condition, got %d bits" % len(s))
+        x, y = self._pair(x, y)
+        return [self._gate([(s[0], x[i]), (s[0], y[i])], [y[i]]) for i in range(len(x))]
+
+    def min(self, a, b):
+        return self.select(self.lt(a, b), a, b)
+
+    def max(self, a, b):
+        return self.select(self.lt(a, b), b, a)
+
+    def mul(self, a, b):
+        """a * b mod 2^W: schoolbook rows a*b_j shifted by j, each added to the accumulator with ripple carries
+        (a column of three addends carries their majority, of two their product)."""
+        a, b = self._pair(a, b)
+        W, z = len(a), self.zero
+        acc = [z] * W
+        for j in range(W):
+            pp = [z] * j + [self._gate([(a[i], b[j])], []) for i in range(W - j)]
+            c, out = z, []
+            for k in range(W):
+                ops = [x for x in (acc[k], pp[k], c) if x != z]
+                out.append(self._gate([], ops))
+                prods = [(ops[p], ops[q]) for p in range(len(ops)) for q in range(p + 1, len(ops))]
+                c = self._gate(prods, []) if prods and k + 1 < W else z
+            acc = out
+        return acc
+
+    def and_(self, a, b):
+        a, b = self._pair(a, b)
+        return [self._gate([(x, y)], []) for x, y in zip(a, b)]
+
+    def xor(self, a, b):
+        a, b = self._pair(a, b)
+        return [self._gate([], [x, y]) for x, y in zip(a, b)]
+
+    def or_(self, a, b):
+        a, b = self._pair(a, b)
+        return [self._gate([(x, y)], [x, y]) for x, y in zip(a, b)]
+
+    def shl(self, a, k):
+        """a << k, keeping a's width (no gates)."""
+        a, k = list(a), int(k)
+        if k < 0:
+            raise ValueError("negative shift")
+        return ([self.zero] * k + a)[:len(a)]
+
+    def shr(self, a, k):
+        """a >> k, keeping a's width (no gates)."""
+        a, k = list(a), int(k)
+        if k < 0:
+            raise ValueError("negative shift")
+        return (a + [self.zero] * k)[k:k + len(a)]
+
+    # -- evaluation -----------------------------------------------------------------------------------------------
+    def evaluate(self, operands, results, min_bits=None, cancel=False, lane_capacity=0, one=None):
+        """One Circuit.evaluate call (csgn_seg_circuit) for every result (a list of wires each): one EncryptedUInt per
+        result.  operands: one EncryptedUInt per operand, of at most `width` bits (missing high bits are zero);
+        one: the CiphertextArray that encrypts 1 in every lane, for a circuit built with one=True."""
+        operands = list(operands)
+        if len(operands) != self.n_operands:
+            raise ValueError("the circuit has %d operands, got %d" % (self.n_operands, len(operands)))
+        if (one is None) != (self.one is None):
+            raise ValueError("the circuit was built with one=%s" % (self.one is not None))
+        arrays = [one] if one is not None else []
+        for x in operands:
+            arrays.append(x.planes[0])
+        if not arrays:
+            raise ValueError("evaluate needs at least one operand or the `one` input")
+        n, ctx = len(arrays[0]), arrays[0].ctx
+        zero = CiphertextArray(Ciphertext.empty(0, ctx), np.zeros(n + 1, dtype=np.uint64))
+        inputs = []
+        for x in operands:
+            if x.width > self.width:
+                raise ValueError("an operand of %d bits in a %d-bit circuit" % (x.width, self.width))
+            inputs += list(x.planes) + [zero] * (self.width - x.width)
+        if one is not None:
+            inputs.append(one)
+        inputs.append(zero)
+        results = [[int(w) for w in r] for r in results]
+        flat = [w for r in results for w in r]
+        arrs = self.circuit.evaluate(inputs, flat, min_bits, cancel, lane_capacity)
+        out, at = [], 0
+        for r in results:
+            out.append(EncryptedUInt(arrs[at:at + len(r)]))
+            at += len(r)
+        return out
+
+
+class EncryptedUInt:
+    """A vector of n encrypted W-bit unsigned integers: W CiphertextArrays of n elements, its bit planes, LSB first
+    (planes[j] element k encrypts bit j of lane k).  Made by SecretKey.encrypt_uint or UIntCircuit.evaluate, read by
+    SecretKey.decrypt_uint.  The operators + - * (mod 2^W), < > (1-bit results) and & ^ | each build a one-operation
+    UIntCircuit and make one call, compacted and cancelled."""
+
+    def __init__(self, planes):
+        self.planes = list(planes)
+        if not self.planes:
+            raise ValueError("an encrypted integer needs at least one bit plane")
+        n = len(self.planes[0])
+        if any(len(p) != n for p in self.planes):
+            raise ValueError("bit planes of different lengths")
+        self.ctx = self.planes[0].ctx
+
+    @property
+    def width(self):
+        return len(self.planes)
+
+    def __len__(self):
+        return len(self.planes[0])
+
+    @staticmethod
+    def _apply(op, *xs):
+        c = UIntCircuit(max(x.width for x in xs), len(xs))
+        return c.evaluate(xs, [getattr(c, op)(*c.inputs)], cancel=True)[0]
+
+    def __add__(self, other):
+        return self._apply("add", self, other)
+
+    def __sub__(self, other):
+        return self._apply("sub", self, other)
+
+    def __mul__(self, other):
+        return self._apply("mul", self, other)
+
+    def __lt__(self, other):
+        return self._apply("lt", self, other)
+
+    def __gt__(self, other):
+        return self._apply("gt", self, other)
+
+    def __and__(self, other):
+        return self._apply("and_", self, other)
+
+    def __xor__(self, other):
+        return self._apply("xor", self, other)
+
+    def __or__(self, other):
+        return self._apply("or_", self, other)
+
+    @staticmethod
+    def select(c, x, y):
+        """c ? x : y lane by lane, c a 1-bit EncryptedUInt."""
+        if c.width != 1:
+            raise ValueError("select needs a 1-bit condition, got %d bits" % c.width)
+        u = UIntCircuit(max(x.width, y.width), 3)
+        return u.evaluate([c, x, y], [u.select(u.inputs[0][:1], u.inputs[1], u.inputs[2])], cancel=True)[0]
+
+
 class Result:
     """A decrypt whose count the host reads later (csgn_result)."""
 
@@ -674,6 +954,33 @@ class SecretKey:
         """CiphertextArray of len(bits) one-block encryptions (csgn_encrypt_batch, offsets 0, 1, ..., n)."""
         n = np.asarray(bits).size
         return CiphertextArray(self.encrypt_batch(bits, seed, first_block), np.arange(n + 1, dtype=np.uint64))
+
+    def encrypt_uint(self, values, width, seed, first_block=0):
+        """EncryptedUInt of len(values) lanes of `width` bits (csgn_encrypt_uint: one launch, no synchronisation).
+        A value that does not fit in `width` bits is an error."""
+        v = np.ascontiguousarray(np.asarray(values, dtype=np.uint64).reshape(-1))
+        width = int(width)
+        h = (_vp * max(1, width))()
+        check(_lib().csgn_encrypt_uint(self._h, v.ctypes.data_as(_vp), v.size, width, int(first_block), int(seed), h))
+        off = np.arange(v.size + 1, dtype=np.uint64)
+        return EncryptedUInt([CiphertextArray(Ciphertext(_vp(h[j]), self.ctx), off) for j in range(width)])
+
+    def _uint_args(self, x):
+        planes = (_vp * x.width)(*[p.storage._h for p in x.planes])
+        offs = (_vp * x.width)(*[p.offsets.ctypes.data for p in x.planes])
+        return planes, offs
+
+    def decrypt_uint(self, x):
+        """csgn_decrypt_uint: the lanes of x as a numpy uint64 array (one launch, one synchronisation)."""
+        values = np.zeros(len(x), dtype=np.uint64)
+        planes, offs = self._uint_args(x)
+        check(_lib().csgn_decrypt_uint(planes, offs, x.width, len(x), self._h, values.ctypes.data_as(_vp)))
+        return values
+
+    def decrypt_uint_async(self, x, device_values_ptr):
+        """csgn_decrypt_uint_async: the lanes of x to len(x) device uint64 words, no synchronisation."""
+        planes, offs = self._uint_args(x)
+        check(_lib().csgn_decrypt_uint_async(planes, offs, x.width, len(x), self._h, _vp(device_values_ptr)))
 
     def decrypt_array_count_async(self, arr, device_counts_ptr):
         """csgn_seg_decrypt_count_async: device_counts[k] = satisfied blocks of element k, no synchronisation."""

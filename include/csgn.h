@@ -309,6 +309,30 @@ int csgn_seg_circuit(const csgn_buf *const *in, const uint64_t *const *in_off, u
                      const uint32_t *outputs, uint32_t n_outputs, uint32_t min_bits, int cancel,
                      uint64_t lane_capacity, uint64_t *const *out_off, csgn_buf **out, uint64_t *n_fallback);
 
+/* ---- encrypted integers ------------------------------------------------------------------------------------------
+ * A W-bit integer vector of n lanes is W ciphertext arrays, its bit planes, LSB first: element k of plane j encrypts bit
+ * j of lane k.  Circuits over them (csgn_seg_circuit) compute sums, comparisons and products lane by lane. */
+/* width (1..64) bit planes of n lanes.  Plane j (LSB = 0) is an array of n one-block elements with offsets 0, 1, .., n.
+ * Block k of plane j encrypts bit j of values[k].  out[0..width) receive width handles that share ONE allocation, as in
+ * csgn_buf_upload_batch; each can be freed on its own.  Word for word, block k of plane j is block j*n + k of
+ * csgn_encrypt_batch(key, bit planes laid one after another, width*n, first_block, seed): the same Philox counter
+ * (first_block + j*n + k, unit).  values go to the device through the library's pinned staging, so the call makes no
+ * host synchronisation (unlike csgn_encrypt_batch) and the caller may reuse `values` as soon as it returns (beyond
+ * 64 MB of values the call copies from the caller's memory and waits).  A value with a set bit at position `width` or
+ * above is rejected (CSGN_ERR_INVALID_ARGUMENT), never masked.  n == 0 gives width buffers of 0 blocks.  One launch. */
+int csgn_encrypt_uint(const csgn_key *key, const uint64_t *values, uint64_t n, uint32_t width,
+                      uint64_t first_block, uint64_t seed, csgn_buf **out);
+/* device_values[k] = sum over j of (satisfied blocks of element k of plane j & 1) << j.  The planes may be separate
+ * buffers of any sizes, such as circuit outputs; plane j has offsets plane_off[j][0..n].  No host synchronisation.
+ * All elements below 8 MB, of every plane, are served by one launch; larger ones are counted one launch each and
+ * merged by one more.  The checks (null arguments, width 1..64, every plane's offsets, L of every plane against the
+ * key) run on the host and allocate nothing on error; n == 0 makes no launch. */
+int csgn_decrypt_uint_async(const csgn_buf *const *planes, const uint64_t *const *plane_off, uint32_t width,
+                            uint64_t n, const csgn_key *key, uint64_t *device_values);
+/* The same, with values on the host: one host synchronisation. */
+int csgn_decrypt_uint(const csgn_buf *const *planes, const uint64_t *const *plane_off, uint32_t width, uint64_t n,
+                      const csgn_key *key, uint64_t *values);
+
 /* Permutation as a device source map: out_bit[i] = in_bit[perm[i]], i < N
  * (src/Ciphertext.cpp:33-34).  Fails unless perm is a bijection of [0,N). */
 int csgn_perm_create(uint64_t N, const uint64_t *perm, csgn_perm **out);
